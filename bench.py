@@ -3,6 +3,7 @@
 
     python bench.py --gpus 1 --steps K --warmup W                      # this implementation
     python bench.py --impl reference --gpus 1 --steps K --warmup W      # CPU port of the reference
+    python bench.py ... --dump-outputs DIR                              # + the last timed step's outputs as DIR/*.npy
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 A step = id draw + gather + normalise + logits + diagonal CE + full backward to the dense
@@ -66,6 +67,8 @@ def parse():
     ap.add_argument("--no-head-line", action="store_true", help="skip the secondary head-mode measurement")
     ap.add_argument("--clock-period", type=float, default=0.02, help="seconds between NVML clock samples (0: no sampling)")
     ap.add_argument("--settle", type=float, default=0.0, help="experiment: seconds to idle after the maps are created, before warm-up")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (loss, ids, gradients; rank 0) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -172,12 +175,55 @@ class ClockSampler:
 
 
 def cpu_port_step(orc, src, tgt, tau, patches):
-    """One fwd+bwd of the oracle's op-for-op torch port (same ATen sequence as the reference)."""
+    """One fwd+bwd of the oracle's op-for-op torch port (same ATen sequence as the reference) -> (loss, ids)."""
     for t in tgt:
         t.grad = None
-    loss, _ = orc.patchnce_loss_torch(src, tgt, tau, patches)
+    loss, ids = orc.patchnce_loss_torch(src, tgt, tau, patches)
     loss.backward()
-    return loss
+    return loss, ids
+
+
+DUMP_BYTES = 64 << 20
+DUMP_FLAT = 65536
+
+
+def dump_outputs(out_dir, loss, tgt, ids, head=None):
+    """--dump-outputs: what one step handed its caller, so that two builds can be compared file for file (the inputs
+    and ids are seeded: same arguments, same step).  All float32 / float64, at most DUMP_BYTES in all:
+      loss.npy                       the loss (float64, shape (1,))
+      ids_l{l}.npy                   the patch positions drawn for layer l (float64)
+      grad_l{l}.npy                  d loss / d tgt_feats[l] at those positions, (images, C, P) float32: every value the
+                                     step can make non-zero; all images, or a fixed seeded sample of them (images_sampled.npy)
+                                     when all would pass the budget
+      grad_l{l}_flat.npy             a fixed seeded sample of DUMP_FLAT entries of the whole gradient map, which shows a
+                                     write outside the sampled positions
+      head_{name}.npy                head mode: the gradient of every netF parameter"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": np.array([float(loss.detach().double().item())])}
+    if head is not None:
+        for name, p in head.named_parameters():
+            if p.grad is not None:
+                arrays["head_" + name.replace(".", "_")] = p.grad.detach().float().cpu().numpy()
+    g = torch.Generator().manual_seed(0)
+    for l, (t, i) in enumerate(zip(tgt, ids)):
+        arrays[f"ids_l{l}"] = i.detach().double().cpu().numpy()
+        flat = torch.randint(0, t.numel(), (min(DUMP_FLAT, t.numel()),), generator=g)
+        arrays[f"grad_l{l}_flat"] = t.grad.detach().contiguous().view(-1)[flat.to(t.device)].float().cpu().numpy()
+    used = sum(a.nbytes for a in arrays.values())
+    per_image = sum(t.shape[1] * i.numel() * 4 for t, i in zip(tgt, ids))
+    batch = tgt[0].shape[0]
+    n_img = min(batch, (DUMP_BYTES - used - 8 * batch) // per_image)
+    if n_img <= 0:
+        raise SystemExit(f"--dump-outputs: one image's gradients ({per_image} bytes) do not fit in {DUMP_BYTES} bytes")
+    images = torch.arange(batch) if n_img == batch else torch.randperm(batch, generator=g)[:n_img].sort().values
+    if n_img < batch:
+        arrays["images_sampled"] = images.double().numpy()
+    for l, (t, i) in enumerate(zip(tgt, ids)):
+        cols = t.grad.detach().flatten(2)[:, :, i.to(t.device)]           # (B, C, P)
+        arrays[f"grad_l{l}"] = cols[images.to(t.device)].float().cpu().numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def cpu_baseline(args, layers, seconds, min_steps=2):
@@ -230,8 +276,10 @@ def run_reference(args):
         cpu_port_step(orc, src, tgt, args.tau, args.patches)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_port_step(orc, src, tgt, args.tau, args.patches)
+        loss, ids = cpu_port_step(orc, src, tgt, args.tau, args.patches)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, loss, tgt, ids)
     n_patches = b * sum(min(args.patches, h * w) for _, h, w, _ in layers)
     value = n_patches * args.steps / dt
     sample = (f"each step = B={b} images of the workload (reference backward is O(B^2), full B={args.batch} "
@@ -318,6 +366,7 @@ def main():
     ev_b1 = {i: torch.cuda.Event(enable_timing=True) for i in range(0, args.steps, EV_STRIDE)}
     ev_step = [torch.cuda.Event(enable_timing=True) for _ in range(args.steps)]     # end of every step
     host_us = []
+    head_ids = [None]
 
     def step(i=None):
         for t in tgt:
@@ -328,8 +377,8 @@ def main():
             netF.zero_grad(set_to_none=True)
             # dp_group: the head gradients leave backward() already averaged over the ranks -- the only
             # collective of the path (SURVEY.md 8e), started on a side stream under the dense kernel
-            loss, _ = pn.patchnce_with_head(netF, src, tgt, args.tau, args.patches, math=math,
-                                            dp_group=True if world > 1 else None)
+            loss, head_ids[0] = pn.patchnce_with_head(netF, src, tgt, args.tau, args.patches, math=math,
+                                                      dp_group=True if world > 1 else None)
         if i in ev_b0:
             ev_b0[i].record()
         loss.backward()
@@ -373,6 +422,8 @@ def main():
     barrier()
     gc.enable()
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, loss, tgt, crit.last_patch_ids if netF is None else head_ids[0], netF)
     ms = e0.elapsed_time(e1)
     tmax = torch.tensor([ms], device=dev)
     if world > 1:

@@ -1,7 +1,6 @@
 """Encoder-feature reuse (SURVEY.md section 8f row 2): the maps tapped during ``generator(x)`` are, bit for bit,
-what ``generator.get_feature_layers(x, ids)`` returns -- for the stand-in generator and, where the reference tree
-is mounted, for the unmodified reference generator -- and every condition under which they would not be is a miss."""
-import os
+what ``generator.get_feature_layers(x, ids)`` returns -- for the stand-in generator, narrow and at the reference
+generator's default size -- and every condition under which they would not be is a miss."""
 import sys
 
 import pytest
@@ -10,8 +9,6 @@ import torch
 from standin_generator import StandInGenerator
 from gan_variant_research_b200.feature_reuse import (EncoderFeatureCache, enable_encoder_feature_reuse,
                                                      logical_layer_modules)
-
-REF = "/root/reference"
 
 
 def _same(a, b):
@@ -75,16 +72,12 @@ def test_every_stale_condition_is_a_miss():
     assert not hasattr(gen, "_pnce_encoder_feature_cache")
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "GAN_Variant1")), reason="reference tree not mounted")
 @pytest.mark.parametrize("ids", [[0, 4, 8, 12, 16], [0, 4, 8, 12, 13]])
 def test_against_the_unmodified_reference_generator(ids):
-    sys.path.insert(0, REF)
-    try:
-        from GAN_Variant1.models.generator_resnet_attn import ResNetGenerator
-    finally:
-        sys.path.remove(REF)
+    """The reference's ``ResNetGenerator()`` at its defaults (ngf=64, 9 residual blocks, 14 logical layers), which the
+    stand-in reproduces on the maps and losses frozen from the reference (tests/test_oracle_golden.py)."""
     torch.manual_seed(0)
-    gen = ResNetGenerator()
+    gen = StandInGenerator(ngf=64, n_blocks=9)
     cache = enable_encoder_feature_reuse(gen, ids)
     x = torch.randn(1, 3, 64, 64)
     fake = gen(x)                                                    # train_cutpp.py:270
@@ -145,11 +138,30 @@ def test_compute_patchnce_loss_with_reuse_equals_without(monkeypatch):
             assert float((a - b).abs().max()) <= 0.3 * float(a.abs().max())
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "GAN_Variant1")), reason="reference tree not mounted")
-def test_shim_repoints_the_optimiser_side_seams():
+REFERENCE_SEAMS = {          # module of the reference package -> the names install_reference_shim re-points there
+    "utils/io_ckpt.py": "class EMA:\n    pass\n",                                                     # train_cutpp.py:34
+    "utils/amp_utils.py": "class AMPContext:\n    def step_optimizer(self, *a, **k):\n        pass\n",    # amp_utils.py:29
+    "training/diffaugment.py": "class DiffAugment:\n    pass\n",                                        # train_cutpp.py:30
+    "losses/adv_hinge.py": "def discriminator_hinge_loss(*a):\n    pass\n\n\ndef generator_hinge_loss(*a):\n    pass\n",
+    "losses/patchnce_cut.py": "class PatchNCELoss:\n    pass\n\n\ndef compute_patchnce_loss(*a):\n    pass\n",
+}
+
+
+def test_shim_repoints_the_optimiser_side_seams(tmp_path):
+    """On a package with the reference's module layout (GAN_Variant1/..., the seams as placeholders): the shim must
+    re-point every seam a training script imports by name, and win over the on-disk patchnce_cut module."""
     import gan_variant_research_b200 as pn
-    sys.path.insert(0, REF)
+    for path, body in REFERENCE_SEAMS.items():
+        f = tmp_path / "GAN_Variant1" / path
+        f.parent.mkdir(parents=True, exist_ok=True)
+        f.write_text(body)
+        for d in (f.parent, f.parent.parent):
+            (d / "__init__.py").touch()
+    root = str(tmp_path)
+    sys.path.insert(0, root)
     saved = {k: v for k, v in sys.modules.items() if k.startswith("GAN_Variant1")}
+    for k in saved:
+        del sys.modules[k]
     try:
         import GAN_Variant1.utils.amp_utils as au
         import GAN_Variant1.utils.io_ckpt as ck
@@ -164,7 +176,7 @@ def test_shim_repoints_the_optimiser_side_seams():
         assert compute_patchnce_loss is pn.compute_patchnce_loss
         ck.EMA, au.AMPContext.step_optimizer = keep
     finally:
-        sys.path.remove(REF)
+        sys.path.remove(root)
         for k in [k for k in sys.modules if k.startswith("GAN_Variant1")]:
             del sys.modules[k]
         sys.modules.update(saved)
