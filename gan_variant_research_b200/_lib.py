@@ -11,7 +11,7 @@ MATH_SIMT_F32, MATH_TC_BF16X3, MATH_TC_BF16 = 0, 1, 2
 MAX_LAYERS = 8
 MAX_PATCHES = 4096
 MAX_CHANNELS = 1024
-ABI_VERSION = 5
+ABI_VERSION = 6
 LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
 
 EXPORTS = [
@@ -24,6 +24,7 @@ EXPORTS = [
     "pnce_diffaug_scratch_floats", "pnce_diffaug", "pnce_hinge_fwd", "pnce_hinge_bwd",
     "pnce_netf_workspace_bytes", "pnce_netf_fwd", "pnce_netf_bwd",
     "pnce_head_fwd_ex", "pnce_head_bwd_ex", "pnce_head_workspace_bytes", "pnce_head_fwd", "pnce_head_bwd", "pnce_head_bwd_params", "pnce_head_bwd_dense",
+    "pnce_mb_workspace_bytes", "pnce_mb_fwd", "pnce_rows_mb_workspace_bytes", "pnce_rows_mb_fwd_bwd",
 ]
 
 
@@ -99,6 +100,10 @@ def load():
     lib.pnce_rows_loss_fwd_bwd.argtypes = [vp, vp, i32, i32, i32, f32, i32, vp, sz, vp, vp, vp, vp, vp]
     lib.pnce_rows_loss_multi_workspace_bytes.argtypes = [ctypes.POINTER(PnceRows), i32, i32, ctypes.POINTER(sz)]
     lib.pnce_rows_loss_multi_fwd_bwd.argtypes = [ctypes.POINTER(PnceRows), i32, i32, f32, i32, vp, sz, vp, vp, vp]
+    lib.pnce_mb_workspace_bytes.argtypes = [ctypes.POINTER(PnceLayer), i32, i32, ctypes.POINTER(sz)]
+    lib.pnce_mb_fwd.argtypes = lib.pnce_fwd_ex.argtypes
+    lib.pnce_rows_mb_workspace_bytes.argtypes = lib.pnce_rows_loss_multi_workspace_bytes.argtypes
+    lib.pnce_rows_mb_fwd_bwd.argtypes = lib.pnce_rows_loss_multi_fwd_bwd.argtypes
     lib.pnce_head_workspace_bytes.argtypes = [ctypes.POINTER(PnceLayer), i32, i32, i32, ctypes.POINTER(sz)]
     lib.pnce_head_fwd.argtypes = [ctypes.POINTER(PnceLayer), ctypes.POINTER(PnceHead), i32, i32, i32, i32, f32, i32,
                                   vp, sz, vp, vp, vp]

@@ -64,6 +64,8 @@ struct Params {
                              // normalisation, no normalise backward), d loss / d q leaves row-major in dq_rows
   int nhwc;                  // channels-last maps (nhwc.cuh): src/tgt/dtgt are (B, HW, C) storage and dxT holds ROW-major
                              // rows [image][sorted slot][C]; tensor-core path only
+  int mb;                    // minibatch negatives (k_loss_tc_mb): each layer's B * P rows are ONE group (one CE mean,
+                             // one non-finite guard) instead of B images
   int b0, bn;                // images [b0, b0+bn) of the batch are covered by this launch (chunked forward)
   unsigned total_ctas;       // loss CTAs over all chunks: the one that arrives last finalises
   float* loss_out;           // [1 + n_layers]

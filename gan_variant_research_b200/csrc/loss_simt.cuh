@@ -37,6 +37,34 @@ __device__ void finalize_losses(const Params& p, void* scratch) {
     const LayerDev& L = p.L[l];
     float acc = 0.f;
     int nbad = 0;
+    if (p.mb) {
+      // minibatch negatives: the layer is one group of B * P rows -- mean over all of them, and the image guard
+      // (:97-99) applied to that single group: a non-finite group contributes 0 and all its rows are guarded
+      for (int b = tid; b < B; b += nthr)
+        for (int t = 0; t < L.nparts; ++t) acc += __ldcg(L.partial + (size_t)b * L.nparts + t);
+      acc = warp_sum(acc);
+      if (lane == 0) w_sum[warp] = acc;
+      __syncthreads();
+      if (tid == 0) {
+        float s = 0.f;
+        for (int w = 0; w < nwarp; ++w) s += w_sum[w];
+        const float sl = s / ((float)L.P * (float)B);
+        const int bad = isfinite(sl) ? 0 : 1;
+        layer_bad[l] = 0;                                       // guarded like an image: NaN rows keep their NaN
+        w_bad[0] = bad;
+        p.loss_out[1 + l] = bad ? 0.f : sl;
+        total += bad ? 0.f : sl;
+        bad_total += bad;                                       // nonfinite[0] counts guarded layers in this mode
+      }
+      __syncthreads();
+      const int bad = w_bad[0];
+      for (int b = tid; b < B; b += nthr) {
+        p.lossimg[l * B + b] = 0.f;
+        p.valid[l * B + b] = bad ? 0 : 1;
+      }
+      __syncthreads();
+      continue;
+    }
     for (int b = tid; b < B; b += nthr) {
       float s = 0.f;
       for (int t = 0; t < L.nparts; ++t) s += __ldcg(L.partial + (size_t)b * L.nparts + t);

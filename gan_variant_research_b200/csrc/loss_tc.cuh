@@ -411,9 +411,37 @@ __device__ __forceinline__ void tc_dq_epilogue(uint32_t tacc, int nstage, int C,
   }
 }
 
-__global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant__ Params p,
-                                                           const __grid_constant__ BlockMap m) {
-  pdl_launch();
+// 1/||k_j|| of the 256 keys [key0, key0 + 256) of image bk, folded from the gather's partial sums of squares (minibatch
+// mode: an item walks the keys of every image, so the weights are built per key block instead of once per image; 8 KB
+// of L2 reads per block next to the 64-256 KB of operand bytes the block streams).  A non-finite key raises badk.
+__device__ __forceinline__ float tc_mb_key_weight(const LayerDev& L, int bk, int key, int nstage) {
+  float ss = 0.f;
+  for (int s = 0; s < nstage; ++s) ss += __ldcg(L.kss + ((size_t)bk * nstage + s) * L.Ppad + key);
+  const float nrm = sqrtf(ss);
+  return (nrm == nrm) ? 1.0f / fmaxf(nrm, kNormEps) : nrm;      // NaN: the gather saw a non-finite element
+}
+__device__ __forceinline__ void tc_mb_key_weights(const LayerDev& L, int bk, int key0, int nstage, int et, float* invk_s,
+                                                  int* badk) {
+  asm volatile("bar.sync 1, 128;" ::: "memory");
+  for (int j = et; j < 256; j += 128) {
+    const int key = key0 + j;
+    float w = 0.f;
+    if (key < L.P) {
+      w = tc_mb_key_weight(L, bk, key, nstage);
+      if (!(w == w)) { *badk = 1; w = 0.f; }
+    }
+    invk_s[j] = w;
+  }
+  asm volatile("bar.sync 1, 128;" ::: "memory");
+}
+
+// MB = false: k_loss_tc, one image's P x P problem per item.  MB = true: k_loss_tc_mb (minibatch negatives): the item
+// (layer, image b, 128-row half) walks the key blocks (b', kb) of EVERY image of the batch -- the K blobs of the batch
+// are one key-blocked blob of B * Ppad keys, and the ids are shared, so the sorted-slot order is a common permutation of
+// all rows.  The item's own block (b, kb(row)) goes last, its diagonal chunks last.  Rows mode (p.rows_mode, MB only):
+// rows are used as given and d loss / d q leaves row-major in dq_rows.
+template <bool MB>
+__device__ __forceinline__ void loss_tc_body(const Params& p, const BlockMap& m) {
   extern __shared__ __align__(1024) unsigned char smem[];
   using namespace umma;
   unsigned char* stage0 = smem;
@@ -433,14 +461,18 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
   // keys are processed in blocks of <= 256 (the logits block must fit 256 TMEM columns next to the dQ
   // accumulator).  One block (P <= 256): Z is computed once.  More blocks: flash-style two passes --
   // pass 1 accumulates the row sums of exp2 block by block, pass 2 recomputes each Z block for dZ.
-  const int nkb = (Ppad + 255) >> 8;
+  // minibatch mode: nkb counts the blocks of every image, block g = image g / nkbi, block g % nkbi of that image
+  const int nkbi = (Ppad + 255) >> 8;
+  const int nkb = MB ? p.B * nkbi : nkbi;
   const bool multi = nkb > 1;
   const int nslots1 = multi ? 2 : kTcSlots1;                  // the dZ region is busy in pass 2 of the multi-block case
   const bool x3 = (p.math == PNCE_MATH_TC_BF16X3);
   // more than one key block and the +-50 clamp cannot bind (|cos| <= 1, every CUT temperature): ONE pass per block --
-  // exp2 once, unnormalised operand, no recomputation of the logits (the two-pass form stays for clamp-binding tau)
+  // exp2 once, unnormalised operand, no recomputation of the logits (the two-pass form stays for clamp-binding tau).
+  // Minibatch mode has no running maximum either: the row sum stays below N 2^(1.02 log2e / tau), finite in fp32 for
+  // N = B * Ppad <= 65536 at every tau where the clamp cannot bind.
   const bool single = multi && !((1.0f / p.tau) * 1.02f > kClamp);
-  const int kbd_item = (mh * 128) >> 8;                       // key block with the diagonals of this item's rows
+  const int kbd_item = (MB ? b * nkbi : 0) + ((mh * 128) >> 8);   // key block with the diagonals of this item's rows
   const int dlo_item = ((mh * 128) & 255) >> 5;               // and the first of its (up to four) diagonal chunks
   volatile int* dead = &sh->dead;
   long long* tr = nullptr;                                   // debug stamps (pnce_debug_set key 3)
@@ -481,16 +513,18 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
     if (lane == 0) {
       const unsigned char* gq_hi = reinterpret_cast<const unsigned char*>(L.qhi) + ((size_t)b * halves + mh) * Cp8 * 2048;
       const unsigned char* gq_lo = reinterpret_cast<const unsigned char*>(L.qlo) + ((size_t)b * halves + mh) * Cp8 * 2048;
-      const unsigned char* gk_hi = reinterpret_cast<const unsigned char*>(L.khi) + (size_t)b * Ppad * Cp * 2;
-      const unsigned char* gk_lo = reinterpret_cast<const unsigned char*>(L.klo) + (size_t)b * Ppad * Cp * 2;
-      const unsigned char* g2_hi = reinterpret_cast<const unsigned char*>(L.k2hi) + (size_t)b * Ppad * Cp * 2;
-      const unsigned char* g2_lo = reinterpret_cast<const unsigned char*>(L.k2lo) + (size_t)b * Ppad * Cp * 2;
       const uint32_t k2bytes = (uint32_t)Cp * 64u;            // 32 keys x Cp channels x 2 B
       uint32_t it1 = 0, it2 = 0, nz = 0;
       bool ok = true;
       for (int pass = 0; pass < npass && ok; ++pass) {
         for (int o = 0; o < nkb && ok; ++o) {
-          const int kb = single ? tc_block_at(o, nkb, kbd_item) : o;
+          const int g = single ? tc_block_at(o, nkb, kbd_item) : o;
+          const int bk = MB ? g / nkbi : b, kb = MB ? g % nkbi : g;     // image and block of the keys
+          const size_t kimg = (size_t)bk * Ppad * Cp * 2;
+          const unsigned char* gk_hi = reinterpret_cast<const unsigned char*>(L.khi) + kimg;
+          const unsigned char* gk_lo = reinterpret_cast<const unsigned char*>(L.klo) + kimg;
+          const unsigned char* g2_hi = reinterpret_cast<const unsigned char*>(L.k2hi) + kimg;
+          const unsigned char* g2_lo = reinterpret_cast<const unsigned char*>(L.k2lo) + kimg;
           const int NB = min(256, Ppad - kb * 256);           // keys of this block (128 or 256)
           const uint32_t kbytes = (uint32_t)NB * 64u;         // one K chunk: 4 slabs x NB/8 core matrices x 128 B
           const size_t kblk = (size_t)kb * 256 * Cp * 2;      // blocks are stored one after the other
@@ -540,13 +574,14 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
       PNCE_TR(8);
       for (int pass = 0; pass < npass && ok; ++pass) {
         for (int o = 0; o < nkb && ok; ++o) {
-          const int kb = single ? tc_block_at(o, nkb, kbd_item) : o;
+          const int g = single ? tc_block_at(o, nkb, kbd_item) : o;
+          const int kb = MB ? g % nkbi : g;
           const int NB = min(256, Ppad - kb * 256);
           const uint32_t idesc1 = idesc_bf16(128, NB, 0, 0);
           const uint32_t lbo_k = (uint32_t)NB * 16u;          // slab (c/8) stride of a K chunk in smem
           // the previous Z block must have been read out of TMEM.  Pass 1 of two: the epilogue says so (zfree);
           // pass 2 / single pass, block > 0: implied by having consumed every dzready of the previous block.
-          if (multi && !single && nz > 0 && (pass == 0 || kb == 0)) ok = mbar_wait(&sh->zfree, (nz - 1) & 1u, dead);
+          if (multi && !single && nz > 0 && (pass == 0 || o == 0)) ok = mbar_wait(&sh->zfree, (nz - 1) & 1u, dead);
           // ---- Z block = Q_half K_block^T ----
           for (int s = 0; s < nstage && ok; ++s, ++it1) {
             const int slot = it1 % nslots1;
@@ -622,7 +657,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
       for (int s = 0; s < 8; ++s)
         ssq[s] = (s < nstage && rowok) ? __ldcg(L.qss + ((size_t)b * nstage + s) * Ppad + gi) : 0.f;
       bool anybad = false;
-      for (int j = et; j < Ppad; j += 128) {
+      for (int j = et; j < (MB ? 0 : Ppad); j += 128) {       // minibatch mode: per key block (tc_mb_key_weights)
         float ssk[8];
 #pragma unroll
         for (int s = 0; s < 8; ++s)
@@ -642,17 +677,17 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
 #pragma unroll
       for (int s = 0; s < 8; ++s) ss += ssq[s];
       rownrm = sqrtf(ss);
-      if (rowok)
+      if (rowok && (!MB || L.qinv != nullptr))                 // rows mode carves no qinv
         L.qinv[(size_t)b * P + gi] =
             (rownrm == rownrm) ? (rownrm < kNormEps ? -1.0f / kNormEps : 1.0f / rownrm) : rownrm;
     }
-    if (multi) __threadfence_block();
+    if (!MB && multi) __threadfence_block();
     asm volatile("bar.sync 1, 128;" ::: "memory");            // publishes invk_s (block 0), kinv and badk
     {
       const bool badq = rowok && !(rownrm == rownrm);
       const float sc = (rowok && !badq) ? 1.0f / fmaxf(rownrm, kNormEps) : 0.f;     // 1 / max(||q_i||, eps)
       const bool noproj = rownrm < kNormEps;
-      const bool badrow = badq || (sh->badk != 0);
+      bool badrow = badq || (sh->badk != 0);                  // minibatch mode: re-read once every key block was seen
 
       const float inv_tau = 1.0f / p.tau;
       const float a = sc * inv_tau * kLog2e;                  // acc -> logit in log2 units (times 1/||k_j||)
@@ -675,6 +710,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
       dg.pass = true;
       dg.d_w = 0.f;
       dg.off = (uint32_t)((gi & 255) >> 3) * 2048u + rowoff + (uint32_t)(gi & 7) * 2u;
+      const int kbd_row = (MB ? b * nkbi : 0) + kbd;          // the same as a global block index
+      auto mb_weights = [&](int g) { tc_mb_key_weights(L, g / nkbi, (g % nkbi) * 256, nstage, et, invk_s, &sh->badk); };
       if (single) {
         // ---- ONE pass per key block (P > 256, clamp cannot bind): exp2 once, unnormalised operand, dQ' += E_blk K_blk;
         //      row sums alongside; the block with this item's diagonals last, its diagonal chunks last and released
@@ -683,11 +720,14 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
         float s2 = 0.f, ydacc = 0.f;
         bool own_deferred = false;
         for (int o = 0; o < nkb; ++o) {
-          const int kb = tc_block_at(o, nkb, kbd_item);
+          const int g = tc_block_at(o, nkb, kbd_item);
+          const int kb = MB ? g % nkbi : g;
           const int key0 = kb * 256, keys = min(P, key0 + 256) - key0;
           const int nch = (keys + 31) >> 5;                     // chunks that hold real columns
           const bool lastblk = o == nkb - 1;
-          if (o > 0 || kb != 0) {                                // swap in this block's 1/||k_j|| (the prologue left block 0's)
+          if (MB) {
+            mb_weights(g);
+          } else if (o > 0 || kb != 0) {                         // swap in this block's 1/||k_j|| (the prologue left block 0's)
             asm volatile("bar.sync 1, 128;" ::: "memory");
             for (int j = et; j < 256; j += 128) invk_s[j] = (key0 + j < Ppad) ? __ldcg(L.kinv + (size_t)b * Ppad + key0 + j) : 0.f;
             asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -701,7 +741,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
             tc_q_load(qa, qh, ql, 0, nstage);
             tc_q_load(qb, qh, ql, 1, nstage);
           }
-          const int cd = (kb == kbd) ? chd : -1;
+          const int cd = (g == kbd_row) ? chd : -1;
           uint32_t r0[32], r1[32];
           tmem_ld32(trow + (lastblk ? tc_chunk_last(0, nch, dlo_item) : 0) * 32, r0);
           for (int k = 0; k < nch; k += 2) {
@@ -731,10 +771,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
             }
           }
         }
-        const float wd = __ldcg(L.kinv + (size_t)b * Ppad + (rowok ? gi : 0));
+        const float wd = MB ? fmaxf(tc_mb_key_weight(L, b, rowok ? gi : 0, nstage), 0.f) : __ldcg(L.kinv + (size_t)b * Ppad + (rowok ? gi : 0));
         const float ydr = ydacc * a * wd;                       // diagonal logit (log2 units)
         const float se = (se4[0] + se4[1]) + (se4[2] + se4[3]);
         const float lse2 = lg2f(se);
+        if (MB) badrow = badq || (sh->badk != 0);
         rowloss = rowok ? (lse2 - ydr) * kLn2 : 0.f;            // :94, labels = arange
         if (badrow && rowok) rowloss = __int_as_float(0x7fc00000);
         PNCE_TR(3);
@@ -752,11 +793,14 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
         // ---- pass A: row sum of exp2 over all key blocks, diagonal ----
         float se4[4] = {0.f, 0.f, 0.f, 0.f};
         float ydacc = 0.f;                                      // raw accumulator of the diagonal element
-        for (int kb = 0; kb < nkb; ++kb) {
+        for (int g = 0; g < nkb; ++g) {
+          const int kb = MB ? g % nkbi : g;
           const int key0 = kb * 256, keys = min(P, key0 + 256) - key0;
           const int nch = (keys + 31) >> 5;                     // chunks that hold real columns
           const bool pad = (nch * 32 != keys);                  // the block's last chunk holds padding columns
-          if (kb > 0) {                                          // swap in this block's 1/||k_j||
+          if (MB) {
+            mb_weights(g);
+          } else if (kb > 0) {                                   // swap in this block's 1/||k_j||
             asm volatile("bar.sync 1, 128;" ::: "memory");
             for (int j = et; j < 256; j += 128) invk_s[j] = (key0 + j < Ppad) ? __ldcg(L.kinv + (size_t)b * Ppad + key0 + j) : 0.f;
             asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -764,8 +808,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
           mbar_wait(&sh->zfull, nz & 1u, dead);
           ++nz;
           tc_fence_after();
-          if (kb == 0) PNCE_TR(2);
-          const int cd = (kb == kbd) ? chd : -1;
+          if (g == 0) PNCE_TR(2);
+          const int cd = (g == kbd_row) ? chd : -1;
           if (need_clamp) tc_row_pass_a<true>(trow, nch, invk_s, a, cl, cd, lane, se4, ydacc, pad);
           else tc_row_pass_a<false>(trow, nch, invk_s, a, cl, cd, lane, se4, ydacc, pad);
           if (multi) {
@@ -773,11 +817,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
             mbar_arrive(&sh->zfree);                             // this Z block may be overwritten
           }
         }
-        const float wd = multi ? __ldcg(L.kinv + (size_t)b * Ppad + (rowok ? gi : 0)) : invk_s[gi];
+        const float wd = MB ? fmaxf(tc_mb_key_weight(L, b, rowok ? gi : 0, nstage), 0.f) : multi ? __ldcg(L.kinv + (size_t)b * Ppad + (rowok ? gi : 0)) : invk_s[gi];
         const float ydr = ydacc * a * wd;                       // unclamped diagonal logit (log2 units)
         const float yd = need_clamp ? fminf(fmaxf(ydr, -cl), cl) : ydr;
         const float se = (se4[0] + se4[1]) + (se4[2] + se4[3]);   // padding columns were masked out in pass A
         const float lse2 = lg2f(se);
+        if (MB) badrow = badq || (sh->badk != 0);
         rowloss = rowok ? (lse2 - yd) * kLn2 : 0.f;              // :94, labels = arange
         if (badrow && rowok) rowloss = __int_as_float(0x7fc00000);
         PNCE_TR(3);
@@ -790,20 +835,25 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
         float s2 = 0.f;
         dg.pass = !need_clamp || fabsf(ydr) <= cl;
         dg.d_w = dg.pass ? (ex2f(yd - lse2) - 1.f) * coef * wd : 0.f;
-        for (int kb = 0; kb < nkb; ++kb) {
+        for (int g = 0; g < nkb; ++g) {
+          const int kb = MB ? g % nkbi : g;
           const int key0 = kb * 256, keys = min(P, key0 + 256) - key0;
           const int nch = (keys + 31) >> 5;
           if (multi) {
             // this block's 1/||k_j||; the Z block is recomputed by the MMA thread (pass 2).  zfull of this
             // block also means the previous block's dQ MMAs have finished reading the dZ operand.
-            asm volatile("bar.sync 1, 128;" ::: "memory");
-            for (int j = et; j < 256; j += 128) invk_s[j] = (key0 + j < Ppad) ? __ldcg(L.kinv + (size_t)b * Ppad + key0 + j) : 0.f;
-            asm volatile("bar.sync 1, 128;" ::: "memory");
+            if (MB) {
+              mb_weights(g);
+            } else {
+              asm volatile("bar.sync 1, 128;" ::: "memory");
+              for (int j = et; j < 256; j += 128) invk_s[j] = (key0 + j < Ppad) ? __ldcg(L.kinv + (size_t)b * Ppad + key0 + j) : 0.f;
+              asm volatile("bar.sync 1, 128;" ::: "memory");
+            }
             mbar_wait(&sh->zfull, nz & 1u, dead);
             ++nz;
             tc_fence_after();
           }
-          const int cd = (kb == kbd) ? chd : -1;
+          const int cd = (g == kbd_row) ? chd : -1;
           uint64_t* dzr = sh->dzready;
           if (need_clamp) tc_row_pass_b<true>(trow, nch, invk_s, a, cl, lse2, coef, x3, dzhi, dzlo, rowoff, cd, dg, dzr, s2);
           else tc_row_pass_b<false>(trow, nch, invk_s, a, cl, lse2, coef, x3, dzhi, dzlo, rowoff, cd, dg, dzr, s2);
@@ -829,7 +879,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
       // head mode: d loss / d (head output) as a row blob [tile = b*halves+mh][c/8][16][8][8]
       __nv_bfloat16* dyh = L.dyhi ? L.dyhi + qoff : nullptr;
       __nv_bfloat16* dyl = (L.dyhi && L.dylo) ? L.dylo + qoff : nullptr;
-      if (p.nhwc) tc_dq_epilogue<0>(trow + 256u, nstage, C, qh, ql, dxrow, c1, c2, rowok, dyh, dyl, &sh->dqfull, dead, qa, qb, C, 0u, true);
+      // rows mode (minibatch only): rows used as given -- no normalise backward (c2 = 0), d loss / d q row-major in the
+      // caller's row order
+      const bool rows = MB && p.rows_mode;
+      if (rows) dxrow = L.dq_rows + ((size_t)b * P + (rowok ? gi : 0)) * C;
+      if (p.nhwc || rows) tc_dq_epilogue<0>(trow + 256u, nstage, C, qh, ql, dxrow, c1, rows ? 0.f : c2, rowok, dyh, dyl, &sh->dqfull, dead, qa, qb, C, 0u, true);
       else switch (Ppad >> 7) {
         case 1: tc_dq_epilogue<128>(trow + 256u, nstage, C, qh, ql, dxrow, c1, c2, rowok, dyh, dyl, &sh->dqfull, dead, qa, qb); break;
         case 2: tc_dq_epilogue<256>(trow + 256u, nstage, C, qh, ql, dxrow, c1, c2, rowok, dyh, dyl, &sh->dqfull, dead, qa, qb); break;
@@ -854,6 +908,18 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant
     p.trace[64 + 3 * (size_t)blockIdx.x + 2] = (long long)t;
   }
   last_cta_finalize(p, &sh->flag, smem);                       // every CTA-wide phase is over (the __syncthreads above): the ring is free scratch
+}
+
+__global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant__ Params p,
+                                                           const __grid_constant__ BlockMap m) {
+  pdl_launch();
+  loss_tc_body<false>(p, m);
+}
+
+__global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc_mb(const __grid_constant__ Params p,
+                                                              const __grid_constant__ BlockMap m) {
+  pdl_launch();
+  loss_tc_body<true>(p, m);
 }
 
 // -------------------------------------------------------------------------------------------------

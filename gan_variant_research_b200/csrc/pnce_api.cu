@@ -70,6 +70,17 @@ static bool tc_shapes_ok(const pnce_layer_t* layers, int n_layers) {
   return true;
 }
 
+// minibatch negatives: the tensor-core envelope, and at most 65536 keys (B * Ppad) per layer -- the bound under which the
+// single-pass row sum (no running maximum) stays finite in fp32
+static constexpr long long kMbMaxKeys = 65536;
+static bool mb_keys_ok(int B, int P) { return (long long)B * ((P + 127) / 128 * 128) <= kMbMaxKeys; }
+static bool mb_shapes_ok(const pnce_layer_t* layers, int n_layers, int B) {
+  if (!tc_shapes_ok(layers, n_layers)) return false;
+  for (int l = 0; l < n_layers; ++l)
+    if (!mb_keys_ok(B, layers[l].P)) return false;
+  return true;
+}
+
 // Fills Params (pointers into the workspace) for the fused path; returns bytes used.
 // tc = carve the tensor-core operand blobs instead of the fp32 normalised rows.
 // The id bookkeeping of every layer (k_prep's outputs): sid, perm, rank, cslot.  It lives at the head of the
@@ -414,6 +425,13 @@ static int launch_loss_tc(const Params& p, cudaStream_t st, bool single_launch =
   }
   m.start[p.n_layers] = acc;
   if (acc > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
+  if (p.mb) {                                                  // minibatch negatives: one CTA per item, every key block
+    int rc = set_smem(k_loss_tc_mb, kTcSmemBytes);
+    if (rc != PNCE_OK) return rc;
+    launch_k<4>(k_loss_tc_mb, (unsigned)acc, kTcThreads, kTcSmemBytes, st, p, m);
+    PNCE_CUDA(cudaGetLastError());
+    return PNCE_OK;
+  }
   // P <= 256 everywhere (one key block per item): persistent kernel, one CTA per SM walking the item list
   bool persist = single_launch && !g_dbg.no_persist;
   for (int l = 0; l < p.n_layers; ++l)
@@ -486,7 +504,7 @@ static int forward_tc(Params& p, cudaStream_t st, bool planned = false) {
   int rc = PNCE_OK;
   // planned: pnce_plan_ids has run k_prep already (gather CTA 0 resets the counter); small problems: the gather CTAs
   // sort the ids themselves (k_gather_tc_fold), no k_prep launch
-  const bool fold = !planned && g_dbg.fwd_chunks <= 1 && gather_tc_folds(p);
+  const bool fold = !planned && (g_dbg.fwd_chunks <= 1 || p.mb) && gather_tc_folds(p);
   if (!planned && !fold) rc = launch_prep(p, st);
   if (rc != PNCE_OK) return rc;
   int ctas_per_image = 0;
@@ -494,7 +512,7 @@ static int forward_tc(Params& p, cudaStream_t st, bool planned = false) {
   // Chunking is OFF by default: on B200 the 14-image chunks that fill the SMs once make the gather
   // pay ~30% wave quantisation and the overlap does not win it back (measured: 0.70 ms vs 0.50 ms
   // forward at B=64).  Kept behind the debug knob for larger batches.
-  int nchunk = g_dbg.fwd_chunks > 1 ? g_dbg.fwd_chunks : 1;
+  int nchunk = (g_dbg.fwd_chunks > 1 && !p.mb) ? g_dbg.fwd_chunks : 1;   // an mb item needs the keys of every image
   if (nchunk > 16) nchunk = 16;
   if (nchunk > p.B) nchunk = p.B;
   int per = (p.B + nchunk - 1) / nchunk;
@@ -756,7 +774,8 @@ int pnce_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch, si
 
 static int fwd_impl(const pnce_layer_t* layers, int n_layers, int batch, int dtype, float temperature,
                     int math_mode, void* ws, size_t ws_bytes, void* plan, size_t plan_bytes, float* loss_out,
-                    int* nonfinite, void* stream, const unsigned long long* rng = nullptr, int layout = PNCE_LAYOUT_NCHW) {
+                    int* nonfinite, void* stream, const unsigned long long* rng = nullptr, int layout = PNCE_LAYOUT_NCHW,
+                    bool mb = false) {
   int rc = check_layers(layers, n_layers, batch);
   if (layout != PNCE_LAYOUT_NCHW && layout != PNCE_LAYOUT_NHWC) return PNCE_ERR_ARG;
   if (rc != PNCE_OK) return rc;
@@ -769,6 +788,7 @@ static int fwd_impl(const pnce_layer_t* layers, int n_layers, int batch, int dty
   // fp32 CUDA-core kernel -- both are device paths of this library, neither is a fallback off the GPU
   const bool tc = math_mode != PNCE_MATH_SIMT_F32 && tc_shapes_ok(layers, n_layers);
   const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
+  if (mb && (!tc || !mb_shapes_ok(layers, n_layers, batch))) return PNCE_ERR_UNSUPPORTED;
   if (plan != nullptr) {
     if (!tc) return PNCE_ERR_UNSUPPORTED;                      // planned ids: tensor-core path only
     if ((reinterpret_cast<uintptr_t>(plan) & 255u) || carve_plan(layers, n_layers, nullptr, nullptr) > plan_bytes)
@@ -783,6 +803,7 @@ static int fwd_impl(const pnce_layer_t* layers, int n_layers, int batch, int dty
   p.nonfinite = nonfinite;
   p.trace = g_dbg.trace;
   p.b0 = 0; p.bn = batch;
+  p.mb = mb ? 1 : 0;
   if (layout == PNCE_LAYOUT_NHWC) {
     if (!tc) return PNCE_ERR_UNSUPPORTED;                      // channels-last maps: tensor-core path only
     p.nhwc = 1;
@@ -938,6 +959,27 @@ int pnce_bwd_planned(const pnce_layer_t* layers, int n_layers, int batch, int dt
                      size_t ws_bytes, void* plan, size_t plan_bytes, const float* grad_out, void* stream) {
   if (plan == nullptr) return PNCE_ERR_ARG;
   return bwd_impl(layers, n_layers, batch, dtype, math_mode, ws, ws_bytes, plan, plan_bytes, grad_out, stream);
+}
+
+// ---- minibatch negatives (nce_includes_all_negatives_from_minibatch) ----------------------------------------------
+int pnce_mb_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch, size_t* bytes) {
+  if (bytes == nullptr) return PNCE_ERR_ARG;
+  int rc = check_layers(layers, n_layers, batch);
+  if (rc != PNCE_OK) return rc;
+  if (!mb_shapes_ok(layers, n_layers, batch)) return PNCE_ERR_UNSUPPORTED;
+  *bytes = carve_fused(layers, n_layers, batch, true, true, nullptr, nullptr);
+  return PNCE_OK;
+}
+
+int pnce_mb_fwd(const pnce_layer_t* layers, int n_layers, int batch, int dtype, int layout, float temperature,
+                int math_mode, void* ws, size_t ws_bytes, void* plan, size_t plan_bytes,
+                const unsigned long long* philox, float* loss_out, int* nonfinite, void* stream) {
+  if (math_mode == PNCE_MATH_SIMT_F32) return PNCE_ERR_UNSUPPORTED;
+  const int rc = check_layers(layers, n_layers, batch);
+  if (rc != PNCE_OK) return rc;
+  if (!mb_shapes_ok(layers, n_layers, batch)) return PNCE_ERR_UNSUPPORTED;
+  return fwd_impl(layers, n_layers, batch, dtype, temperature, math_mode, ws, ws_bytes, plan, plan_bytes, loss_out,
+                  nonfinite, stream, philox, layout, true);
 }
 
 // ---- module-split API ------------------------------------------------------------------------
@@ -1330,6 +1372,59 @@ int pnce_rows_loss_multi_fwd_bwd(const pnce_rows_t* rows, int n_layers, int batc
   t.loss_out = loss_out;
   t.nonfinite = nonfinite;
   t.b0 = 0; t.bn = batch;
+  PNCE_CUDA(cudaMemsetAsync(t.counter, 0, 2 * sizeof(unsigned), st));
+  long long most = 0;
+  for (int l = 0; l < n_layers; ++l) {
+    const long long threads = 2ll * batch * t.L[l].Ppad * (t.L[l].Cp >> 3);
+    if (threads > most) most = threads;
+  }
+  const dim3 grid((unsigned)((most + kThreads - 1) / kThreads), (unsigned)n_layers);
+  launch_k(k_rows_pack, grid, kThreads, 0, st, t);
+  PNCE_CUDA(cudaGetLastError());
+  return launch_loss_tc(t, st);
+}
+
+static int check_rows_mb(const pnce_rows_t* rows, int n, int batch) {
+  if (rows == nullptr || n < 1 || n > PNCE_MAX_LAYERS || batch < 1) return PNCE_ERR_ARG;
+  for (int l = 0; l < n; ++l) {
+    if (rows[l].P < 1 || rows[l].D < 1) return PNCE_ERR_ARG;
+    if (!rows_tc_ok(rows[l].P, rows[l].D) || !mb_keys_ok(batch, rows[l].P)) return PNCE_ERR_UNSUPPORTED;
+  }
+  return PNCE_OK;
+}
+
+int pnce_rows_mb_workspace_bytes(const pnce_rows_t* rows, int n_layers, int batch, size_t* bytes) {
+  if (bytes == nullptr) return PNCE_ERR_ARG;
+  int rc = check_rows_mb(rows, n_layers, batch);
+  if (rc != PNCE_OK) return rc;
+  *bytes = carve_rows_multi_tc(rows, n_layers, batch, true, nullptr, nullptr);
+  return PNCE_OK;
+}
+
+int pnce_rows_mb_fwd_bwd(const pnce_rows_t* rows, int n_layers, int batch, float temperature, int math_mode,
+                         void* ws, size_t ws_bytes, float* loss_out, int* nonfinite, void* stream) {
+  using namespace pnce;
+  int rc = check_rows_mb(rows, n_layers, batch);
+  if (rc != PNCE_OK) return rc;
+  if (!loss_out || !(temperature > 0.f)) return PNCE_ERR_ARG;
+  if (math_mode != PNCE_MATH_TC_BF16X3 && math_mode != PNCE_MATH_TC_BF16) return PNCE_ERR_UNSUPPORTED;
+  if (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 255u)) return PNCE_ERR_WORKSPACE;
+  for (int l = 0; l < n_layers; ++l) {
+    if (!rows[l].q || !rows[l].k || !rows[l].dq) return PNCE_ERR_ARG;
+    if (reinterpret_cast<uintptr_t>(rows[l].dq) & 31u) return PNCE_ERR_ALIGN;   // 32-byte row stores (k_loss_tc_mb)
+  }
+  static thread_local Params t;
+  if (carve_rows_multi_tc(rows, n_layers, batch, math_mode == PNCE_MATH_TC_BF16X3, ws, &t) > ws_bytes)
+    return PNCE_ERR_WORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  t.math = math_mode;
+  t.tau = temperature;
+  t.loss_out = loss_out;
+  t.nonfinite = nonfinite;
+  t.b0 = 0; t.bn = batch;
+  t.mb = 1;
+  t.total_ctas = 0;
+  for (int l = 0; l < n_layers; ++l) t.total_ctas += (unsigned)(batch * (t.L[l].Ppad / 128));
   PNCE_CUDA(cudaMemsetAsync(t.counter, 0, 2 * sizeof(unsigned), st));
   long long most = 0;
   for (int l = 0; l < n_layers; ++l) {

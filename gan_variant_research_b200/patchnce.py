@@ -242,11 +242,13 @@ class _WarnQueue:
         self.host = None
         self.words = None            # numpy view of the pinned buffer: plain loads and stores, no tensor indexing
         self.free = []
+        self.mb = [False] * self.SLOTS       # slot -> minibatch-negatives launch (the count is of layers)
         self.lock = threading.Lock()
 
-    def acquire(self):
+    def acquire(self, mb: bool = False):
         """-> (slot, device-usable pointer to int32[2]) or (None, 0) while a CUDA graph is being captured
-        (then the failure of a launch shows in-band: the loss is NaN, include/pnce.h)."""
+        (then the failure of a launch shows in-band: the loss is NaN, include/pnce.h).  ``mb``: a minibatch-negatives
+        launch, whose count is of guarded layers."""
         if torch.cuda.is_current_stream_capturing():
             return None, 0
         with self.lock:
@@ -261,6 +263,7 @@ class _WarnQueue:
                     torch.cuda.synchronize()
                     self._poll(True)
             slot = self.free.pop()
+            self.mb[slot] = mb
             self.words[slot, 0] = -1                 # "in flight"; word 1 is cleared by the sequence's first kernel
             self.words[slot, 1] = 0
             self.pending.append(slot)
@@ -286,7 +289,11 @@ class _WarnQueue:
                 self.free.append(slot)
                 proto_err = proto_err or bool(w[slot, 1])
                 if n > 0:
-                    print(f"Warning: NaN in PatchNCE loss. {n} (layer, image) loss(es) replaced by 0.")
+                    if self.mb[slot]:
+                        for _ in range(n):
+                            print("Warning: NaN in PatchNCE loss (minibatch negatives). A layer's loss replaced by 0.")
+                    else:
+                        print(f"Warning: NaN in PatchNCE loss. {n} (layer, image) loss(es) replaced by 0.")
                     total += n
             else:
                 keep.append(slot)
@@ -328,10 +335,14 @@ class _ShapePlan:
     guarded by a lock so that two Python threads sharing a shape do not interleave their pointer stores."""
 
     __slots__ = ("n", "batch", "dtype", "dtype_code", "math", "math_code", "dev", "p_list", "p_total", "tc",
-                 "ws_bytes", "plan_bytes", "fwd_layers", "bwd_layers", "fwd_lock", "bwd_lock", "big", "shapes", "nhwc")
+                 "ws_bytes", "plan_bytes", "fwd_layers", "bwd_layers", "fwd_lock", "bwd_lock", "big", "shapes", "nhwc",
+                 "mb")
 
-    def __init__(self, dev, dtype, shapes, p_list, math, nhwc=False):
+    def __init__(self, dev, dtype, shapes, p_list, math, nhwc=False, mb=False):
+        if mb:
+            mb_check(shapes[0][0], [s[1] for s in shapes], p_list, math)
         lib = _lib.load()
+        self.mb = mb                             # minibatch negatives (pnce_mb_fwd)
         self.n, self.batch, self.dtype, self.dev, self.math = len(shapes), shapes[0][0], dtype, dev, math
         self.nhwc = nhwc                         # channels-last storage (pnce_fwd_ex / pnce_bwd_ex, LAYOUT_NHWC)
         self.dtype_code, self.math_code = _DTYPES[dtype], _MATH[math]
@@ -343,8 +354,12 @@ class _ShapePlan:
             for l, ((_, c, h, w), p) in enumerate(zip(shapes, p_list)):
                 arr[l].C, arr[l].H, arr[l].W, arr[l].P = c, h, w, p
         nbytes = ctypes.c_size_t(0)
-        _lib.check(lib.pnce_workspace_bytes(self.fwd_layers, self.n, self.batch, ctypes.byref(nbytes)),
-                   "pnce_workspace_bytes")
+        if mb:
+            _lib.check(lib.pnce_mb_workspace_bytes(self.fwd_layers, self.n, self.batch, ctypes.byref(nbytes)),
+                       "pnce_mb_workspace_bytes")
+        else:
+            _lib.check(lib.pnce_workspace_bytes(self.fwd_layers, self.n, self.batch, ctypes.byref(nbytes)),
+                       "pnce_workspace_bytes")
         self.ws_bytes = nbytes.value
         # the tensor-core kernels' envelope (csrc/pnce_api.cu tc_shapes_ok); outside it the fp32 CUDA-core kernels run
         self.tc = tc_envelope(shapes, p_list, math)
@@ -369,19 +384,39 @@ def tc_envelope(shapes, p_list, math) -> bool:
     return math != "simt_f32" and all(s[1] <= 256 and p <= 1024 for s, p in zip(shapes, p_list))
 
 
+MB_MAX_KEYS = 65536      # keys (B * round_up(P, 128)) per layer of the minibatch-negatives kernel (include/pnce.h)
+
+
+def mb_check(batch, channels, p_list, math, rows=False):
+    """The envelope of minibatch negatives (``nce_includes_all_negatives_from_minibatch``): tensor-core math, C <= 256,
+    P <= 1024 per image (P <= 256 on the row route) and B * round_up(P, 128) <= 65536 per layer.  Raises RuntimeError
+    outside it: there is no other implementation of this mode to fall back to."""
+    if math == "simt_f32":
+        raise RuntimeError("nce_includes_all_negatives_from_minibatch needs a tensor-core math mode (tc_bf16x3 or tc_bf16), "
+                           "not simt_f32")
+    pmax = 256 if rows else 1024
+    for c, p in zip(channels, p_list):
+        if c > 256 or p > pmax:
+            raise RuntimeError(f"nce_includes_all_negatives_from_minibatch supports C <= 256 and P <= {pmax} per layer "
+                               f"(got C={c}, P={p})")
+        if batch * ((p + 127) // 128 * 128) > MB_MAX_KEYS:
+            raise RuntimeError(f"nce_includes_all_negatives_from_minibatch supports at most {MB_MAX_KEYS} keys per layer "
+                               f"(batch * round_up(P, 128)); got batch={batch}, P={p}")
+
+
 def _is_nhwc(t) -> bool:
     """(B, C, H, W) tensor whose storage is dense (B, H, W, C): torch.channels_last (and not also plain contiguous)."""
     return t.dim() == 4 and not t.is_contiguous() and t.is_contiguous(memory_format=torch.channels_last)
 
 
-def _shape_plan(tgt, p_list, math, nhwc=False) -> _ShapePlan:
+def _shape_plan(tgt, p_list, math, nhwc=False, mb=False) -> _ShapePlan:
     t0 = tgt[0]
-    key = (t0.device.index, t0.dtype, math, nhwc, tuple(p_list), *[t.shape for t in tgt])
+    key = (t0.device.index, t0.dtype, math, nhwc, mb, tuple(p_list), *[t.shape for t in tgt])
     sp = _SHAPE_PLANS.get(key)
     if sp is None:
         if len(_SHAPE_PLANS) > 256:                  # a caller cycling through many shapes: do not grow without bound
             _SHAPE_PLANS.clear()
-        sp = _SHAPE_PLANS[key] = _ShapePlan(t0.device, t0.dtype, [tuple(t.shape) for t in tgt], p_list, math, nhwc)
+        sp = _SHAPE_PLANS[key] = _ShapePlan(t0.device, t0.dtype, [tuple(t.shape) for t in tgt], p_list, math, nhwc, mb)
     return sp
 
 
@@ -443,7 +478,7 @@ def _run_fwd(call: _Call, tgt_feats):
     with _on_device(dev):
         ws = torch.empty(sp.ws_bytes, dtype=torch.uint8, device=dev)
         out = torch.empty(1 + n, dtype=torch.float32, device=dev)
-        slot, flag_ptr = _warn_queue(dev).acquire()           # both words are written by the kernels
+        slot, flag_ptr = _warn_queue(dev).acquire(sp.mb)      # both words are written by the kernels
         st = _stream_ptr(dev)
         src, ids = call.src, call.ids
         with sp.fwd_lock:
@@ -451,7 +486,14 @@ def _run_fwd(call: _Call, tgt_feats):
             for l in range(n):
                 a = layers[l]
                 a.src, a.tgt, a.ids = src[l].data_ptr(), tgt_feats[l].data_ptr(), ids[l].data_ptr()
-            if sp.nhwc:
+            if sp.mb:
+                philox = (ctypes.c_ulonglong * 2)(call.rng[0], call.rng[1]) if call.rng is not None else None
+                pl = call.idplan
+                rc = lib.pnce_mb_fwd(layers, n, sp.batch, sp.dtype_code, _lib.LAYOUT_NHWC if sp.nhwc else _lib.LAYOUT_NCHW,
+                                     call.temperature, sp.math_code, ws.data_ptr(), sp.ws_bytes,
+                                     pl.data_ptr() if pl is not None else None, pl.numel() if pl is not None else 0, philox,
+                                     out.data_ptr(), flag_ptr or None, st)
+            elif sp.nhwc:
                 philox = (ctypes.c_ulonglong * 2)(call.rng[0], call.rng[1]) if call.rng is not None else None
                 pl = call.idplan
                 rc = lib.pnce_fwd_ex(layers, n, sp.batch, sp.dtype_code, _lib.LAYOUT_NHWC, call.temperature,
@@ -550,9 +592,10 @@ def _run_bwd(call: _Call, ws, grad_out, tgt_like):
             for l in range(sp.n):
                 layers[l].dtgt, layers[l].ids = grads[l].data_ptr(), ids[l].data_ptr()
             gp = g.data_ptr() if g is not None else None
-            if sp.nhwc:
+            if sp.nhwc or sp.mb:
                 pl = call.idplan
-                rc = lib.pnce_bwd_ex(layers, sp.n, sp.batch, sp.dtype_code, _lib.LAYOUT_NHWC, sp.math_code,
+                rc = lib.pnce_bwd_ex(layers, sp.n, sp.batch, sp.dtype_code,
+                                     _lib.LAYOUT_NHWC if sp.nhwc else _lib.LAYOUT_NCHW, sp.math_code,
                                      ws.data_ptr(), sp.ws_bytes, pl.data_ptr() if pl is not None else None,
                                      pl.numel() if pl is not None else 0, gp, st)
             elif call.idplan is None:
@@ -646,15 +689,17 @@ def _prepare_maps(src_feats, tgt_feats, math=None, patches=None):
     return src, tgt, n_src, uniform
 
 
-def _fused_call(src, tgt, ids, temperature, math, rng=None, idplan=None):
-    sp = _shape_plan(tgt, [i.numel() for i in ids], math, _is_nhwc(tgt[0]))
+def _fused_call(src, tgt, ids, temperature, math, rng=None, idplan=None, mb=False):
+    sp = _shape_plan(tgt, [i.numel() for i in ids], math, _is_nhwc(tgt[0]), mb and tgt[0].shape[0] > 1)
     return _FusedPatchNCE.apply(_Call(sp, src, ids, temperature, rng, idplan), *tgt)
 
 
 def fused_patchnce(src_feats, tgt_feats, ids_list, temperature=0.07, math: Optional[str] = None,
-                   denom_layers: Optional[int] = None):
+                   denom_layers: Optional[int] = None, nce_includes_all_negatives_from_minibatch: bool = False):
     """All-layer PatchNCE on dense NCHW maps with given ids.  Returns the scalar loss tensor
-    (fp32, on device, differentiable w.r.t. every ``tgt_feats[l]`` that requires grad)."""
+    (fp32, on device, differentiable w.r.t. every ``tgt_feats[l]`` that requires grad).
+    ``nce_includes_all_negatives_from_minibatch``: see ``PatchNCELoss``."""
+    mb = bool(nce_includes_all_negatives_from_minibatch)
     math = math or DEFAULT_MATH
     if len(ids_list) < min(len(src_feats), len(tgt_feats)):
         raise RuntimeError(f"{len(ids_list)} id tensors for {min(len(src_feats), len(tgt_feats))} layers")
@@ -670,10 +715,10 @@ def fused_patchnce(src_feats, tgt_feats, ids_list, temperature=0.07, math: Optio
         ids.append(i)
     denom = n_src if denom_layers is None else denom_layers
     if uniform:
-        loss = _fused_call(src, tgt, ids, temperature, math)
+        loss = _fused_call(src, tgt, ids, temperature, math, mb=mb)
     else:
         # layers of different batch size / dtype: one call per layer, summed like the reference's loop (:36-40)
-        loss = sum(_fused_call([s], [t], [i], temperature, math) for s, t, i in zip(src, tgt, ids)) / float(n)
+        loss = sum(_fused_call([s], [t], [i], temperature, math, mb=mb) for s, t, i in zip(src, tgt, ids)) / float(n)
     if denom != n:                       # zip truncation case: kernel divided by n, reference by len(src)
         loss = loss * (float(n) / float(denom))
     return loss
@@ -687,15 +732,26 @@ class PatchNCELoss(nn.Module):
     id draw per zipped layer, loss = sum over layers / len(src_feats).
     ``forward(feat_q, feat_k)`` with two (B*P, D) row tensors (rows grouped per image, already
     L2-normalised, e.g. from ``PatchSampleF``) returns that layer's mean diagonal CE; the number of
-    images is ``feat_q.shape[0] // min(num_patches, rows)`` unless ``batch_size`` is given."""
+    images is ``feat_q.shape[0] // min(num_patches, rows)`` unless ``batch_size`` is given.
+
+    ``nce_includes_all_negatives_from_minibatch=True`` is upstream CUT's switch of that name (``batch_dim_for_bmm = 1``;
+    the reference's config declares it, configs/train_gan_cutpp.yaml:80): each query patch of a layer is contrasted with
+    the patches of ALL images of the batch, not only its own image's.  Per layer the loss is the reference's
+    (:42-110) on one group of B * P rows -- logits N x N with N = B * P, diagonal positives, +-50 clamp, mean CE over the
+    N rows, the non-finite guard applied to the group -- computed on the tensor cores (k_loss_tc_mb) without the N x N
+    logits ever reaching memory.  At B = 1 it is the per-image loss.  Under data parallelism the negatives are the
+    rank's own shard, as upstream CUT under DDP.  Tensor-core math modes only; C <= 256, P <= 1024 (<= 256 on the row
+    route) and B * round_up(P, 128) <= 65536 per layer, RuntimeError otherwise."""
 
     def __init__(self, temperature: float = 0.07, num_patches: int = 256,
-                 nce_layers: Sequence[int] = (0, 4, 8, 12, 16), math: Optional[str] = None):
+                 nce_layers: Sequence[int] = (0, 4, 8, 12, 16), math: Optional[str] = None,
+                 nce_includes_all_negatives_from_minibatch: bool = False):
         super().__init__()
         self.temperature = temperature
         self.num_patches = num_patches
         self.nce_layers = list(nce_layers)      # stored, never used -- as in the reference (:22)
         self.math = math
+        self.nce_includes_all_negatives_from_minibatch = bool(nce_includes_all_negatives_from_minibatch)
         self._last_ids = None
 
     @property
@@ -707,11 +763,14 @@ class PatchNCELoss(nn.Module):
         return v
 
     def forward(self, a, b, batch_size: Optional[int] = None):
+        mb = self.nce_includes_all_negatives_from_minibatch
         if isinstance(a, torch.Tensor) and a.dim() == 2:
+            if mb:
+                return rows_patchnce_multi([a], [b], self.temperature, self.num_patches, batch_size, self.math, True)
             return rows_patchnce(a, b, self.temperature, self.num_patches, batch_size, self.math)
         if not isinstance(a, torch.Tensor) and len(a) > 0 and a[0].dim() == 2:
             # two lists of (B*P_l, D_l) rows (what PatchSampleF returns): every layer in one call, mean over layers
-            return rows_patchnce_multi(a, b, self.temperature, self.num_patches, batch_size, self.math)
+            return rows_patchnce_multi(a, b, self.temperature, self.num_patches, batch_size, self.math, mb)
         call, tgt, scale = self._begin(a, b)
         if call is None:
             return tgt                               # mixed layers: the per-layer composition already ran
@@ -744,14 +803,17 @@ class PatchNCELoss(nn.Module):
         n = len(tgt)
         dev = tgt[0].device
         _warn_queue(dev).poll()
+        mb = self.nce_includes_all_negatives_from_minibatch
         if not uniform:
             ids = draw_patch_ids_all(src, self.num_patches)                           # :60-63
             self.__dict__["_last_ids"] = ids
-            return None, fused_patchnce(src, tgt, ids, self.temperature, math, denom_layers=n_src), None
+            return None, fused_patchnce(src, tgt, ids, self.temperature, math, denom_layers=n_src,
+                                        nce_includes_all_negatives_from_minibatch=mb), None
         p_list = [patch_count(self.num_patches, t.shape[2] * t.shape[3]) for t in tgt]    # :60
         if max(p_list) > _lib.MAX_PATCHES:
             raise RuntimeError(f"num_patches > {_lib.MAX_PATCHES} is not supported")
-        sp = _shape_plan(tgt, p_list, math, _is_nhwc(tgt[0]))
+        # B = 1: minibatch negatives ARE the per-image loss -- the per-image kernels, bit for bit
+        sp = _shape_plan(tgt, p_list, math, _is_nhwc(tgt[0]), mb and tgt[0].shape[0] > 1)
         rng = idplan = None
         if sp.tc and not torch.cuda.is_current_stream_capturing() and _philox_ready(dev):
             # the library draws the ids (bit for bit torch.randint's, :63) inside its id-sort launch: no randint
@@ -790,12 +852,15 @@ class PatchNCELoss(nn.Module):
 
 
 def compute_patchnce_loss(generator, src_images, tgt_images, nce_layers, temperature=0.07,
-                          num_patches=256, math: Optional[str] = None):
+                          num_patches=256, math: Optional[str] = None,
+                          nce_includes_all_negatives_from_minibatch: bool = False):
     """Drop-in for ``compute_patchnce_loss`` -- patchnce_cut.py:113-149 (call site
     training/train_cutpp.py:285-292).  ``generator`` only needs ``get_feature_layers``.  After
     ``enable_encoder_feature_reuse(generator, nce_layers)`` the source features are the activations of the
-    ``generator(src_images)`` call that produced ``tgt_images`` (feature_reuse.py), not a second pass."""
-    nce_loss_fn = PatchNCELoss(temperature, num_patches, nce_layers, math=math)       # :135
+    ``generator(src_images)`` call that produced ``tgt_images`` (feature_reuse.py), not a second pass.
+    ``nce_includes_all_negatives_from_minibatch``: see ``PatchNCELoss``."""
+    nce_loss_fn = PatchNCELoss(temperature, num_patches, nce_layers, math=math,                       # :135
+                               nce_includes_all_negatives_from_minibatch=nce_includes_all_negatives_from_minibatch)
     from .feature_reuse import cached_source_features
     src_feats = cached_source_features(generator, src_images, nce_layers)  # maps of the generator(src) just run, if tapped
     if src_feats is None:
@@ -1087,16 +1152,16 @@ class _RowsLossFn(torch.autograd.Function):
 class _RowsLossMultiFn(torch.autograd.Function):
     """``mean_l PatchNCELoss(feat_q[l], feat_k[l])`` for every layer of a ``PatchSampleF`` output in ONE call of the
     library (pnce_rows_loss_multi_fwd_bwd: one pack launch, one tcgen05 loss launch).  Inputs: batch, temperature, math,
-    n, the n query row tensors, the n (detached) key row tensors."""
+    n, mb (minibatch negatives: pnce_rows_mb_fwd_bwd), the n query row tensors, the n (detached) key row tensors."""
 
     @staticmethod
-    def forward(ctx, batch, temperature, math, n, *args):
+    def forward(ctx, batch, temperature, math, n, mb, *args):
         lib = _lib.load()
         qs = [_f32c(a) for a in args[:n]]
         ks = [_f32c(a) for a in args[n:]]
         dev = qs[0].device
         rows = (_lib.PnceRows * n)()
-        key = ["multi", batch]
+        key = ["mb" if mb else "multi", batch]
         with _on_device(dev):
             dqs = [torch.empty_like(q) for q in qs]
             for l in range(n):
@@ -1108,15 +1173,15 @@ class _RowsLossMultiFn(torch.autograd.Function):
             ws_bytes = _ROWS_WS_BYTES.get(key)
             if ws_bytes is None:
                 nbytes = ctypes.c_size_t(0)
-                _lib.check(lib.pnce_rows_loss_multi_workspace_bytes(rows, n, batch, ctypes.byref(nbytes)),
-                           "pnce_rows_loss_multi_workspace_bytes")
+                wsq = lib.pnce_rows_mb_workspace_bytes if mb else lib.pnce_rows_loss_multi_workspace_bytes
+                _lib.check(wsq(rows, n, batch, ctypes.byref(nbytes)), "rows workspace query")
                 ws_bytes = _ROWS_WS_BYTES[key] = nbytes.value
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
             out = torch.empty(1 + n, dtype=torch.float32, device=dev)
-            slot, flag_ptr = _warn_queue(dev).acquire()
-            _lib.check(lib.pnce_rows_loss_multi_fwd_bwd(rows, n, batch, temperature, _MATH[math], ws.data_ptr(), ws_bytes,
-                                                        out.data_ptr(), flag_ptr or None, _stream_ptr(dev)),
-                       "pnce_rows_loss_multi_fwd_bwd")
+            slot, flag_ptr = _warn_queue(dev).acquire(mb)
+            fn = lib.pnce_rows_mb_fwd_bwd if mb else lib.pnce_rows_loss_multi_fwd_bwd
+            _lib.check(fn(rows, n, batch, temperature, _MATH[math], ws.data_ptr(), ws_bytes, out.data_ptr(),
+                          flag_ptr or None, _stream_ptr(dev)), "pnce_rows_mb_fwd_bwd" if mb else "pnce_rows_loss_multi_fwd_bwd")
         ctx.save_for_backward(*dqs)
         ctx.q_dtypes = [a.dtype for a in args[:n]]
         ctx.layer_losses = out[1:]
@@ -1126,14 +1191,15 @@ class _RowsLossMultiFn(torch.autograd.Function):
     def backward(ctx, grad_out):
         dqs = torch._foreach_mul(list(ctx.saved_tensors), grad_out)            # one launch for every layer
         dqs = [d if d.dtype is dt else d.to(dt) for d, dt in zip(dqs, ctx.q_dtypes)]
-        return (None, None, None, None, *dqs, *([None] * len(dqs)))
+        return (None, None, None, None, None, *dqs, *([None] * len(dqs)))
 
 
-def rows_patchnce_multi(feat_q, feat_k, temperature=0.07, num_patches=256, batch_size=None, math=None):
+def rows_patchnce_multi(feat_q, feat_k, temperature=0.07, num_patches=256, batch_size=None, math=None, mb=False):
     """``mean_l PatchNCELoss(feat_q[l], feat_k[l])`` over two LISTS of row tensors (one (B*P_l, D_l) pair per layer, as
     ``PatchSampleF`` returns them) -- upstream CUT's ``for f_q, f_k in zip(feat_q, feat_k): total += crit(f_q, f_k)``
     followed by ``/ n_layers``, as one call of the library when every layer fits the tensor-core kernel (P, D <= 256);
-    other shapes take the per-layer calls."""
+    other shapes take the per-layer calls.  ``mb``: minibatch negatives (``PatchNCELoss``), one library call
+    (pnce_rows_mb_fwd_bwd) for every layer."""
     feat_q, feat_k = list(feat_q), list(feat_k)
     n = len(feat_q)
     if n == 0 or n != len(feat_k):
@@ -1156,6 +1222,13 @@ def rows_patchnce_multi(feat_q, feat_k, temperature=0.07, num_patches=256, batch
                 raise RuntimeError(f"{rows} rows are not a multiple of batch_size={batch_size}")
             batches.append(int(batch_size))
     b0, dev = batches[0], feat_q[0].device
+    if mb and b0 > 1:
+        if any(b != b0 for b in batches) or any(q.device != dev for q in feat_q) or n > _lib.MAX_LAYERS:
+            raise RuntimeError("nce_includes_all_negatives_from_minibatch on rows needs layers of one batch size and "
+                               f"device, at most {_lib.MAX_LAYERS} of them")
+        mb_check(b0, [q.shape[1] for q in feat_q], [q.shape[0] // b0 for q in feat_q], math, rows=True)
+        ks = [k.detach() if k.requires_grad else k for k in feat_k]      # upstream CUT and the reference (:142) detach k
+        return _RowsLossMultiFn.apply(b0, float(temperature), math, n, True, *feat_q, *ks)
     fused = (math != "simt_f32" and n <= _lib.MAX_LAYERS and all(b == b0 for b in batches)
              and all(q.device == dev and q.shape[0] // b0 <= 256 and q.shape[1] <= 256 for q in feat_q))
     if not fused:
@@ -1165,7 +1238,7 @@ def rows_patchnce_multi(feat_q, feat_k, temperature=0.07, num_patches=256, batch
             total = l if total is None else total + l
         return total / n
     ks = [k.detach() if k.requires_grad else k for k in feat_k]          # upstream CUT and the reference (:142) detach k
-    return _RowsLossMultiFn.apply(b0, float(temperature), math, n, *feat_q, *ks)
+    return _RowsLossMultiFn.apply(b0, float(temperature), math, n, False, *feat_q, *ks)
 
 
 def rows_patchnce(feat_q, feat_k, temperature=0.07, num_patches=256, batch_size=None, math=None):
@@ -1409,7 +1482,11 @@ def patchnce_with_head(netF: "PatchSampleF", src_feats, tgt_feats, temperature=0
     sharded over the ranks -- the head gradients that come out of ``backward`` are already AVERAGED over
     the group: one flat all-reduce, started on a side stream as soon as the weight-gradient kernels are
     done, so it runs under the HBM-bound dense-gradient kernel (SURVEY.md section 8e).  Do not call
-    ``allreduce_head_grads`` as well."""
+    ``allreduce_head_grads`` as well.
+
+    Per-image negatives only.  For minibatch negatives compose it as upstream CUT does:
+    ``PatchSampleF(use_mlp=True)`` for both sides, then
+    ``PatchNCELoss(nce_includes_all_negatives_from_minibatch=True)(feat_q, feat_k)`` on the two lists."""
     if fused is None:
         fused = fused_head_supported(netF, tgt_feats, num_patches) and (math or DEFAULT_MATH) != "simt_f32"
     if not fused:
@@ -1459,7 +1536,8 @@ def head_loss_and_grads(netF: "PatchSampleF", src_feats, tgt_feats, temperature=
     there.  Same ids, kernels and values as the autograd route; no ``Function.apply``, no engine hand-off and no
     ``AccumulateGrad`` per parameter (20 of them for five layers): at the batches the reference trains with, that
     host work is longer than the GPU's (DESIGN.md 4.5).  For loops that drive the generator's backward themselves:
-    ``torch.autograd.backward(tgt_feats, grads)``."""
+    ``torch.autograd.backward(tgt_feats, grads)``.  Per-image negatives only (see ``patchnce_with_head`` for the
+    minibatch composition)."""
     if (math or DEFAULT_MATH) == "simt_f32":
         raise RuntimeError("head_loss_and_grads runs the tensor-core head only")
     plan, tgt, params, ids = _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group)
@@ -1501,7 +1579,8 @@ def _one(dev) -> torch.Tensor:
     return t
 
 
-def install_reference_shim(optimiser_side: bool = False, d_side: bool = False):
+def install_reference_shim(optimiser_side: bool = False, d_side: bool = False,
+                           nce_includes_all_negatives_from_minibatch: bool = False):
     """Make ``from GAN_Variant1.losses.patchnce_cut import compute_patchnce_loss`` resolve to this
     implementation, so the unchanged reference training loop (train_cutpp.py:28) uses the B200
     path.  Call before importing ``GAN_Variant1.training.train_cutpp``.
@@ -1510,7 +1589,12 @@ def install_reference_shim(optimiser_side: bool = False, d_side: bool = False):
     reference package must be importable): ``GAN_Variant1.utils.io_ckpt.EMA`` (imported by name at
     train_cutpp.py:34) -> the one-launch ``EMA``, and ``AMPContext.step_optimizer`` (amp_utils.py:29) -> the
     three-launch ``amp_step_optimizer``.  ``d_side=True`` does the same for row 4: ``training.diffaugment.DiffAugment``
-    (imported by name at train_cutpp.py:30) and ``losses.adv_hinge.discriminator_hinge_loss`` / ``generator_hinge_loss``."""
+    (imported by name at train_cutpp.py:30) and ``losses.adv_hinge.discriminator_hinge_loss`` / ``generator_hinge_loss``.
+
+    ``nce_includes_all_negatives_from_minibatch`` becomes the default of the shimmed ``compute_patchnce_loss`` and
+    ``PatchNCELoss``: the reference loop passes only three keywords to ``compute_patchnce_loss`` (train_cutpp.py:285-292),
+    so this is how ``patchnce.nce_includes_all_negatives_from_minibatch`` of the config reaches the loss."""
+    import functools
     import types
     if d_side:
         import importlib
@@ -1525,8 +1609,13 @@ def install_reference_shim(optimiser_side: bool = False, d_side: bool = False):
         importlib.import_module("GAN_Variant1.utils.io_ckpt").EMA = EMA
         importlib.import_module("GAN_Variant1.utils.amp_utils").AMPContext.step_optimizer = amp_step_optimizer
     mod = types.ModuleType("GAN_Variant1.losses.patchnce_cut")
-    mod.PatchNCELoss = PatchNCELoss
-    mod.compute_patchnce_loss = compute_patchnce_loss
+    if nce_includes_all_negatives_from_minibatch:
+        mod.PatchNCELoss = functools.partial(PatchNCELoss, nce_includes_all_negatives_from_minibatch=True)
+        mod.compute_patchnce_loss = functools.partial(compute_patchnce_loss,
+                                                      nce_includes_all_negatives_from_minibatch=True)
+    else:
+        mod.PatchNCELoss = PatchNCELoss
+        mod.compute_patchnce_loss = compute_patchnce_loss
     mod.__doc__ = "B200-native PatchNCE (gan_variant_research_b200) behind the reference's module path."
     sys.modules["GAN_Variant1.losses.patchnce_cut"] = mod
     pkg = sys.modules.get("GAN_Variant1.losses")

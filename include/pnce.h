@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define PNCE_ABI_VERSION 5
+#define PNCE_ABI_VERSION 6
 #define PNCE_MAX_LAYERS 8      /* nce_layers per call (reference config uses 5 ids -> 4 maps)   */
 #define PNCE_MAX_PATCHES 4096  /* P = min(num_patches, H*W)  patchnce_cut.py:60; argument check only: the
                                 * kernels take P <= 1024 (tensor cores, C <= 256) or P <= 1280 (fp32 CUDA cores),
@@ -145,6 +145,26 @@ int pnce_bwd_ex(const pnce_layer_t* layers, int n_layers, int batch, int dtype, 
                 void* dev_workspace, size_t workspace_bytes, void* dev_plan, size_t plan_bytes,
                 const float* dev_grad_out, void* stream);
 
+/* ---- minibatch negatives: upstream CUT's nce_includes_all_negatives_from_minibatch (ABI 6) --------------------------
+ * The reference's configs/train_gan_cutpp.yaml:80 declares patchnce.nce_includes_all_negatives_from_minibatch; upstream
+ * CUT implements it as batch_dim_for_bmm = 1, i.e. the loss of patchnce_cut.py:42-110 applied to ONE "image" whose rows
+ * are the whole batch.  Per layer, with N = B * P rows in image-major order:
+ *   Q, K = normalize(tgt / src patches of every image) (:77-78), Z = clamp(Q K^T / tau, -50, 50) (N x N, :85-88),
+ *   loss_l = mean over the N rows of CE(Z_i, i) (:91-94), the image guard of :97-99 applied to that single group (a
+ *   non-finite group contributes 0 and its rows get a zero upstream gradient), total = sum_l loss_l / n_layers (:40).
+ * d loss / d tgt keeps the factor 1 / (P B n_layers); keys carry no gradient (:142).  The N x N logits never leave the
+ * SM (k_loss_tc_mb).  Under data parallelism the negatives are those of the caller's shard (as upstream CUT under DDP).
+ * Tensor-core math modes only; P <= 1024, C <= 256 and B * round_up(P, 128) <= 65536 per layer (PNCE_ERR_UNSUPPORTED
+ * otherwise).
+ *   pnce_mb_workspace_bytes : bytes of the workspace pnce_mb_fwd needs
+ *   pnce_mb_fwd             : the arguments of pnce_fwd_ex (layout, id plan or Philox draw -- same ids, same generator
+ *                             advance as pnce_fwd_ex); dev_nonfinite[0] counts the LAYERS whose loss was replaced by 0.
+ *                             The backward is pnce_bwd_ex on the same workspace, layout and math mode.            */
+int pnce_mb_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch, size_t* bytes);
+int pnce_mb_fwd(const pnce_layer_t* layers, int n_layers, int batch, int dtype, int layout, float temperature,
+                int math_mode, void* dev_workspace, size_t workspace_bytes, void* dev_plan, size_t plan_bytes,
+                const unsigned long long* philox_seed_offset, float* dev_loss_out, int* dev_nonfinite, void* stream);
+
 /* ---- north-star module split (SURVEY.md section 8b / row a13) ------------------------------ */
 
 /* PatchSampleF(use_mlp=False) forward for one map: rows_out (B*P, C) fp32 = L2-normalised patches
@@ -186,6 +206,14 @@ int pnce_rows_loss_multi_workspace_bytes(const pnce_rows_t* rows, int n_layers, 
 int pnce_rows_loss_multi_fwd_bwd(const pnce_rows_t* rows, int n_layers, int batch, float temperature, int math_mode,
                                  void* dev_workspace, size_t workspace_bytes, float* dev_loss_out, int* dev_nonfinite,
                                  void* stream);
+/* pnce_rows_loss_multi_fwd_bwd with minibatch negatives (see pnce_mb_fwd): per layer, every row of feat_q is contrasted
+ * with the B * P rows of feat_k, label = its own row (upstream CUT's PatchNCELoss with batch_dim_for_bmm = 1 on the
+ * PatchSampleF output, patchnce_cut.py:83-103 on one group).  P <= 256, D <= 256, B * round_up(P, 128) <= 65536 per
+ * layer; rows[l].dq 32-byte aligned (PNCE_ERR_ALIGN otherwise); dev_nonfinite[0] counts guarded layers.            */
+int pnce_rows_mb_workspace_bytes(const pnce_rows_t* rows, int n_layers, int batch, size_t* bytes);
+int pnce_rows_mb_fwd_bwd(const pnce_rows_t* rows, int n_layers, int batch, float temperature, int math_mode,
+                         void* dev_workspace, size_t workspace_bytes, float* dev_loss_out, int* dev_nonfinite,
+                         void* stream);
 
 /* All maps of one PatchSampleF call in ONE launch each way (the per-map entry points above cost a launch per
  * layer and leave the GPU half empty on the small layers): forward reads feat / ids and writes rows (and inv,
