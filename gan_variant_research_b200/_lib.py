@@ -11,7 +11,7 @@ MATH_SIMT_F32, MATH_TC_BF16X3, MATH_TC_BF16 = 0, 1, 2
 MAX_LAYERS = 8
 MAX_PATCHES = 4096
 MAX_CHANNELS = 1024
-ABI_VERSION = 6
+ABI_VERSION = 7
 LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
 
 EXPORTS = [
@@ -25,6 +25,7 @@ EXPORTS = [
     "pnce_netf_workspace_bytes", "pnce_netf_fwd", "pnce_netf_bwd",
     "pnce_head_fwd_ex", "pnce_head_bwd_ex", "pnce_head_workspace_bytes", "pnce_head_fwd", "pnce_head_bwd", "pnce_head_bwd_params", "pnce_head_bwd_dense",
     "pnce_mb_workspace_bytes", "pnce_mb_fwd", "pnce_rows_mb_workspace_bytes", "pnce_rows_mb_fwd_bwd",
+    "pnce_mb_shard_workspace_bytes", "pnce_mb_shard_keys", "pnce_mb_shard_loss",
 ]
 
 
@@ -104,6 +105,12 @@ def load():
     lib.pnce_mb_fwd.argtypes = lib.pnce_fwd_ex.argtypes
     lib.pnce_rows_mb_workspace_bytes.argtypes = lib.pnce_rows_loss_multi_workspace_bytes.argtypes
     lib.pnce_rows_mb_fwd_bwd.argtypes = lib.pnce_rows_loss_multi_fwd_bwd.argtypes
+    lib.pnce_mb_shard_workspace_bytes.argtypes = [ctypes.POINTER(PnceLayer), i32, i32, i32, ctypes.POINTER(sz),
+                                                  ctypes.POINTER(sz), ctypes.POINTER(sz)]
+    lib.pnce_mb_shard_keys.argtypes = [ctypes.POINTER(PnceLayer), i32, i32, i32, i32, i32, i32, i32, vp, sz, vp, sz,
+                                       ctypes.POINTER(u64), vp]
+    lib.pnce_mb_shard_loss.argtypes = [ctypes.POINTER(PnceLayer), i32, i32, i32, i32, i32, i32, f32, i32, vp, sz, vp, sz,
+                                       vp, vp, vp]
     lib.pnce_head_workspace_bytes.argtypes = [ctypes.POINTER(PnceLayer), i32, i32, i32, ctypes.POINTER(sz)]
     lib.pnce_head_fwd.argtypes = [ctypes.POINTER(PnceLayer), ctypes.POINTER(PnceHead), i32, i32, i32, i32, f32, i32,
                                   vp, sz, vp, vp, vp]

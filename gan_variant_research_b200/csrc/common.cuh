@@ -79,6 +79,13 @@ struct Params {
   unsigned long long rng_seed, rng_offset;
   int rng_draw;
   long long* trace;          // debug: clock64 stamps of two CTAs of the tcgen05 loss kernel, or NULL
+  // global negatives (pnce_mb_shard_loss; kworld = 0 otherwise): the key blobs of every layer (khi, klo, k2hi, k2lo,
+  // kss) point into slot 0 of kworld slots of kslot bytes; slot w holds the keys of global images [w B, (w + 1) B).
+  // This launch's query images are global images kimg0 + b.  qbad: slot 0's per-layer "a query row of that rank is
+  // non-finite" flags (int[PNCE_MAX_LAYERS] at the head of every slot).
+  int kworld, kimg0;
+  size_t kslot;
+  const int* qbad;
 };
 
 // CTA -> layer map for one launch: blocks [start[l], start[l+1]) work on layer l.

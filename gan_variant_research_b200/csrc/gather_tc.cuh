@@ -134,6 +134,31 @@ __global__ void __launch_bounds__(kThreads) k_gather_tc_fold(const __grid_consta
   else gather_tc_chunk<__nv_bfloat16>(p.L[l], p.b0, p.bn, local, p.side0, keys);
 }
 
+// Global negatives (pnce_mb_shard_keys), after the gather: flags[l] = 1 when a query row of layer l of this rank is
+// non-finite -- the gather marks such a row's partial sums of squares with NaN (the padding rows hold 0).  The flags
+// travel in the rank's slot next to its keys, so that every rank's finalize guards the layer on the rows of every rank.
+// The caller zeroes the flags first; CTA (x, l) scans kMbQbadFloats of layer l's qss.  A separate launch rather than a
+// store in the three gather variants: those are HBM-bound and shared by every mode, this reads ~1 % of their bytes
+// back from L2.
+constexpr int kMbQbadFloats = kThreads * 16;
+__global__ void __launch_bounds__(kThreads) k_mb_qbad(const __grid_constant__ Params p, int* flags) {
+  pdl_enter();
+  const int l = blockIdx.y;
+  const LayerDev& L = p.L[l];
+  const size_t n4 = (size_t)p.B * L.nchunk * L.Ppad / 4;     // Ppad is a multiple of 128
+  const float4* q = reinterpret_cast<const float4*>(L.qss);
+  bool bad = false;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const size_t i = (size_t)blockIdx.x * (kMbQbadFloats / 4) + k * kThreads + threadIdx.x;
+    if (i < n4) {
+      const float4 v = __ldcg(q + i);
+      bad |= !(v.x == v.x) || !(v.y == v.y) || !(v.z == v.z) || !(v.w == v.w);
+    }
+  }
+  if (__syncthreads_or(bad) && threadIdx.x == 0) flags[l] = 1;
+}
+
 // One CTA per layer: ids -> (sid, perm, rank, ustart, bitmap, prefix); CTA 0 also resets the
 // last-CTA counter and the protocol flag of the launch sequence.
 __global__ void __launch_bounds__(kThreads) k_prep(const __grid_constant__ Params p) {

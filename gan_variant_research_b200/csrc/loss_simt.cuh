@@ -21,7 +21,9 @@ __host__ __device__ inline size_t loss_simt_smem_bytes(int P) {
 // non-finite guards, batch and layer means.  Parallel over the batch (a block-wide reduction in a
 // fixed order per layer) -- a single thread walking L*B values costs one L2 round trip per value,
 // ~40 us at B=64, on the critical path of every step.
+// GN: global negatives (k_loss_tc_mb_gn) -- the guard of a layer also reads every rank's query flags.
 constexpr int kFinalizeScratchBytes = (32 + 32 + PNCE_MAX_LAYERS + 1) * 4;
+template <bool GN = false>
 __device__ void finalize_losses(const Params& p, void* scratch) {
   const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarp = nthr >> 5;
   const int B = p.B, nl = p.n_layers;
@@ -49,7 +51,10 @@ __device__ void finalize_losses(const Params& p, void* scratch) {
         float s = 0.f;
         for (int w = 0; w < nwarp; ++w) s += w_sum[w];
         const float sl = s / ((float)L.P * (float)B);
-        const int bad = isfinite(sl) ? 0 : 1;
+        int bad = isfinite(sl) ? 0 : 1;
+        // global negatives: the group is every rank's rows -- a non-finite query row on any rank guards the layer
+        for (int w = 0; GN && w < p.kworld; ++w)
+          bad |= __ldcg(reinterpret_cast<const int*>(reinterpret_cast<const unsigned char*>(p.qbad) + w * p.kslot) + l) != 0;
         layer_bad[l] = 0;                                       // guarded like an image: NaN rows keep their NaN
         w_bad[0] = bad;
         p.loss_out[1 + l] = bad ? 0.f : sl;
@@ -134,6 +139,7 @@ __device__ void finalize_losses(const Params& p, void* scratch) {
   }
 }
 
+template <bool GN = false>
 __device__ __forceinline__ void last_cta_finalize(const Params& p, int* flag_s, void* scratch) {
   __threadfence();
   __syncthreads();
@@ -144,7 +150,7 @@ __device__ __forceinline__ void last_cta_finalize(const Params& p, int* flag_s, 
   __syncthreads();
   if (*flag_s) {
     __threadfence();
-    finalize_losses(p, scratch);
+    finalize_losses<GN>(p, scratch);
     if (threadIdx.x == 0) { p.counter[0] = 0u; p.counter[1] = 0u; }
   }
 }

@@ -411,23 +411,40 @@ __device__ __forceinline__ void tc_dq_epilogue(uint32_t tacc, int nstage, int C,
   }
 }
 
+// Global negatives: where key image bk (a global image index) lives -- slot bk / B of p.kslot bytes, image bk % B inside
+// it.  GN = false (one rank): the caller's own blobs, image bk.
+template <bool GN>
+__device__ __forceinline__ size_t tc_mb_key_slot(const Params& p, int bk, int& local) {
+  if (!GN) {
+    local = bk;
+    return 0;
+  }
+  const int w = bk / p.B;
+  local = bk - w * p.B;
+  return (size_t)w * p.kslot;
+}
+
 // 1/||k_j|| of the 256 keys [key0, key0 + 256) of image bk, folded from the gather's partial sums of squares (minibatch
 // mode: an item walks the keys of every image, so the weights are built per key block instead of once per image; 8 KB
 // of L2 reads per block next to the 64-256 KB of operand bytes the block streams).  A non-finite key raises badk.
-__device__ __forceinline__ float tc_mb_key_weight(const LayerDev& L, int bk, int key, int nstage) {
+template <bool GN>
+__device__ __forceinline__ float tc_mb_key_weight(const Params& p, const LayerDev& L, int bk, int key, int nstage) {
+  int lb;
+  const float* kss = reinterpret_cast<const float*>(reinterpret_cast<const unsigned char*>(L.kss) + tc_mb_key_slot<GN>(p, bk, lb));
   float ss = 0.f;
-  for (int s = 0; s < nstage; ++s) ss += __ldcg(L.kss + ((size_t)bk * nstage + s) * L.Ppad + key);
+  for (int s = 0; s < nstage; ++s) ss += __ldcg(kss + ((size_t)lb * nstage + s) * L.Ppad + key);
   const float nrm = sqrtf(ss);
   return (nrm == nrm) ? 1.0f / fmaxf(nrm, kNormEps) : nrm;      // NaN: the gather saw a non-finite element
 }
-__device__ __forceinline__ void tc_mb_key_weights(const LayerDev& L, int bk, int key0, int nstage, int et, float* invk_s,
-                                                  int* badk) {
+template <bool GN>
+__device__ __forceinline__ void tc_mb_key_weights(const Params& p, const LayerDev& L, int bk, int key0, int nstage, int et,
+                                                  float* invk_s, int* badk) {
   asm volatile("bar.sync 1, 128;" ::: "memory");
   for (int j = et; j < 256; j += 128) {
     const int key = key0 + j;
     float w = 0.f;
     if (key < L.P) {
-      w = tc_mb_key_weight(L, bk, key, nstage);
+      w = tc_mb_key_weight<GN>(p, L, bk, key, nstage);
       if (!(w == w)) { *badk = 1; w = 0.f; }
     }
     invk_s[j] = w;
@@ -438,9 +455,12 @@ __device__ __forceinline__ void tc_mb_key_weights(const LayerDev& L, int bk, int
 // MB = false: k_loss_tc, one image's P x P problem per item.  MB = true: k_loss_tc_mb (minibatch negatives): the item
 // (layer, image b, 128-row half) walks the key blocks (b', kb) of EVERY image of the batch -- the K blobs of the batch
 // are one key-blocked blob of B * Ppad keys, and the ids are shared, so the sorted-slot order is a common permutation of
-// all rows.  The item's own block (b, kb(row)) goes last, its diagonal chunks last.  Rows mode (p.rows_mode, MB only):
-// rows are used as given and d loss / d q leaves row-major in dq_rows.
-template <bool MB>
+// all rows.  The item's own block (b, kb(row)) goes last, its diagonal chunks last.  GN = true (MB only):
+// k_loss_tc_mb_gn, global negatives -- the key images are those of every rank's slot (tc_mb_key_slot) and the item's
+// image is global image kimg0 + b, so a rank walks exactly the blocks, in exactly the order, that one GPU walks for the
+// same row (a template parameter: as runtime fields the slot arithmetic cost k_loss_tc_mb ~1 % at B = 16 and 64).
+// Rows mode (p.rows_mode, MB only): rows are used as given and d loss / d q leaves row-major in dq_rows.
+template <bool MB, bool GN = false>
 __device__ __forceinline__ void loss_tc_body(const Params& p, const BlockMap& m) {
   extern __shared__ __align__(1024) unsigned char smem[];
   using namespace umma;
@@ -462,8 +482,11 @@ __device__ __forceinline__ void loss_tc_body(const Params& p, const BlockMap& m)
   // accumulator).  One block (P <= 256): Z is computed once.  More blocks: flash-style two passes --
   // pass 1 accumulates the row sums of exp2 block by block, pass 2 recomputes each Z block for dZ.
   // minibatch mode: nkb counts the blocks of every image, block g = image g / nkbi, block g % nkbi of that image
+  // global negatives: the key images are the kworld * B images of every rank's slot, this item's image is global
+  // image gb = kimg0 + b (its diagonal block and diagonal key weight)
   const int nkbi = (Ppad + 255) >> 8;
-  const int nkb = MB ? p.B * nkbi : nkbi;
+  const int nkb = MB ? (GN ? p.kworld : 1) * p.B * nkbi : nkbi;
+  const int gb = GN ? p.kimg0 + b : b;
   const bool multi = nkb > 1;
   const int nslots1 = multi ? 2 : kTcSlots1;                  // the dZ region is busy in pass 2 of the multi-block case
   const bool x3 = (p.math == PNCE_MATH_TC_BF16X3);
@@ -472,7 +495,7 @@ __device__ __forceinline__ void loss_tc_body(const Params& p, const BlockMap& m)
   // Minibatch mode has no running maximum either: the row sum stays below N 2^(1.02 log2e / tau), finite in fp32 for
   // N = B * Ppad <= 65536 at every tau where the clamp cannot bind.
   const bool single = multi && !((1.0f / p.tau) * 1.02f > kClamp);
-  const int kbd_item = (MB ? b * nkbi : 0) + ((mh * 128) >> 8);   // key block with the diagonals of this item's rows
+  const int kbd_item = (MB ? gb * nkbi : 0) + ((mh * 128) >> 8);   // key block with the diagonals of this item's rows
   const int dlo_item = ((mh * 128) & 255) >> 5;               // and the first of its (up to four) diagonal chunks
   volatile int* dead = &sh->dead;
   long long* tr = nullptr;                                   // debug stamps (pnce_debug_set key 3)
@@ -519,8 +542,10 @@ __device__ __forceinline__ void loss_tc_body(const Params& p, const BlockMap& m)
       for (int pass = 0; pass < npass && ok; ++pass) {
         for (int o = 0; o < nkb && ok; ++o) {
           const int g = single ? tc_block_at(o, nkb, kbd_item) : o;
-          const int bk = MB ? g / nkbi : b, kb = MB ? g % nkbi : g;     // image and block of the keys
-          const size_t kimg = (size_t)bk * Ppad * Cp * 2;
+          const int kb = MB ? g % nkbi : g;                  // block of the keys, in image g / nkbi (minibatch mode)
+          int lb = b;
+          const size_t kslot = MB ? tc_mb_key_slot<GN>(p, g / nkbi, lb) : 0;
+          const size_t kimg = kslot + (size_t)lb * Ppad * Cp * 2;
           const unsigned char* gk_hi = reinterpret_cast<const unsigned char*>(L.khi) + kimg;
           const unsigned char* gk_lo = reinterpret_cast<const unsigned char*>(L.klo) + kimg;
           const unsigned char* g2_hi = reinterpret_cast<const unsigned char*>(L.k2hi) + kimg;
@@ -710,8 +735,8 @@ __device__ __forceinline__ void loss_tc_body(const Params& p, const BlockMap& m)
       dg.pass = true;
       dg.d_w = 0.f;
       dg.off = (uint32_t)((gi & 255) >> 3) * 2048u + rowoff + (uint32_t)(gi & 7) * 2u;
-      const int kbd_row = (MB ? b * nkbi : 0) + kbd;          // the same as a global block index
-      auto mb_weights = [&](int g) { tc_mb_key_weights(L, g / nkbi, (g % nkbi) * 256, nstage, et, invk_s, &sh->badk); };
+      const int kbd_row = (MB ? gb * nkbi : 0) + kbd;         // the same as a global block index
+      auto mb_weights = [&](int g) { tc_mb_key_weights<GN>(p, L, g / nkbi, (g % nkbi) * 256, nstage, et, invk_s, &sh->badk); };
       if (single) {
         // ---- ONE pass per key block (P > 256, clamp cannot bind): exp2 once, unnormalised operand, dQ' += E_blk K_blk;
         //      row sums alongside; the block with this item's diagonals last, its diagonal chunks last and released
@@ -771,7 +796,7 @@ __device__ __forceinline__ void loss_tc_body(const Params& p, const BlockMap& m)
             }
           }
         }
-        const float wd = MB ? fmaxf(tc_mb_key_weight(L, b, rowok ? gi : 0, nstage), 0.f) : __ldcg(L.kinv + (size_t)b * Ppad + (rowok ? gi : 0));
+        const float wd = MB ? fmaxf(tc_mb_key_weight<GN>(p, L, gb, rowok ? gi : 0, nstage), 0.f) : __ldcg(L.kinv + (size_t)b * Ppad + (rowok ? gi : 0));
         const float ydr = ydacc * a * wd;                       // diagonal logit (log2 units)
         const float se = (se4[0] + se4[1]) + (se4[2] + se4[3]);
         const float lse2 = lg2f(se);
@@ -817,7 +842,7 @@ __device__ __forceinline__ void loss_tc_body(const Params& p, const BlockMap& m)
             mbar_arrive(&sh->zfree);                             // this Z block may be overwritten
           }
         }
-        const float wd = MB ? fmaxf(tc_mb_key_weight(L, b, rowok ? gi : 0, nstage), 0.f) : multi ? __ldcg(L.kinv + (size_t)b * Ppad + (rowok ? gi : 0)) : invk_s[gi];
+        const float wd = MB ? fmaxf(tc_mb_key_weight<GN>(p, L, gb, rowok ? gi : 0, nstage), 0.f) : multi ? __ldcg(L.kinv + (size_t)b * Ppad + (rowok ? gi : 0)) : invk_s[gi];
         const float ydr = ydacc * a * wd;                       // unclamped diagonal logit (log2 units)
         const float yd = need_clamp ? fminf(fmaxf(ydr, -cl), cl) : ydr;
         const float se = (se4[0] + se4[1]) + (se4[2] + se4[3]);   // padding columns were masked out in pass A
@@ -907,7 +932,7 @@ __device__ __forceinline__ void loss_tc_body(const Params& p, const BlockMap& m)
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
     p.trace[64 + 3 * (size_t)blockIdx.x + 2] = (long long)t;
   }
-  last_cta_finalize(p, &sh->flag, smem);                       // every CTA-wide phase is over (the __syncthreads above): the ring is free scratch
+  last_cta_finalize<GN>(p, &sh->flag, smem);                   // every CTA-wide phase is over (the __syncthreads above): the ring is free scratch
 }
 
 __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc(const __grid_constant__ Params p,
@@ -920,6 +945,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc_mb(const __grid_const
                                                               const __grid_constant__ BlockMap m) {
   pdl_launch();
   loss_tc_body<true>(p, m);
+}
+
+__global__ void __launch_bounds__(kTcThreads, 1) k_loss_tc_mb_gn(const __grid_constant__ Params p,
+                                                                 const __grid_constant__ BlockMap m) {
+  pdl_launch();
+  loss_tc_body<true, true>(p, m);
 }
 
 // -------------------------------------------------------------------------------------------------

@@ -426,9 +426,10 @@ static int launch_loss_tc(const Params& p, cudaStream_t st, bool single_launch =
   m.start[p.n_layers] = acc;
   if (acc > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
   if (p.mb) {                                                  // minibatch negatives: one CTA per item, every key block
-    int rc = set_smem(k_loss_tc_mb, kTcSmemBytes);
+    auto kernel = p.kworld > 0 ? k_loss_tc_mb_gn : k_loss_tc_mb;   // global negatives: keys from every rank's slot
+    int rc = set_smem(kernel, kTcSmemBytes);
     if (rc != PNCE_OK) return rc;
-    launch_k<4>(k_loss_tc_mb, (unsigned)acc, kTcThreads, kTcSmemBytes, st, p, m);
+    launch_k<4>(kernel, (unsigned)acc, kTcThreads, kTcSmemBytes, st, p, m);
     PNCE_CUDA(cudaGetLastError());
     return PNCE_OK;
   }
@@ -980,6 +981,136 @@ int pnce_mb_fwd(const pnce_layer_t* layers, int n_layers, int batch, int dtype, 
   if (!mb_shapes_ok(layers, n_layers, batch)) return PNCE_ERR_UNSUPPORTED;
   return fwd_impl(layers, n_layers, batch, dtype, temperature, math_mode, ws, ws_bytes, plan, plan_bytes, loss_out,
                   nonfinite, stream, philox, layout, true);
+}
+
+// ---- global negatives: minibatch negatives over the shards of every rank (configs/train_gan_cutpp.yaml:80,
+//      patchnce_cut.py:42-110 on the group of world * batch_local * P rows) ---------------------------------------------
+// Workspace: the prefix of pnce_mb_workspace_bytes(batch_local) (query blobs, id tables, gradient rows -- what
+// pnce_bwd_ex reads), then `world` slots.  A slot holds one rank's qbad flags and, per layer, its key blobs khi, k2hi,
+// kss, klo, k2lo for batch_local images, every piece 256-byte aligned.  The low parts are reserved in both tensor-core
+// modes so that the layout does not depend on the math mode.
+static size_t carve_mb_slot(const pnce_layer_t* layers, int n_layers, int B, bool x3, void* base, Params* p) {
+  Carver cv(base);
+  int* flags = cv.take<int>(PNCE_MAX_LAYERS);
+  if (p != nullptr) p->qbad = flags;
+  for (int l = 0; l < n_layers; ++l) {
+    const size_t Ppad = (layers[l].P + 127) / 128 * 128, Cp = (layers[l].C + 31) / 32 * 32, nchunk = Cp / 32;
+    const size_t blob = (size_t)B * Ppad * Cp;
+    __nv_bfloat16* khi = cv.take<__nv_bfloat16>(blob);
+    __nv_bfloat16* k2hi = cv.take<__nv_bfloat16>(blob);
+    float* kss = cv.take<float>((size_t)B * nchunk * Ppad);
+    __nv_bfloat16* klo = cv.take<__nv_bfloat16>(blob);
+    __nv_bfloat16* k2lo = cv.take<__nv_bfloat16>(blob);
+    if (p != nullptr) {
+      LayerDev& L = p->L[l];
+      L.khi = khi; L.k2hi = k2hi; L.kss = kss;
+      L.klo = x3 ? klo : nullptr;
+      L.k2lo = x3 ? k2lo : nullptr;
+    }
+  }
+  return align_up(cv.off, 256);
+}
+
+// The checks of both shard calls, all before any CUDA call; fills Params with the prefix carve and with slot `slot`'s
+// key blobs.  *slot_bytes: the slot stride.
+static int mb_shard_params(const pnce_layer_t* layers, int n_layers, int batch_local, int dtype, int layout, int world,
+                           int rank, int math_mode, void* ws, size_t ws_bytes, void* plan, size_t plan_bytes, int slot,
+                           Params* p, size_t* slot_bytes) {
+  int rc = check_layers(layers, n_layers, batch_local);
+  if (rc != PNCE_OK) return rc;
+  if (world < 1 || rank < 0 || rank >= world) return PNCE_ERR_ARG;
+  if (dtype < PNCE_F32 || dtype > PNCE_BF16) return PNCE_ERR_ARG;
+  if (layout != PNCE_LAYOUT_NCHW && layout != PNCE_LAYOUT_NHWC) return PNCE_ERR_ARG;
+  if (math_mode < PNCE_MATH_SIMT_F32 || math_mode > PNCE_MATH_TC_BF16) return PNCE_ERR_ARG;
+  if (math_mode == PNCE_MATH_SIMT_F32) return PNCE_ERR_UNSUPPORTED;
+  if ((long long)world * batch_local > 0x7fffffffLL || !mb_shapes_ok(layers, n_layers, world * batch_local))
+    return PNCE_ERR_UNSUPPORTED;                               // the envelope of the GLOBAL batch
+  rc = check_alignment(layers, n_layers, dtype, false);
+  if (rc != PNCE_OK) return rc;
+  if (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 255u)) return PNCE_ERR_WORKSPACE;
+  if (plan != nullptr &&
+      ((reinterpret_cast<uintptr_t>(plan) & 255u) || carve_plan(layers, n_layers, nullptr, nullptr) > plan_bytes))
+    return PNCE_ERR_WORKSPACE;
+  const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
+  const size_t prefix = carve_fused(layers, n_layers, batch_local, true, true, nullptr, nullptr);
+  *slot_bytes = carve_mb_slot(layers, n_layers, batch_local, true, nullptr, nullptr);
+  if (prefix + (size_t)world * *slot_bytes > ws_bytes) return PNCE_ERR_WORKSPACE;
+  carve_fused(layers, n_layers, batch_local, true, x3, ws, p, plan);
+  carve_mb_slot(layers, n_layers, batch_local, x3, static_cast<unsigned char*>(ws) + prefix + (size_t)slot * *slot_bytes, p);
+  p->dtype = dtype;
+  p->math = math_mode;
+  p->b0 = 0; p->bn = batch_local;
+  p->mb = 1;
+  p->nhwc = layout == PNCE_LAYOUT_NHWC ? 1 : 0;
+  return PNCE_OK;
+}
+
+int pnce_mb_shard_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch_local, int world, size_t* bytes,
+                                  size_t* slot_offset, size_t* slot_bytes) {
+  if (bytes == nullptr || slot_offset == nullptr || slot_bytes == nullptr) return PNCE_ERR_ARG;
+  const int rc = check_layers(layers, n_layers, batch_local);
+  if (rc != PNCE_OK) return rc;
+  if (world < 1) return PNCE_ERR_ARG;
+  if ((long long)world * batch_local > 0x7fffffffLL || !mb_shapes_ok(layers, n_layers, world * batch_local))
+    return PNCE_ERR_UNSUPPORTED;
+  *slot_offset = carve_fused(layers, n_layers, batch_local, true, true, nullptr, nullptr);
+  *slot_bytes = carve_mb_slot(layers, n_layers, batch_local, true, nullptr, nullptr);
+  *bytes = *slot_offset + (size_t)world * *slot_bytes;
+  return PNCE_OK;
+}
+
+int pnce_mb_shard_keys(const pnce_layer_t* layers, int n_layers, int batch_local, int dtype, int layout, int world,
+                       int rank, int math_mode, void* ws, size_t ws_bytes, void* plan, size_t plan_bytes,
+                       const unsigned long long* philox, void* stream) {
+  Params p;
+  size_t slot_bytes = 0;
+  int rc = mb_shard_params(layers, n_layers, batch_local, dtype, layout, world, rank, math_mode, ws, ws_bytes, plan,
+                           plan_bytes, rank, &p, &slot_bytes);
+  if (rc != PNCE_OK) return rc;
+  if (philox != nullptr) {
+    if (plan != nullptr) return PNCE_ERR_UNSUPPORTED;          // the draw rides on the id prep (unplanned)
+    p.rng_draw = 1; p.rng_seed = philox[0]; p.rng_offset = philox[1];
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // id prep (unless planned) and the gather: keys straight into slot `rank`, queries into the prefix
+  const bool fold = plan == nullptr && gather_tc_folds(p);
+  if (plan == nullptr && !fold) rc = launch_prep(p, st);
+  if (rc != PNCE_OK) return rc;
+  rc = launch_gather_tc(p, st, fold);
+  if (rc != PNCE_OK) return rc;
+  int* flags = const_cast<int*>(p.qbad);
+  PNCE_CUDA(cudaMemsetAsync(flags, 0, PNCE_MAX_LAYERS * sizeof(int), st));
+  long long most = 1;
+  for (int l = 0; l < n_layers; ++l) {
+    const long long n = (long long)batch_local * p.L[l].nchunk * p.L[l].Ppad;
+    if ((n + kMbQbadFloats - 1) / kMbQbadFloats > most) most = (n + kMbQbadFloats - 1) / kMbQbadFloats;
+  }
+  if (most > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
+  launch_k<2>(k_mb_qbad, dim3((unsigned)most, (unsigned)n_layers), kThreads, 0, st, p, flags);
+  PNCE_CUDA(cudaGetLastError());
+  return PNCE_OK;
+}
+
+int pnce_mb_shard_loss(const pnce_layer_t* layers, int n_layers, int batch_local, int dtype, int layout, int world,
+                       int rank, float temperature, int math_mode, void* ws, size_t ws_bytes, void* plan,
+                       size_t plan_bytes, float* loss_out, int* nonfinite, void* stream) {
+  Params p;
+  size_t slot_bytes = 0;
+  int rc = mb_shard_params(layers, n_layers, batch_local, dtype, layout, world, rank, math_mode, ws, ws_bytes, plan,
+                           plan_bytes, 0, &p, &slot_bytes);
+  if (rc != PNCE_OK) return rc;
+  if (loss_out == nullptr || !(temperature > 0.f)) return PNCE_ERR_ARG;
+  p.tau = temperature;
+  p.loss_out = loss_out;
+  p.nonfinite = nonfinite;
+  p.trace = g_dbg.trace;
+  p.kworld = world;
+  p.kimg0 = rank * batch_local;
+  p.kslot = slot_bytes;
+  int ctas_per_image = 0;
+  for (int l = 0; l < n_layers; ++l) ctas_per_image += p.L[l].Ppad / 128;
+  p.total_ctas = (unsigned)(batch_local * ctas_per_image);
+  return launch_loss_tc(p, static_cast<cudaStream_t>(stream));
 }
 
 // ---- module-split API ------------------------------------------------------------------------

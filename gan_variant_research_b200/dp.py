@@ -13,6 +13,10 @@ Only the netF head (north-star extension, absent from the reference) owns parame
 gradients must be summed: ``allreduce_head_grads`` does it as ONE flat all-reduce (<= 2.1 MB, latency
 bound on NVLink 5) on the current stream; torch.distributed (NCCL on GPUs, gloo in the CPU tests)
 is plumbing here.
+
+Global negatives (``PatchNCELoss(..., nce_includes_all_negatives_from_minibatch=True, negatives_group=...)``) add one
+collective to the forward: the all-gather of every rank's detached keys (``allgather_slots_``).  The backward stays
+local.
 """
 from __future__ import annotations
 
@@ -68,6 +72,23 @@ def resolve_group(group):
     if group is True:
         group = dist.group.WORLD
     return group if dist.get_world_size(group) > 1 else None
+
+
+def allgather_slots_(region: torch.Tensor, rank: int, group=None) -> torch.Tensor:
+    """In-place all-gather of equal slots: ``region`` (a flat uint8 tensor of ``world`` slots) holds this rank's bytes
+    in slot ``rank``; afterwards slot ``w`` holds rank ``w``'s.  The key exchange of global negatives
+    (``PatchNCELoss(negatives_group=...)``): ordered after the work already queued on the current stream, and the
+    current stream waits for it -- no host synchronisation under NCCL."""
+    world = dist.get_world_size(group)
+    if world == 1:
+        return region
+    slots = region.view(world, -1)
+    if dist.get_backend(group) == "nccl":
+        dist.all_gather_into_tensor(region, slots[rank], group=group)      # NCCL allgather in place
+    else:
+        # gloo takes CUDA tensors in the list form only; the input must not alias an output it writes
+        dist.all_gather(list(slots.unbind(0)), slots[rank].clone(), group=group)
+    return region
 
 
 def allreduce_flat_(flat: torch.Tensor, group=None, average: bool = True) -> torch.Tensor:

@@ -26,6 +26,7 @@ import threading
 from typing import List, Optional, Sequence
 
 import torch
+import torch.distributed as dist
 import torch.nn as nn
 
 from . import _lib
@@ -336,13 +337,15 @@ class _ShapePlan:
 
     __slots__ = ("n", "batch", "dtype", "dtype_code", "math", "math_code", "dev", "p_list", "p_total", "tc",
                  "ws_bytes", "plan_bytes", "fwd_layers", "bwd_layers", "fwd_lock", "bwd_lock", "big", "shapes", "nhwc",
-                 "mb")
+                 "mb", "world", "slot_offset", "slot_bytes")
 
-    def __init__(self, dev, dtype, shapes, p_list, math, nhwc=False, mb=False):
+    def __init__(self, dev, dtype, shapes, p_list, math, nhwc=False, mb=False, world=1):
         if mb:
-            mb_check(shapes[0][0], [s[1] for s in shapes], p_list, math)
+            mb_check(shapes[0][0], [s[1] for s in shapes], p_list, math, world=world)
         lib = _lib.load()
         self.mb = mb                             # minibatch negatives (pnce_mb_fwd)
+        self.world = world                       # > 1: global negatives over `world` ranks (pnce_mb_shard_*)
+        self.slot_offset = self.slot_bytes = 0
         self.n, self.batch, self.dtype, self.dev, self.math = len(shapes), shapes[0][0], dtype, dev, math
         self.nhwc = nhwc                         # channels-last storage (pnce_fwd_ex / pnce_bwd_ex, LAYOUT_NHWC)
         self.dtype_code, self.math_code = _DTYPES[dtype], _MATH[math]
@@ -354,7 +357,12 @@ class _ShapePlan:
             for l, ((_, c, h, w), p) in enumerate(zip(shapes, p_list)):
                 arr[l].C, arr[l].H, arr[l].W, arr[l].P = c, h, w, p
         nbytes = ctypes.c_size_t(0)
-        if mb:
+        if world > 1:
+            so, sb = ctypes.c_size_t(0), ctypes.c_size_t(0)
+            _lib.check(lib.pnce_mb_shard_workspace_bytes(self.fwd_layers, self.n, self.batch, world, ctypes.byref(nbytes),
+                                                         ctypes.byref(so), ctypes.byref(sb)), "pnce_mb_shard_workspace_bytes")
+            self.slot_offset, self.slot_bytes = so.value, sb.value
+        elif mb:
             _lib.check(lib.pnce_mb_workspace_bytes(self.fwd_layers, self.n, self.batch, ctypes.byref(nbytes)),
                        "pnce_mb_workspace_bytes")
         else:
@@ -387,10 +395,11 @@ def tc_envelope(shapes, p_list, math) -> bool:
 MB_MAX_KEYS = 65536      # keys (B * round_up(P, 128)) per layer of the minibatch-negatives kernel (include/pnce.h)
 
 
-def mb_check(batch, channels, p_list, math, rows=False):
+def mb_check(batch, channels, p_list, math, rows=False, world=1):
     """The envelope of minibatch negatives (``nce_includes_all_negatives_from_minibatch``): tensor-core math, C <= 256,
     P <= 1024 per image (P <= 256 on the row route) and B * round_up(P, 128) <= 65536 per layer.  Raises RuntimeError
-    outside it: there is no other implementation of this mode to fall back to."""
+    outside it: there is no other implementation of this mode to fall back to.  ``world``: global negatives over that
+    many equal shards of ``batch`` images each -- the key bound applies to the global batch ``world * batch``."""
     if math == "simt_f32":
         raise RuntimeError("nce_includes_all_negatives_from_minibatch needs a tensor-core math mode (tc_bf16x3 or tc_bf16), "
                            "not simt_f32")
@@ -399,9 +408,10 @@ def mb_check(batch, channels, p_list, math, rows=False):
         if c > 256 or p > pmax:
             raise RuntimeError(f"nce_includes_all_negatives_from_minibatch supports C <= 256 and P <= {pmax} per layer "
                                f"(got C={c}, P={p})")
-        if batch * ((p + 127) // 128 * 128) > MB_MAX_KEYS:
+        if world * batch * ((p + 127) // 128 * 128) > MB_MAX_KEYS:
+            got = f"batch={batch}" if world == 1 else f"global batch={world * batch} ({world} ranks x {batch})"
             raise RuntimeError(f"nce_includes_all_negatives_from_minibatch supports at most {MB_MAX_KEYS} keys per layer "
-                               f"(batch * round_up(P, 128)); got batch={batch}, P={p}")
+                               f"(batch * round_up(P, 128)); got {got}, P={p}")
 
 
 def _is_nhwc(t) -> bool:
@@ -409,14 +419,15 @@ def _is_nhwc(t) -> bool:
     return t.dim() == 4 and not t.is_contiguous() and t.is_contiguous(memory_format=torch.channels_last)
 
 
-def _shape_plan(tgt, p_list, math, nhwc=False, mb=False) -> _ShapePlan:
+def _shape_plan(tgt, p_list, math, nhwc=False, mb=False, world=1) -> _ShapePlan:
     t0 = tgt[0]
-    key = (t0.device.index, t0.dtype, math, nhwc, mb, tuple(p_list), *[t.shape for t in tgt])
+    key = (t0.device.index, t0.dtype, math, nhwc, mb, world, tuple(p_list), *[t.shape for t in tgt])
     sp = _SHAPE_PLANS.get(key)
     if sp is None:
         if len(_SHAPE_PLANS) > 256:                  # a caller cycling through many shapes: do not grow without bound
             _SHAPE_PLANS.clear()
-        sp = _SHAPE_PLANS[key] = _ShapePlan(t0.device, t0.dtype, [tuple(t.shape) for t in tgt], p_list, math, nhwc, mb)
+        sp = _SHAPE_PLANS[key] = _ShapePlan(t0.device, t0.dtype, [tuple(t.shape) for t in tgt], p_list, math, nhwc, mb,
+                                            world)
     return sp
 
 
@@ -447,12 +458,13 @@ class _FlatIds:
 
 class _Call:
     """One fused call: the shape plan plus what is not a differentiable input."""
-    __slots__ = ("sp", "src", "ids", "temperature", "rng", "idplan")
+    __slots__ = ("sp", "src", "ids", "temperature", "rng", "idplan", "group")
 
-    def __init__(self, sp, src, ids, temperature, rng=None, idplan=None):
+    def __init__(self, sp, src, ids, temperature, rng=None, idplan=None, group=None):
         self.sp, self.src, self.ids, self.temperature = sp, src, ids, float(temperature)
         self.rng = rng            # (philox seed, offset): the library draws the ids itself (pnce_fwd_draw)
         self.idplan = idplan      # k_prep's outputs when the id draw + sort already ran on the side stream
+        self.group = group        # global negatives: the process group of sp.world ranks the keys are gathered over
 
 
 def _layer_array(src, tgt, dtgt, ids):
@@ -486,7 +498,9 @@ def _run_fwd(call: _Call, tgt_feats):
             for l in range(n):
                 a = layers[l]
                 a.src, a.tgt, a.ids = src[l].data_ptr(), tgt_feats[l].data_ptr(), ids[l].data_ptr()
-            if sp.mb:
+            if sp.world > 1:
+                rc = _run_fwd_global(lib, call, layers, ws, out, flag_ptr, st)
+            elif sp.mb:
                 philox = (ctypes.c_ulonglong * 2)(call.rng[0], call.rng[1]) if call.rng is not None else None
                 pl = call.idplan
                 rc = lib.pnce_mb_fwd(layers, n, sp.batch, sp.dtype_code, _lib.LAYOUT_NHWC if sp.nhwc else _lib.LAYOUT_NCHW,
@@ -513,6 +527,25 @@ def _run_fwd(call: _Call, tgt_feats):
         if rc != 0:
             _lib.check(rc, "pnce_fwd")
     return ws, out
+
+
+def _run_fwd_global(lib, call: _Call, layers, ws, out, flag_ptr, st) -> int:
+    """Global negatives: this rank's keys into its slot of the workspace, the all-gather of the slots (the one
+    collective of the mode; keys carry no gradient, so the backward is local), then the loss over every rank's keys."""
+    from . import dp
+    sp = call.sp
+    rank = dist.get_rank(call.group)
+    layout = _lib.LAYOUT_NHWC if sp.nhwc else _lib.LAYOUT_NCHW
+    philox = (ctypes.c_ulonglong * 2)(call.rng[0], call.rng[1]) if call.rng is not None else None
+    pl = call.idplan
+    plp, pln = (pl.data_ptr(), pl.numel()) if pl is not None else (None, 0)
+    rc = lib.pnce_mb_shard_keys(layers, sp.n, sp.batch, sp.dtype_code, layout, sp.world, rank, sp.math_code,
+                                ws.data_ptr(), sp.ws_bytes, plp, pln, philox, st)
+    if rc != 0:
+        return rc
+    dp.allgather_slots_(ws[sp.slot_offset:sp.slot_offset + sp.world * sp.slot_bytes], rank, call.group)
+    return lib.pnce_mb_shard_loss(layers, sp.n, sp.batch, sp.dtype_code, layout, sp.world, rank, call.temperature,
+                                  sp.math_code, ws.data_ptr(), sp.ws_bytes, plp, pln, out.data_ptr(), flag_ptr or None, st)
 
 
 # ---- compressible memory for the dense gradients (csrc/comp_alloc.cuh) ---------------------------------------------
@@ -689,17 +722,36 @@ def _prepare_maps(src_feats, tgt_feats, math=None, patches=None):
     return src, tgt, n_src, uniform
 
 
-def _fused_call(src, tgt, ids, temperature, math, rng=None, idplan=None, mb=False):
-    sp = _shape_plan(tgt, [i.numel() for i in ids], math, _is_nhwc(tgt[0]), mb and tgt[0].shape[0] > 1)
-    return _FusedPatchNCE.apply(_Call(sp, src, ids, temperature, rng, idplan), *tgt)
+def _negatives_group(mb, negatives_group):
+    """-> (process group, world) of global negatives, or (None, 1): minibatch negatives on this rank's batch alone."""
+    if negatives_group is None:
+        return None, 1
+    if not mb:
+        raise ValueError("negatives_group needs nce_includes_all_negatives_from_minibatch=True")
+    from . import dp
+    group = dp.resolve_group(negatives_group)
+    return (group, dist.get_world_size(group)) if group is not None else (None, 1)
+
+
+def _mb_plan(tgt, p_list, math, mb, world):
+    # B = 1 on one rank: minibatch negatives ARE the per-image loss -- the per-image kernels, bit for bit
+    return _shape_plan(tgt, p_list, math, _is_nhwc(tgt[0]), mb and (tgt[0].shape[0] > 1 or world > 1), world)
+
+
+def _fused_call(src, tgt, ids, temperature, math, rng=None, idplan=None, mb=False, group=None, world=1):
+    sp = _mb_plan(tgt, [i.numel() for i in ids], math, mb, world)
+    return _FusedPatchNCE.apply(_Call(sp, src, ids, temperature, rng, idplan, group), *tgt)
 
 
 def fused_patchnce(src_feats, tgt_feats, ids_list, temperature=0.07, math: Optional[str] = None,
-                   denom_layers: Optional[int] = None, nce_includes_all_negatives_from_minibatch: bool = False):
+                   denom_layers: Optional[int] = None, nce_includes_all_negatives_from_minibatch: bool = False,
+                   negatives_group=None):
     """All-layer PatchNCE on dense NCHW maps with given ids.  Returns the scalar loss tensor
     (fp32, on device, differentiable w.r.t. every ``tgt_feats[l]`` that requires grad).
-    ``nce_includes_all_negatives_from_minibatch``: see ``PatchNCELoss``."""
+    ``nce_includes_all_negatives_from_minibatch``, ``negatives_group``: see ``PatchNCELoss`` (every rank passes the
+    same ids)."""
     mb = bool(nce_includes_all_negatives_from_minibatch)
+    group, world = _negatives_group(mb, negatives_group)
     math = math or DEFAULT_MATH
     if len(ids_list) < min(len(src_feats), len(tgt_feats)):
         raise RuntimeError(f"{len(ids_list)} id tensors for {min(len(src_feats), len(tgt_feats))} layers")
@@ -715,10 +767,11 @@ def fused_patchnce(src_feats, tgt_feats, ids_list, temperature=0.07, math: Optio
         ids.append(i)
     denom = n_src if denom_layers is None else denom_layers
     if uniform:
-        loss = _fused_call(src, tgt, ids, temperature, math, mb=mb)
+        loss = _fused_call(src, tgt, ids, temperature, math, mb=mb, group=group, world=world)
     else:
         # layers of different batch size / dtype: one call per layer, summed like the reference's loop (:36-40)
-        loss = sum(_fused_call([s], [t], [i], temperature, math, mb=mb) for s, t, i in zip(src, tgt, ids)) / float(n)
+        loss = sum(_fused_call([s], [t], [i], temperature, math, mb=mb, group=group, world=world)
+                   for s, t, i in zip(src, tgt, ids)) / float(n)
     if denom != n:                       # zip truncation case: kernel divided by n, reference by len(src)
         loss = loss * (float(n) / float(denom))
     return loss
@@ -740,18 +793,30 @@ class PatchNCELoss(nn.Module):
     (:42-110) on one group of B * P rows -- logits N x N with N = B * P, diagonal positives, +-50 clamp, mean CE over the
     N rows, the non-finite guard applied to the group -- computed on the tensor cores (k_loss_tc_mb) without the N x N
     logits ever reaching memory.  At B = 1 it is the per-image loss.  Under data parallelism the negatives are the
-    rank's own shard, as upstream CUT under DDP.  Tensor-core math modes only; C <= 256, P <= 1024 (<= 256 on the row
-    route) and B * round_up(P, 128) <= 65536 per layer, RuntimeError otherwise."""
+    rank's own shard, as upstream CUT under DDP, unless ``negatives_group`` is given (below).  Tensor-core math modes only; C <= 256, P <= 1024 (<= 256 on the row
+    route) and B * round_up(P, 128) <= 65536 per layer, RuntimeError otherwise.
+
+    ``negatives_group`` (with the flag only, ValueError otherwise): global negatives under data parallelism.  ``True``
+    (the default process group) or a ``ProcessGroup`` of W ranks, each holding an equal shard of B_l images in rank
+    order (``dp.shard_batch``) and drawing the same ids (one seed, or ``dp.broadcast_patch_ids``): every rank's query
+    rows are contrasted with the keys of all W * B_l images, which are all-gathered without gradient in the forward.
+    Each rank returns the mean over its own rows, so averaging gradients over the ranks (``dp.GradReducer``, DDP)
+    reproduces one GPU on the global batch; a non-finite row or key anywhere zeroes the layer on every rank.  The
+    envelope above applies to the global batch.  ``None`` (default), or a group of one rank: the rank's own batch.
+    Maps route only: the row route raises RuntimeError."""
 
     def __init__(self, temperature: float = 0.07, num_patches: int = 256,
                  nce_layers: Sequence[int] = (0, 4, 8, 12, 16), math: Optional[str] = None,
-                 nce_includes_all_negatives_from_minibatch: bool = False):
+                 nce_includes_all_negatives_from_minibatch: bool = False, negatives_group=None):
         super().__init__()
+        if negatives_group is not None and not nce_includes_all_negatives_from_minibatch:
+            raise ValueError("negatives_group needs nce_includes_all_negatives_from_minibatch=True")
         self.temperature = temperature
         self.num_patches = num_patches
         self.nce_layers = list(nce_layers)      # stored, never used -- as in the reference (:22)
         self.math = math
         self.nce_includes_all_negatives_from_minibatch = bool(nce_includes_all_negatives_from_minibatch)
+        self.negatives_group = negatives_group
         self._last_ids = None
 
     @property
@@ -764,6 +829,11 @@ class PatchNCELoss(nn.Module):
 
     def forward(self, a, b, batch_size: Optional[int] = None):
         mb = self.nce_includes_all_negatives_from_minibatch
+        rows = (isinstance(a, torch.Tensor) and a.dim() == 2) or (not isinstance(a, torch.Tensor) and len(a) > 0
+                                                                   and a[0].dim() == 2)
+        if rows and self.negatives_group is not None:
+            raise RuntimeError("negatives_group covers the maps route (PatchNCELoss(src_feats, tgt_feats)); global "
+                               "negatives on the row route (PatchNCELoss(feat_q, feat_k)) are out of scope")
         if isinstance(a, torch.Tensor) and a.dim() == 2:
             if mb:
                 return rows_patchnce_multi([a], [b], self.temperature, self.num_patches, batch_size, self.math, True)
@@ -808,12 +878,13 @@ class PatchNCELoss(nn.Module):
             ids = draw_patch_ids_all(src, self.num_patches)                           # :60-63
             self.__dict__["_last_ids"] = ids
             return None, fused_patchnce(src, tgt, ids, self.temperature, math, denom_layers=n_src,
-                                        nce_includes_all_negatives_from_minibatch=mb), None
+                                        nce_includes_all_negatives_from_minibatch=mb,
+                                        negatives_group=self.negatives_group), None
         p_list = [patch_count(self.num_patches, t.shape[2] * t.shape[3]) for t in tgt]    # :60
         if max(p_list) > _lib.MAX_PATCHES:
             raise RuntimeError(f"num_patches > {_lib.MAX_PATCHES} is not supported")
-        # B = 1: minibatch negatives ARE the per-image loss -- the per-image kernels, bit for bit
-        sp = _shape_plan(tgt, p_list, math, _is_nhwc(tgt[0]), mb and tgt[0].shape[0] > 1)
+        group, world = _negatives_group(mb, self.negatives_group)
+        sp = _mb_plan(tgt, p_list, math, mb, world)
         rng = idplan = None
         if sp.tc and not torch.cuda.is_current_stream_capturing() and _philox_ready(dev):
             # the library draws the ids (bit for bit torch.randint's, :63) inside its id-sort launch: no randint
@@ -848,19 +919,21 @@ class PatchNCELoss(nn.Module):
             ids = draw_patch_ids_all(src, self.num_patches)                           # :60-63
             self.__dict__["_last_ids"] = ids
         # zip truncation: the kernel divides by n, the reference by len(src_feats) (:40)
-        return _Call(sp, src, ids, self.temperature, rng, idplan), tgt, (None if n_src == n else float(n) / float(n_src))
+        return (_Call(sp, src, ids, self.temperature, rng, idplan, group), tgt,
+                (None if n_src == n else float(n) / float(n_src)))
 
 
 def compute_patchnce_loss(generator, src_images, tgt_images, nce_layers, temperature=0.07,
                           num_patches=256, math: Optional[str] = None,
-                          nce_includes_all_negatives_from_minibatch: bool = False):
+                          nce_includes_all_negatives_from_minibatch: bool = False, negatives_group=None):
     """Drop-in for ``compute_patchnce_loss`` -- patchnce_cut.py:113-149 (call site
     training/train_cutpp.py:285-292).  ``generator`` only needs ``get_feature_layers``.  After
     ``enable_encoder_feature_reuse(generator, nce_layers)`` the source features are the activations of the
     ``generator(src_images)`` call that produced ``tgt_images`` (feature_reuse.py), not a second pass.
-    ``nce_includes_all_negatives_from_minibatch``: see ``PatchNCELoss``."""
+    ``nce_includes_all_negatives_from_minibatch``, ``negatives_group``: see ``PatchNCELoss``."""
     nce_loss_fn = PatchNCELoss(temperature, num_patches, nce_layers, math=math,                       # :135
-                               nce_includes_all_negatives_from_minibatch=nce_includes_all_negatives_from_minibatch)
+                               nce_includes_all_negatives_from_minibatch=nce_includes_all_negatives_from_minibatch,
+                               negatives_group=negatives_group)
     from .feature_reuse import cached_source_features
     src_feats = cached_source_features(generator, src_images, nce_layers)  # maps of the generator(src) just run, if tapped
     if src_feats is None:
@@ -1580,7 +1653,7 @@ def _one(dev) -> torch.Tensor:
 
 
 def install_reference_shim(optimiser_side: bool = False, d_side: bool = False,
-                           nce_includes_all_negatives_from_minibatch: bool = False):
+                           nce_includes_all_negatives_from_minibatch: bool = False, negatives_group=None):
     """Make ``from GAN_Variant1.losses.patchnce_cut import compute_patchnce_loss`` resolve to this
     implementation, so the unchanged reference training loop (train_cutpp.py:28) uses the B200
     path.  Call before importing ``GAN_Variant1.training.train_cutpp``.
@@ -1593,9 +1666,13 @@ def install_reference_shim(optimiser_side: bool = False, d_side: bool = False,
 
     ``nce_includes_all_negatives_from_minibatch`` becomes the default of the shimmed ``compute_patchnce_loss`` and
     ``PatchNCELoss``: the reference loop passes only three keywords to ``compute_patchnce_loss`` (train_cutpp.py:285-292),
-    so this is how ``patchnce.nce_includes_all_negatives_from_minibatch`` of the config reaches the loss."""
+    so this is how ``patchnce.nce_includes_all_negatives_from_minibatch`` of the config reaches the loss.
+    ``negatives_group`` (with that flag only, ValueError otherwise) becomes their default as well: global negatives
+    over the ranks of a data-parallel run (``PatchNCELoss``)."""
     import functools
     import types
+    if negatives_group is not None and not nce_includes_all_negatives_from_minibatch:
+        raise ValueError("negatives_group needs nce_includes_all_negatives_from_minibatch=True")
     if d_side:
         import importlib
         from . import dside
@@ -1610,9 +1687,11 @@ def install_reference_shim(optimiser_side: bool = False, d_side: bool = False,
         importlib.import_module("GAN_Variant1.utils.amp_utils").AMPContext.step_optimizer = amp_step_optimizer
     mod = types.ModuleType("GAN_Variant1.losses.patchnce_cut")
     if nce_includes_all_negatives_from_minibatch:
-        mod.PatchNCELoss = functools.partial(PatchNCELoss, nce_includes_all_negatives_from_minibatch=True)
-        mod.compute_patchnce_loss = functools.partial(compute_patchnce_loss,
-                                                      nce_includes_all_negatives_from_minibatch=True)
+        kw = {"nce_includes_all_negatives_from_minibatch": True}
+        if negatives_group is not None:
+            kw["negatives_group"] = negatives_group
+        mod.PatchNCELoss = functools.partial(PatchNCELoss, **kw)
+        mod.compute_patchnce_loss = functools.partial(compute_patchnce_loss, **kw)
     else:
         mod.PatchNCELoss = PatchNCELoss
         mod.compute_patchnce_loss = compute_patchnce_loss

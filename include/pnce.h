@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define PNCE_ABI_VERSION 6
+#define PNCE_ABI_VERSION 7
 #define PNCE_MAX_LAYERS 8      /* nce_layers per call (reference config uses 5 ids -> 4 maps)   */
 #define PNCE_MAX_PATCHES 4096  /* P = min(num_patches, H*W)  patchnce_cut.py:60; argument check only: the
                                 * kernels take P <= 1024 (tensor cores, C <= 256) or P <= 1280 (fp32 CUDA cores),
@@ -153,7 +153,8 @@ int pnce_bwd_ex(const pnce_layer_t* layers, int n_layers, int batch, int dtype, 
  *   loss_l = mean over the N rows of CE(Z_i, i) (:91-94), the image guard of :97-99 applied to that single group (a
  *   non-finite group contributes 0 and its rows get a zero upstream gradient), total = sum_l loss_l / n_layers (:40).
  * d loss / d tgt keeps the factor 1 / (P B n_layers); keys carry no gradient (:142).  The N x N logits never leave the
- * SM (k_loss_tc_mb).  Under data parallelism the negatives are those of the caller's shard (as upstream CUT under DDP).
+ * SM (k_loss_tc_mb).  Under data parallelism the negatives are those of the caller's shard (as upstream CUT under DDP);
+ * the pnce_mb_shard_* calls below contrast with every rank's keys instead.
  * Tensor-core math modes only; P <= 1024, C <= 256 and B * round_up(P, 128) <= 65536 per layer (PNCE_ERR_UNSUPPORTED
  * otherwise).
  *   pnce_mb_workspace_bytes : bytes of the workspace pnce_mb_fwd needs
@@ -164,6 +165,35 @@ int pnce_mb_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch,
 int pnce_mb_fwd(const pnce_layer_t* layers, int n_layers, int batch, int dtype, int layout, float temperature,
                 int math_mode, void* dev_workspace, size_t workspace_bytes, void* dev_plan, size_t plan_bytes,
                 const unsigned long long* philox_seed_offset, float* dev_loss_out, int* dev_nonfinite, void* stream);
+
+/* ---- global negatives: minibatch negatives across data-parallel ranks (ABI 7) ---------------------------------------
+ * configs/train_gan_cutpp.yaml:80 (nce_includes_all_negatives_from_minibatch) with the batch sharded over `world` ranks,
+ * rank r holding global images r * batch_local ... r * batch_local + batch_local - 1, every rank using the same ids.
+ * Per layer, rank r's batch_local * P query rows are contrasted with the keys of ALL world * batch_local images
+ * (patchnce_cut.py:42-110 on the group of world * batch_local * P rows, row i's positive = the key of the same global
+ * (image, patch)); rank r's loss is the mean row CE over its own rows, so the mean of the ranks' losses is the one-GPU
+ * minibatch loss of the global batch, and d loss_r / d tgt_r divided by world is the one-GPU gradient of shard r.  The
+ * guard is global: a non-finite query row on any rank, or a non-finite key, zeroes the layer on every rank
+ * (dev_nonfinite[0] counts guarded layers).  The envelope is pnce_mb_fwd's, applied to the global batch.  The library
+ * has no collective of its own; the caller exchanges the slots:
+ *   pnce_mb_shard_workspace_bytes : total bytes, and where the `world` slots start (slot_offset, always
+ *                                   pnce_mb_workspace_bytes(batch_local)) and their stride (slot_bytes, 256-aligned)
+ *   pnce_mb_shard_keys            : the id prep (plan or Philox draw as in pnce_fwd_ex) and the gather; fills slot `rank`
+ *                                   with this rank's keys and its "a query row is non-finite" flags
+ *   -- the caller all-gathers the slot region [slot_offset, slot_offset + world * slot_bytes) in place --
+ *   pnce_mb_shard_loss            : logits, CE and d loss / d q over every slot's keys (k_loss_tc_mb_gn); the backward is
+ *                                   pnce_bwd_ex(batch_local) on the same workspace
+ * Keys carry no gradient (:142), so the backward needs no exchange.  world < 1, rank outside [0, world), dtype or layout
+ * out of range: PNCE_ERR_ARG; simt_f32 or a global batch outside the envelope: PNCE_ERR_UNSUPPORTED; NULL or short
+ * workspace: PNCE_ERR_WORKSPACE -- all before any CUDA call.                                                          */
+int pnce_mb_shard_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch_local, int world, size_t* bytes,
+                                  size_t* slot_offset, size_t* slot_bytes);
+int pnce_mb_shard_keys(const pnce_layer_t* layers, int n_layers, int batch_local, int dtype, int layout, int world,
+                       int rank, int math_mode, void* dev_workspace, size_t workspace_bytes, void* dev_plan,
+                       size_t plan_bytes, const unsigned long long* philox_seed_offset, void* stream);
+int pnce_mb_shard_loss(const pnce_layer_t* layers, int n_layers, int batch_local, int dtype, int layout, int world,
+                       int rank, float temperature, int math_mode, void* dev_workspace, size_t workspace_bytes,
+                       void* dev_plan, size_t plan_bytes, float* dev_loss_out, int* dev_nonfinite, void* stream);
 
 /* ---- north-star module split (SURVEY.md section 8b / row a13) ------------------------------ */
 
