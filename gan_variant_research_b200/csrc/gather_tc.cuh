@@ -159,6 +159,53 @@ __global__ void __launch_bounds__(kThreads) k_mb_qbad(const __grid_constant__ Pa
   if (__syncthreads_or(bad) && threadIdx.x == 0) flags[l] = 1;
 }
 
+// netF head with minibatch negatives (pnce_head_mb_fwd), after the head's second GEMM: the group guard needs a sampled
+// patch holding a NaN / Inf to make its layer non-finite, but the head's ReLU (fmaxf) turns a NaN row of X W1^T into
+// zeros, so the head's output would be finite.  The gather marks such a raw row in xqss / xkss (NaN partial sums of
+// squares); this kernel carries the mark onto the head output's sums of squares (chunk 0 of yqss / ykss), where the
+// loss kernel reads it as a non-finite row or key and guards the layer.  A marked query row of X is also zeroed: the
+// guarded layer's dY is zero, and dW1 = dH^T X must then be 0, not 0 * NaN.  One thread per (layer, image, slot).
+struct HeadGuardLayer {
+  const float* xqss;           // [B][nchunk][Ppad] of the raw patches (the gather's marks)
+  const float* xkss;
+  float* yqss;                 // [B][ncy][Ppad] of the head's output
+  float* ykss;
+  __nv_bfloat16* xq_hi;        // raw query rows: the row blob the gather writes (tile-major, 8-channel core matrices)
+  __nv_bfloat16* xq_lo;        // NULL in single-pass bf16
+  int P, Ppad, Cp8, nchunk, ncy;
+};
+struct HeadGuardLaunch {
+  HeadGuardLayer L[PNCE_MAX_LAYERS];
+  int B;
+};
+
+__global__ void __launch_bounds__(kThreads) k_head_mb_guard(const __grid_constant__ HeadGuardLaunch g) {
+  pdl_enter();
+  const HeadGuardLayer& L = g.L[blockIdx.y];
+  const long long r = (long long)blockIdx.x * kThreads + threadIdx.x;
+  if (r >= (long long)g.B * L.Ppad) return;
+  const int b = (int)(r / L.Ppad), p = (int)(r % L.Ppad);
+  if (p >= L.P) return;
+  bool bq = false, bk = false;
+  for (int s = 0; s < L.nchunk; ++s) {
+    const size_t i = ((size_t)b * L.nchunk + s) * L.Ppad + p;
+    const float q = __ldcg(L.xqss + i), k = __ldcg(L.xkss + i);
+    bq |= !(q == q);
+    bk |= !(k == k);
+  }
+  const float nan = __int_as_float(0x7fc00000);
+  if (bk) L.ykss[(size_t)b * L.ncy * L.Ppad + p] = nan;
+  if (bq) {
+    L.yqss[(size_t)b * L.ncy * L.Ppad + p] = nan;
+    for (int c8 = 0; c8 < L.Cp8; ++c8) {
+      const size_t cm = (((size_t)b * (L.Ppad >> 7) + (p >> 7)) * L.Cp8 + c8) * 16 + ((p & 127) >> 3);
+      const size_t off = cm * 64 + (size_t)(p & 7) * 8;
+      *reinterpret_cast<uint4*>(L.xq_hi + off) = make_uint4(0u, 0u, 0u, 0u);
+      if (L.xq_lo != nullptr) *reinterpret_cast<uint4*>(L.xq_lo + off) = make_uint4(0u, 0u, 0u, 0u);
+    }
+  }
+}
+
 // One CTA per layer: ids -> (sid, perm, rank, ustart, bitmap, prefix); CTA 0 also resets the
 // last-CTA counter and the protocol flag of the launch sequence.
 __global__ void __launch_bounds__(kThreads) k_prep(const __grid_constant__ Params p) {

@@ -1670,6 +1670,20 @@ static size_t carve_head(const pnce_layer_t* layers, int n_layers, int B, int nc
   return align_up(cv.off, 256);
 }
 
+// Minibatch negatives (pnce_head_mb_fwd) only: the gather's partial sums of squares of the raw patches, which mark a
+// non-finite patch for k_head_mb_guard.  Carved AFTER carve_head's layout, so that pnce_head_bwd_ex's carve sees the
+// offsets the forward used; with base == nullptr only the size is computed.
+static size_t carve_head_mb(const pnce_layer_t* layers, int n_layers, int B, void* base, Params* pg) {
+  Carver cv(base);
+  for (int l = 0; l < n_layers; ++l) {
+    const size_t Ppad = (layers[l].P + 127) / 128 * 128, nchunk = (layers[l].C + 31) / 32;
+    float* qss = cv.take<float>((size_t)B * nchunk * Ppad);
+    float* kss = cv.take<float>((size_t)B * nchunk * Ppad);
+    if (pg != nullptr) { pg->L[l].qss = qss; pg->L[l].kss = kss; }
+  }
+  return align_up(cv.off, 256);
+}
+
 static int launch_gemm(GemmLaunch& g, cudaStream_t st) {
   g.dbg = g_dbg.gemm_dbg;
   long long acc = 0;
@@ -1725,16 +1739,19 @@ int pnce_head_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batc
   return PNCE_OK;
 }
 
+// mb: minibatch negatives -- the loss launch is k_loss_tc_mb on the same virtual layers (see pnce_head_mb_fwd)
 static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch, int dtype,
                          int layout, int nc, float temperature, int math_mode, void* ws, size_t ws_bytes, float* loss_out,
-                         int* nonfinite, void* stream) {
+                         int* nonfinite, void* stream, bool mb = false) {
   int rc = check_head_args(layers, heads, n_layers, batch, dtype, nc, math_mode, ws, false);
   if (rc != PNCE_OK) return rc;
   if (loss_out == nullptr || !(temperature > 0.f)) return PNCE_ERR_ARG;
   if (layout != PNCE_LAYOUT_NCHW && layout != PNCE_LAYOUT_NHWC) return PNCE_ERR_ARG;
   const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
   static thread_local HeadPlan hp;
-  if (carve_head(layers, n_layers, batch, nc, x3, ws, &hp) > ws_bytes) return PNCE_ERR_WORKSPACE;
+  size_t need = carve_head(layers, n_layers, batch, nc, x3, ws, &hp);
+  if (mb) need += carve_head_mb(layers, n_layers, batch, static_cast<unsigned char*>(ws) + need, &hp.pg);
+  if (need > ws_bytes) return PNCE_ERR_WORKSPACE;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   Params& pg = hp.pg;
   Params& pl = hp.pl;
@@ -1745,6 +1762,7 @@ static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, i
   pg.nonfinite = pl.nonfinite = nonfinite;
   pg.b0 = pl.b0 = 0; pg.bn = pl.bn = batch;
   pg.nhwc = layout == PNCE_LAYOUT_NHWC ? 1 : 0;               // the maps; the head's output (pl) has no layout
+  pl.mb = mb ? 1 : 0;
   pl.trace = g_dbg.trace;
   // 1. ids -> sorted slots; weights -> operand blobs
   const bool fold = gather_tc_folds(pg);                      // small problems: the gather CTAs sort the ids themselves
@@ -1816,6 +1834,24 @@ static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, i
   }
   rc = launch_gemm(g, st);
   if (rc != PNCE_OK) return rc;
+  if (mb) {
+    // 4b. a non-finite raw patch -> a non-finite row / key of the head's output (the layer's group guard)
+    static thread_local HeadGuardLaunch gl;
+    memset(&gl, 0, sizeof(gl));
+    gl.B = batch;
+    long long most = 0;
+    for (int l = 0; l < n_layers; ++l) {
+      const LayerDev& G = pg.L[l];
+      const LayerDev& V = pl.L[l];
+      HeadGuardLayer& h = gl.L[l];
+      h.xqss = G.qss; h.xkss = G.kss; h.yqss = V.qss; h.ykss = V.kss;
+      h.xq_hi = hp.hb[l].xq[0]; h.xq_lo = x3 ? hp.hb[l].xq[1] : nullptr;
+      h.P = G.P; h.Ppad = G.Ppad; h.Cp8 = G.Cp / 8; h.nchunk = G.nchunk; h.ncy = nc / 32;
+      if ((long long)batch * G.Ppad > most) most = (long long)batch * G.Ppad;
+    }
+    launch_k(k_head_mb_guard, dim3((unsigned)((most + kThreads - 1) / kThreads), (unsigned)n_layers), kThreads, 0, st, gl);
+    PNCE_CUDA(cudaGetLastError());
+  }
   // 5. logits / diagonal CE / d loss / d Y (as a row blob) on the head's output
   int ctas = 0;
   for (int l = 0; l < n_layers; ++l) ctas += pl.L[l].Ppad / 128;
@@ -1951,6 +1987,42 @@ int pnce_head_bwd_params(const pnce_layer_t* layers, const pnce_head_t* heads, i
 int pnce_head_bwd_dense(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch, int dtype,
                         int nc, int math_mode, void* ws, size_t ws_bytes, const float* grad_out, void* stream) {
   return head_bwd_phases(2, layers, heads, n_layers, batch, dtype, nc, math_mode, ws, ws_bytes, grad_out, stream);
+}
+
+// ---- netF head with minibatch negatives ----------------------------------------------------------------------------
+// The head's second GEMM writes the key side (khi / klo, k2hi / k2lo, kss) per image in the key-blocked layout of the
+// gather, so the batch's key blobs are the one blob of B * Ppad keys k_loss_tc_mb walks.  k_loss_tc_mb reads nothing
+// carve_head lacks on the virtual layers: qss / kss ([B][nc / 32][Ppad], key norms folded per key block), qinv (B * P),
+// partial (B * max(Ppad / 128, 2) >= B * nparts), lossimg / valid (n_layers * B) and the counter; it writes d loss / d Y
+// into dyhi / dylo (dxT == nullptr: the epilogue's head branch stores no fp32 rows), and its last CTA zeroes the dY rows
+// of a guarded layer (valid = 0 for every image).  kinv is not used in this mode.  The one addition is carve_head_mb's
+// raw-patch sums of squares for k_head_mb_guard, after carve_head's layout: pnce_head_bwd_ex reads the workspace
+// unchanged.
+static bool head_mb_shapes_ok(const pnce_layer_t* layers, int n_layers, int B, int nc) {
+  if (!head_shapes_ok(layers, n_layers, nc)) return false;
+  for (int l = 0; l < n_layers; ++l)
+    if (!mb_keys_ok(B, layers[l].P)) return false;
+  return true;
+}
+
+int pnce_head_mb_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch, int nc, size_t* bytes) {
+  if (bytes == nullptr) return PNCE_ERR_ARG;
+  int rc = check_layers(layers, n_layers, batch);
+  if (rc != PNCE_OK) return rc;
+  if (!head_mb_shapes_ok(layers, n_layers, batch, nc)) return PNCE_ERR_UNSUPPORTED;
+  *bytes = carve_head(layers, n_layers, batch, nc, true, nullptr, nullptr) + carve_head_mb(layers, n_layers, batch, nullptr, nullptr);
+  return PNCE_OK;
+}
+
+int pnce_head_mb_fwd(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch, int dtype, int layout,
+                     int nc, float temperature, int math_mode, void* ws, size_t ws_bytes, float* loss_out,
+                     int* nonfinite, void* stream) {
+  if (math_mode == PNCE_MATH_SIMT_F32) return PNCE_ERR_UNSUPPORTED;
+  const int rc = check_layers(layers, n_layers, batch);
+  if (rc != PNCE_OK) return rc;
+  if (!head_mb_shapes_ok(layers, n_layers, batch, nc)) return PNCE_ERR_UNSUPPORTED;
+  return head_fwd_impl(layers, heads, n_layers, batch, dtype, layout, nc, temperature, math_mode, ws, ws_bytes, loss_out,
+                       nonfinite, stream, true);
 }
 
 

@@ -1397,15 +1397,17 @@ class PatchSampleF(nn.Module):
 
 class _HeadCall:
     """What the two fused head calls need that is not a differentiable input."""
-    __slots__ = ("src_feats", "ids_list", "temperature", "math", "dp_group")
+    __slots__ = ("src_feats", "ids_list", "temperature", "math", "dp_group", "mb")
 
-    def __init__(self, src_feats, ids_list, temperature, math, dp_group=None):
+    def __init__(self, src_feats, ids_list, temperature, math, dp_group=None, mb=False):
         self.src_feats, self.ids_list, self.temperature, self.math = src_feats, ids_list, float(temperature), math
         self.dp_group = dp_group      # process group whose ranks average the head gradients (None: single process)
+        self.mb = mb                  # minibatch negatives (pnce_head_mb_fwd; the per-image call at B = 1)
 
 
 def _head_fwd(plan, nc, tgt, params):
-    """pnce_head_fwd_ex on one set of maps and head parameters -> (workspace, out, state for _head_bwd)."""
+    """pnce_head_fwd_ex (pnce_head_mb_fwd with minibatch negatives) on one set of maps and head parameters
+    -> (workspace, out, state for _head_bwd)."""
     lib = _lib.load()
     n = len(tgt)
     src, ids = plan.src_feats, plan.ids_list
@@ -1419,12 +1421,13 @@ def _head_fwd(plan, nc, tgt, params):
         h.w1, h.b1, h.w2, h.b2 = (params[4 * l].data_ptr(), params[4 * l + 1].data_ptr(),
                                   params[4 * l + 2].data_ptr(), params[4 * l + 3].data_ptr())
     layout = _lib.LAYOUT_NHWC if _is_nhwc(tgt[0]) else _lib.LAYOUT_NCHW      # _prepare_maps made the layers uniform
-    key = (dev.index, dtype, layout, nc, tuple(t.shape for t in tgt), tuple(layers[l].P for l in range(n)))
+    mb = plan.mb and batch > 1        # B = 1: minibatch negatives ARE the per-image loss -- the per-image call, bit for bit
+    key = (dev.index, dtype, layout, nc, mb, tuple(t.shape for t in tgt), tuple(layers[l].P for l in range(n)))
     ws_bytes = _HEAD_WS_BYTES.get(key)
     if ws_bytes is None:
         nbytes = ctypes.c_size_t(0)
-        _lib.check(lib.pnce_head_workspace_bytes(layers, n, batch, nc, ctypes.byref(nbytes)),
-                   "pnce_head_workspace_bytes")
+        query = lib.pnce_head_mb_workspace_bytes if mb else lib.pnce_head_workspace_bytes
+        _lib.check(query(layers, n, batch, nc, ctypes.byref(nbytes)), "pnce_head_workspace_bytes")
         if len(_HEAD_WS_BYTES) > 256:
             _HEAD_WS_BYTES.clear()
         ws_bytes = _HEAD_WS_BYTES[key] = nbytes.value
@@ -1432,10 +1435,10 @@ def _head_fwd(plan, nc, tgt, params):
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         out = torch.empty(1 + n, dtype=torch.float32, device=dev)
         wq = _warn_queue(dev)
-        slot, flag_ptr = wq.acquire()
-        _lib.check(lib.pnce_head_fwd_ex(layers, heads, n, batch, dtype, layout, nc, plan.temperature, _MATH[plan.math],
-                                        ws.data_ptr(), ws_bytes, out.data_ptr(), flag_ptr or None,
-                                        _stream_ptr(dev)), "pnce_head_fwd")
+        slot, flag_ptr = wq.acquire(plan.mb)
+        fwd = lib.pnce_head_mb_fwd if mb else lib.pnce_head_fwd_ex
+        _lib.check(fwd(layers, heads, n, batch, dtype, layout, nc, plan.temperature, _MATH[plan.math],
+                       ws.data_ptr(), ws_bytes, out.data_ptr(), flag_ptr or None, _stream_ptr(dev)), "pnce_head_fwd")
     return ws, out, (ws_bytes, layout, dev, batch, dtype, heads)
 
 
@@ -1557,9 +1560,8 @@ def patchnce_with_head(netF: "PatchSampleF", src_feats, tgt_feats, temperature=0
     done, so it runs under the HBM-bound dense-gradient kernel (SURVEY.md section 8e).  Do not call
     ``allreduce_head_grads`` as well.
 
-    Per-image negatives only.  For minibatch negatives compose it as upstream CUT does:
-    ``PatchSampleF(use_mlp=True)`` for both sides, then
-    ``PatchNCELoss(nce_includes_all_negatives_from_minibatch=True)(feat_q, feat_k)`` on the two lists."""
+    Per-image negatives only.  For minibatch negatives (upstream CUT's ``nce_includes_all_negatives_from_minibatch``)
+    call ``patchnce_with_head_minibatch``, the same fused chain with every image's keys as negatives."""
     if fused is None:
         fused = fused_head_supported(netF, tgt_feats, num_patches) and (math or DEFAULT_MATH) != "simt_f32"
     if not fused:
@@ -1577,10 +1579,15 @@ def patchnce_with_head(netF: "PatchSampleF", src_feats, tgt_feats, temperature=0
     return loss, ids
 
 
-def _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group):
-    """Argument handling + id draw of one fused head call -> (plan, tgt maps, head parameters, ids)."""
+def _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group, mb=False):
+    """Argument handling + id draw of one fused head call -> (plan, tgt maps, head parameters, ids).
+    ``mb``: minibatch negatives -- the envelope (mb_check) is checked before anything touches the device."""
     if not fused_head_supported(netF, tgt_feats, num_patches):
         raise RuntimeError("fused head: nc must be 128 or 256, num_patches <= 1024 and C <= 256")
+    if mb:
+        p_list = ([int(i.numel()) for i in patch_ids] if patch_ids is not None else
+                  [patch_count(num_patches, f.shape[2] * f.shape[3]) for f in tgt_feats])
+        mb_check(tgt_feats[0].shape[0], [f.shape[1] for f in tgt_feats], p_list, math or DEFAULT_MATH)
     if not netF.mlp_init:
         netF.create_mlp(tgt_feats)
     src, tgt, _, uniform = _prepare_maps(src_feats, tgt_feats, math or DEFAULT_MATH, int(num_patches))
@@ -1594,9 +1601,35 @@ def _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids,
     if dp_group is not None:
         from . import dp
         dp_group = dp.resolve_group(dp_group)          # None when not initialised or world size 1
-    plan = _HeadCall(src, ids, temperature, math or DEFAULT_MATH, dp_group)
+    plan = _HeadCall(src, ids, temperature, math or DEFAULT_MATH, dp_group, mb)
     _warn_queue(tgt[0].device).poll()
     return plan, tgt, params, ids
+
+
+def patchnce_with_head_minibatch(netF: "PatchSampleF", src_feats, tgt_feats, temperature=0.07, num_patches=256,
+                                 patch_ids=None, math: Optional[str] = None, dp_group=None):
+    """``patchnce_with_head`` (fused path) with minibatch negatives -- upstream CUT's
+    ``nce_includes_all_negatives_from_minibatch`` on the head's output.  Returns ``(loss, ids)``.
+
+    Per layer, with the ids shared by the batch and N = B * P rows in image-major order:
+    ``q = normalize(netF(raw tgt patches))``, ``k = normalize(netF(raw src patches)).detach()``,
+    ``Z = clamp(q k^T / tau, -50, 50)`` (N x N), loss_l = mean over the N rows of CE(Z_i, i); the total is the mean over
+    the layers.  A non-finite layer contributes 0 and zero gradients (one warning per guarded layer); the head learns
+    through q only.  The whole chain -- gather, both Linear layers, normalisation, the N x N logits (which never reach
+    memory: k_loss_tc_mb), CE and the complete backward including the head gradients -- runs in the tcgen05 kernels of
+    libpnce.  At B = 1 it is ``patchnce_with_head``, bit for bit.  Same ids from the same generator state as
+    ``patchnce_with_head``.
+
+    ``dp_group``: as in ``patchnce_with_head`` -- the head gradients are averaged over the group, and the negatives are
+    the rank's own shard, as upstream CUT under DDP.
+
+    Envelope: nc = 128 or 256, tensor-core math (not simt_f32), C <= 256, P <= 1024 and B * round_up(P, 128) <= 65536
+    per layer.  Outside it a RuntimeError is raised before any launch; there is no other implementation to fall back to.
+    """
+    plan, tgt, params, ids = _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group,
+                                         mb=True)
+    loss = _FusedHeadPatchNCE.apply(plan, netF.nc, *tgt, *params)
+    return loss, ids
 
 
 def head_loss_and_grads(netF: "PatchSampleF", src_feats, tgt_feats, temperature=0.07, num_patches=256,
@@ -1609,11 +1642,28 @@ def head_loss_and_grads(netF: "PatchSampleF", src_feats, tgt_feats, temperature=
     there.  Same ids, kernels and values as the autograd route; no ``Function.apply``, no engine hand-off and no
     ``AccumulateGrad`` per parameter (20 of them for five layers): at the batches the reference trains with, that
     host work is longer than the GPU's (DESIGN.md 4.5).  For loops that drive the generator's backward themselves:
-    ``torch.autograd.backward(tgt_feats, grads)``.  Per-image negatives only (see ``patchnce_with_head`` for the
-    minibatch composition)."""
+    ``torch.autograd.backward(tgt_feats, grads)``.  Per-image negatives only: ``head_minibatch_loss_and_grads`` is the
+    counterpart with minibatch negatives."""
     if (math or DEFAULT_MATH) == "simt_f32":
         raise RuntimeError("head_loss_and_grads runs the tensor-core head only")
     plan, tgt, params, ids = _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group)
+    return _head_loss_and_grads(netF, plan, tgt, params, ids, grad_output)
+
+
+def head_minibatch_loss_and_grads(netF: "PatchSampleF", src_feats, tgt_feats, temperature=0.07, num_patches=256,
+                                  patch_ids=None, math: Optional[str] = None, grad_output: Optional[torch.Tensor] = None,
+                                  dp_group=None):
+    """``patchnce_with_head_minibatch`` and its complete backward in ONE call, without autograd: returns
+    ``(loss, [d (grad_output * loss) / d tgt_feats[l]], ids)`` and ACCUMULATES the head gradients into ``p.grad`` of
+    netF's parameters exactly as ``head_loss_and_grads`` does.  Same ids, kernels and values as
+    ``patchnce_with_head_minibatch(...)`` followed by ``loss.backward(grad_output)``; same envelope and errors."""
+    plan, tgt, params, ids = _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group,
+                                         mb=True)
+    return _head_loss_and_grads(netF, plan, tgt, params, ids, grad_output)
+
+
+def _head_loss_and_grads(netF, plan, tgt, params, ids, grad_output):
+    """The body of the autograd-free head entries: forward, backward, accumulation into ``p.grad``."""
     dev = tgt[0].device
     with torch.no_grad():
         tgt = [t.detach() for t in tgt]

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define PNCE_ABI_VERSION 7
+#define PNCE_ABI_VERSION 8
 #define PNCE_MAX_LAYERS 8      /* nce_layers per call (reference config uses 5 ids -> 4 maps)   */
 #define PNCE_MAX_PATCHES 4096  /* P = min(num_patches, H*W)  patchnce_cut.py:60; argument check only: the
                                 * kernels take P <= 1024 (tensor cores, C <= 256) or P <= 1280 (fp32 CUDA cores),
@@ -305,6 +305,26 @@ int pnce_head_fwd_ex(const pnce_layer_t* layers, const pnce_head_t* heads, int n
 int pnce_head_bwd_ex(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch, int dtype, int layout,
                      int phases, int nc, int math_mode, void* dev_workspace, size_t workspace_bytes,
                      const float* dev_grad_out, void* stream);
+
+/* ---- netF head with minibatch negatives (ABI 8) -----------------------------------------------------------------------
+ * The law of pnce_mb_fwd on the head's output: per layer, with N = B * P rows in image-major order and the ids shared by
+ * the batch, q = normalize(netF(raw tgt patches)), k = normalize(netF(raw src patches)) (no gradient),
+ * Z = clamp(q k^T / tau, -50, 50) (N x N), loss_l = mean over the N rows of CE(Z_i, i), total = sum_l loss_l / n_layers.
+ * A non-finite layer contributes 0 and its rows get a zero upstream gradient (so that layer's head gradients are 0);
+ * dev_nonfinite[0] counts the guarded LAYERS.  d loss / d tgt keeps the factor 1 / (B P n_layers); the head learns
+ * through q only.  At B = 1 this is pnce_head_fwd_ex's loss.
+ *   pnce_head_mb_workspace_bytes : bytes of the workspace; PNCE_ERR_UNSUPPORTED outside the head envelope (nc = 128 or
+ *                                  256, P <= 1024, C <= 256) or the minibatch one (B * round_up(P, 128) <= 65536)
+ *   pnce_head_mb_fwd             : the arguments of pnce_head_fwd_ex; the same prep, weight blobs, gather and head
+ *                                  GEMMs, then the minibatch loss kernel (k_loss_tc_mb).  simt_f32 and shapes outside
+ *                                  the envelope: PNCE_ERR_UNSUPPORTED before any CUDA call.
+ * A sampled patch (either side) holding a NaN / Inf makes its layer non-finite, as in torch, where ReLU keeps the NaN.
+ * The backward is pnce_head_bwd_ex (any phases) on the same workspace, layout and math mode; the workspace is
+ * pnce_head_workspace_bytes' layout followed by the raw patches' sums of squares.                                     */
+int pnce_head_mb_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch, int nc, size_t* bytes);
+int pnce_head_mb_fwd(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch, int dtype, int layout,
+                     int nc, float temperature, int math_mode, void* dev_workspace, size_t workspace_bytes,
+                     float* dev_loss_out, int* dev_nonfinite, void* stream);
 
 /* ---- PatchSampleF(use_mlp=True).forward(feats, num_patches, patch_ids) as a module of its own (north_star's netF
  * signature; absent from the reference, SURVEY.md section 8 row a13): for every map, raw gather -> Linear(C_l, nc) ->
