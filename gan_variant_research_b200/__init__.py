@@ -17,10 +17,12 @@ from .patchnce import (  # noqa: F401
     fused_patchnce,
     gradient_is_compressed,
     head_loss_and_grads,
+    head_global_negatives_loss_and_grads,
     head_minibatch_loss_and_grads,
     install_reference_shim,
     patch_count,
     patchnce_with_head,
+    patchnce_with_head_global_negatives,
     patchnce_with_head_minibatch,
     pinned_as_device,
     poll_nonfinite_warnings,
@@ -38,7 +40,8 @@ __all__ = [
     "PatchNCELoss", "PatchSampleF", "compute_patchnce_loss", "fused_patchnce", "rows_patchnce", "rows_patchnce_multi",
     "draw_patch_ids", "draw_patch_ids_all", "draw_ids", "pinned_as_device", "patch_count", "install_reference_shim", "poll_nonfinite_warnings",
     "DEFAULT_MATH", "patchnce_with_head", "head_loss_and_grads", "patchnce_with_head_minibatch",
-    "head_minibatch_loss_and_grads", "set_gradient_compression", "gradient_is_compressed", "allreduce_head_grads", "broadcast_patch_ids", "shard_batch", "GradReducer", "EMA",
+    "head_minibatch_loss_and_grads", "patchnce_with_head_global_negatives", "head_global_negatives_loss_and_grads",
+    "set_gradient_compression", "gradient_is_compressed", "allreduce_head_grads", "broadcast_patch_ids", "shard_batch", "GradReducer", "EMA",
     "EncoderFeatureCache", "enable_encoder_feature_reuse", "FusedAdamStep", "amp_step_optimizer",
     "DiffAugment", "discriminator_hinge_loss", "generator_hinge_loss",
 ]

@@ -11,7 +11,7 @@ MATH_SIMT_F32, MATH_TC_BF16X3, MATH_TC_BF16 = 0, 1, 2
 MAX_LAYERS = 8
 MAX_PATCHES = 4096
 MAX_CHANNELS = 1024
-ABI_VERSION = 8
+ABI_VERSION = 9
 LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
 
 EXPORTS = [
@@ -27,6 +27,7 @@ EXPORTS = [
     "pnce_mb_workspace_bytes", "pnce_mb_fwd", "pnce_rows_mb_workspace_bytes", "pnce_rows_mb_fwd_bwd",
     "pnce_mb_shard_workspace_bytes", "pnce_mb_shard_keys", "pnce_mb_shard_loss",
     "pnce_head_mb_workspace_bytes", "pnce_head_mb_fwd",
+    "pnce_head_mb_shard_workspace_bytes", "pnce_head_mb_shard_keys", "pnce_head_mb_shard_loss",
 ]
 
 
@@ -121,6 +122,12 @@ def load():
                                      vp, sz, vp, vp]
     lib.pnce_head_mb_workspace_bytes.argtypes = lib.pnce_head_workspace_bytes.argtypes
     lib.pnce_head_mb_fwd.argtypes = lib.pnce_head_fwd_ex.argtypes
+    lib.pnce_head_mb_shard_workspace_bytes.argtypes = [ctypes.POINTER(PnceLayer), i32, i32, i32, i32, ctypes.POINTER(sz),
+                                                       ctypes.POINTER(sz), ctypes.POINTER(sz)]
+    lib.pnce_head_mb_shard_keys.argtypes = [ctypes.POINTER(PnceLayer), ctypes.POINTER(PnceHead), i32, i32, i32, i32, i32,
+                                            i32, i32, i32, vp, sz, vp, vp]
+    lib.pnce_head_mb_shard_loss.argtypes = [ctypes.POINTER(PnceLayer), ctypes.POINTER(PnceHead), i32, i32, i32, i32, i32,
+                                            i32, i32, f32, i32, vp, sz, vp, vp, vp]
     for fn in (lib.pnce_head_bwd, lib.pnce_head_bwd_params, lib.pnce_head_bwd_dense):
         fn.argtypes = [ctypes.POINTER(PnceLayer), ctypes.POINTER(PnceHead), i32, i32, i32, i32, i32, vp, sz, vp, vp]
     lib.pnce_netf_workspace_bytes.argtypes = [ctypes.POINTER(PnceSample), i32, i32, i32, ctypes.POINTER(sz)]

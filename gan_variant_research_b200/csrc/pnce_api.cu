@@ -1739,20 +1739,9 @@ int pnce_head_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batc
   return PNCE_OK;
 }
 
-// mb: minibatch negatives -- the loss launch is k_loss_tc_mb on the same virtual layers (see pnce_head_mb_fwd)
-static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch, int dtype,
-                         int layout, int nc, float temperature, int math_mode, void* ws, size_t ws_bytes, float* loss_out,
-                         int* nonfinite, void* stream, bool mb = false) {
-  int rc = check_head_args(layers, heads, n_layers, batch, dtype, nc, math_mode, ws, false);
-  if (rc != PNCE_OK) return rc;
-  if (loss_out == nullptr || !(temperature > 0.f)) return PNCE_ERR_ARG;
-  if (layout != PNCE_LAYOUT_NCHW && layout != PNCE_LAYOUT_NHWC) return PNCE_ERR_ARG;
-  const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
-  static thread_local HeadPlan hp;
-  size_t need = carve_head(layers, n_layers, batch, nc, x3, ws, &hp);
-  if (mb) need += carve_head_mb(layers, n_layers, batch, static_cast<unsigned char*>(ws) + need, &hp.pg);
-  if (need > ws_bytes) return PNCE_ERR_WORKSPACE;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+// The Params fields of a head forward that the carve leaves open (both parts below read them).
+static void head_fwd_setup(HeadPlan& hp, int batch, int dtype, int layout, int math_mode, float temperature,
+                           float* loss_out, int* nonfinite, bool mb) {
   Params& pg = hp.pg;
   Params& pl = hp.pl;
   pg.dtype = pl.dtype = dtype;
@@ -1764,6 +1753,16 @@ static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, i
   pg.nhwc = layout == PNCE_LAYOUT_NHWC ? 1 : 0;               // the maps; the head's output (pl) has no layout
   pl.mb = mb ? 1 : 0;
   pl.trace = g_dbg.trace;
+}
+
+// Keys part of the head forward: steps 1-4b, up to the head's output on both sides.  The key side of the second GEMM
+// (khi / klo, k2hi / k2lo, kss) and k_head_mb_guard's key marks go to the blobs of kdst's layers: the virtual layers'
+// own (hp.pl), or a slot of the global-negatives workspace (pnce_head_mb_shard_keys).
+static int head_fwd_keys(HeadPlan& hp, const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch,
+                         int nc, bool x3, bool mb, int* nonfinite, const Params& kdst, cudaStream_t st) {
+  Params& pg = hp.pg;
+  Params& pl = hp.pl;
+  int rc = PNCE_OK;
   // 1. ids -> sorted slots; weights -> operand blobs
   const bool fold = gather_tc_folds(pg);                      // small problems: the gather CTAs sort the ids themselves
   if (!fold) rc = launch_prep(pg, st);
@@ -1821,6 +1820,7 @@ static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, i
     const HeadLayerBufs& hb = hp.hb[l];
     const LayerDev& G = pg.L[l];
     const LayerDev& V = pl.L[l];
+    const LayerDev& K = kdst.L[l];
     for (int side = 0; side < 2; ++side) {
       GemmProb& pr = g.pr[g.n++];
       pr.a_hi = side ? hb.hq[0] : hb.hk[0]; pr.a_lo = side ? hb.hq[1] : hb.hk[1];
@@ -1829,7 +1829,7 @@ static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, i
       pr.K = nc; pr.N = nc; pr.tiles = batch * (G.Ppad / 128); pr.mode = side ? GM_YQ : GM_YK;
       pr.P = G.P; pr.Ppad = G.Ppad; pr.halves = G.Ppad / 128; pr.C = nc;
       if (side) { pr.o_hi = V.qhi; pr.o_lo = V.qlo; pr.ss = V.qss; }
-      else { pr.k_hi = V.khi; pr.k_lo = V.klo; pr.k2_hi = V.k2hi; pr.k2_lo = V.k2lo; pr.ss = V.kss; }
+      else { pr.k_hi = K.khi; pr.k_lo = K.klo; pr.k2_hi = K.k2hi; pr.k2_lo = K.k2lo; pr.ss = K.kss; }
     }
   }
   rc = launch_gemm(g, st);
@@ -1844,7 +1844,7 @@ static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, i
       const LayerDev& G = pg.L[l];
       const LayerDev& V = pl.L[l];
       HeadGuardLayer& h = gl.L[l];
-      h.xqss = G.qss; h.xkss = G.kss; h.yqss = V.qss; h.ykss = V.kss;
+      h.xqss = G.qss; h.xkss = G.kss; h.yqss = V.qss; h.ykss = kdst.L[l].kss;
       h.xq_hi = hp.hb[l].xq[0]; h.xq_lo = x3 ? hp.hb[l].xq[1] : nullptr;
       h.P = G.P; h.Ppad = G.Ppad; h.Cp8 = G.Cp / 8; h.nchunk = G.nchunk; h.ncy = nc / 32;
       if ((long long)batch * G.Ppad > most) most = (long long)batch * G.Ppad;
@@ -1852,11 +1852,35 @@ static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, i
     launch_k(k_head_mb_guard, dim3((unsigned)((most + kThreads - 1) / kThreads), (unsigned)n_layers), kThreads, 0, st, gl);
     PNCE_CUDA(cudaGetLastError());
   }
-  // 5. logits / diagonal CE / d loss / d Y (as a row blob) on the head's output
+  return PNCE_OK;
+}
+
+// Loss part of the head forward: step 5, logits / diagonal CE / d loss / d Y (as a row blob) on the head's output.
+static int head_fwd_loss(Params& pl, int batch, cudaStream_t st) {
   int ctas = 0;
-  for (int l = 0; l < n_layers; ++l) ctas += pl.L[l].Ppad / 128;
+  for (int l = 0; l < pl.n_layers; ++l) ctas += pl.L[l].Ppad / 128;
   pl.total_ctas = (unsigned)(batch * ctas);
   return launch_loss_tc(pl, st);
+}
+
+// mb: minibatch negatives -- the loss launch is k_loss_tc_mb on the same virtual layers (see pnce_head_mb_fwd)
+static int head_fwd_impl(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch, int dtype,
+                         int layout, int nc, float temperature, int math_mode, void* ws, size_t ws_bytes, float* loss_out,
+                         int* nonfinite, void* stream, bool mb = false) {
+  int rc = check_head_args(layers, heads, n_layers, batch, dtype, nc, math_mode, ws, false);
+  if (rc != PNCE_OK) return rc;
+  if (loss_out == nullptr || !(temperature > 0.f)) return PNCE_ERR_ARG;
+  if (layout != PNCE_LAYOUT_NCHW && layout != PNCE_LAYOUT_NHWC) return PNCE_ERR_ARG;
+  const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
+  static thread_local HeadPlan hp;
+  size_t need = carve_head(layers, n_layers, batch, nc, x3, ws, &hp);
+  if (mb) need += carve_head_mb(layers, n_layers, batch, static_cast<unsigned char*>(ws) + need, &hp.pg);
+  if (need > ws_bytes) return PNCE_ERR_WORKSPACE;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  head_fwd_setup(hp, batch, dtype, layout, math_mode, temperature, loss_out, nonfinite, mb);
+  rc = head_fwd_keys(hp, layers, heads, n_layers, batch, nc, x3, mb, nonfinite, hp.pl, st);
+  if (rc != PNCE_OK) return rc;
+  return head_fwd_loss(hp.pl, batch, st);
 }
 
 // phases: bit 0 = head backward proper (dH, dX, weight / bias gradients), bit 1 = dense d tgt_feat
@@ -2023,6 +2047,128 @@ int pnce_head_mb_fwd(const pnce_layer_t* layers, const pnce_head_t* heads, int n
   if (!head_mb_shapes_ok(layers, n_layers, batch, nc)) return PNCE_ERR_UNSUPPORTED;
   return head_fwd_impl(layers, heads, n_layers, batch, dtype, layout, nc, temperature, math_mode, ws, ws_bytes, loss_out,
                        nonfinite, stream, true);
+}
+
+// ---- netF head with global negatives: minibatch negatives over the shards of every rank ------------------------------
+// Workspace: the prefix pnce_head_mb_workspace_bytes(batch_local) -- carve_head, then carve_head_mb, exactly what
+// pnce_head_mb_fwd lays out and pnce_head_bwd_ex reads -- followed by `world` slots in the format of pnce_mb_shard_*
+// (carve_mb_slot on the virtual layers, C = nc).  The second GEMM writes this rank's keys straight into its slot and
+// k_loss_tc_mb_gn reads every slot's; carve_head's own key blobs of the virtual layers stay unused in this mode (trimming
+// them would move the offsets the backward reads).
+//
+// The query flags: k_mb_qbad on the virtual layers, i.e. "a NaN among the partial sums of squares of a query row of the
+// head's output".  That is exactly the loss kernel's own row test (badq: the sum of the row's partials is NaN), because
+// every partial is finite or NaN: libpnce.so runs k_gemm_tc_p (g_dbg.no_persist is a constexpr 0), whose GM_YQ / GM_YK
+// epilogue stores NaN for a 32-channel chunk whose sum of squares is not finite (gemm_tc_persist.cuh, isfinite(ssum));
+// k_head_mb_guard stores NaN on chunk 0 for a non-finite raw patch; padding rows are exactly 0.  (k_gemm_tc, reachable
+// only through the experiment build's knob 6, stores +Inf for an overflowing chunk: not covered.)  An unflagged row and
+// key then have norms below 5.2e19, and their logit is non-finite only when q . k overflows fp32, i.e. both norms above
+// 6.5e18: the one window where the owning rank guards alone (DESIGN.md 4.14).
+static void head_virtual_layers(const pnce_layer_t* layers, int n_layers, int nc, pnce_layer_t* out) {
+  for (int l = 0; l < n_layers; ++l) {
+    out[l] = layers[l];
+    out[l].C = nc;
+  }
+}
+
+// The checks of the two shard calls, all before any CUDA call, then the carve of the prefix into hp.  *prefix: the
+// slots' offset; *slot_bytes: their stride; vl: the virtual layers (C = nc) the slots are carved on.
+static int head_shard_plan(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch_local,
+                           int dtype, int layout, int nc, int world, int rank, int math_mode, void* ws, size_t ws_bytes,
+                           HeadPlan& hp, pnce_layer_t* vl, size_t* prefix, size_t* slot_bytes) {
+  int rc = check_layers(layers, n_layers, batch_local);
+  if (rc != PNCE_OK) return rc;
+  if (world < 1 || rank < 0 || rank >= world) return PNCE_ERR_ARG;
+  if (dtype < PNCE_F32 || dtype > PNCE_BF16) return PNCE_ERR_ARG;
+  if (layout != PNCE_LAYOUT_NCHW && layout != PNCE_LAYOUT_NHWC) return PNCE_ERR_ARG;
+  if (math_mode < PNCE_MATH_SIMT_F32 || math_mode > PNCE_MATH_TC_BF16) return PNCE_ERR_ARG;
+  if (heads == nullptr) return PNCE_ERR_ARG;
+  for (int l = 0; l < n_layers; ++l)
+    if (!heads[l].w1 || !heads[l].b1 || !heads[l].w2 || !heads[l].b2) return PNCE_ERR_ARG;
+  if (math_mode == PNCE_MATH_SIMT_F32) return PNCE_ERR_UNSUPPORTED;
+  if ((long long)world * batch_local > 0x7fffffffLL || !head_mb_shapes_ok(layers, n_layers, world * batch_local, nc))
+    return PNCE_ERR_UNSUPPORTED;                               // the envelope of the GLOBAL batch
+  rc = check_alignment(layers, n_layers, dtype, false);
+  if (rc != PNCE_OK) return rc;
+  if (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 255u)) return PNCE_ERR_WORKSPACE;
+  head_virtual_layers(layers, n_layers, nc, vl);
+  *prefix = carve_head(layers, n_layers, batch_local, nc, true, nullptr, nullptr) +
+            carve_head_mb(layers, n_layers, batch_local, nullptr, nullptr);
+  *slot_bytes = carve_mb_slot(vl, n_layers, batch_local, true, nullptr, nullptr);
+  if (*prefix + (size_t)world * *slot_bytes > ws_bytes) return PNCE_ERR_WORKSPACE;
+  const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
+  const size_t used = carve_head(layers, n_layers, batch_local, nc, x3, ws, &hp);
+  carve_head_mb(layers, n_layers, batch_local, static_cast<unsigned char*>(ws) + used, &hp.pg);
+  return PNCE_OK;
+}
+
+int pnce_head_mb_shard_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch_local, int world, int nc,
+                                       size_t* bytes, size_t* slot_offset, size_t* slot_bytes) {
+  if (bytes == nullptr || slot_offset == nullptr || slot_bytes == nullptr) return PNCE_ERR_ARG;
+  const int rc = check_layers(layers, n_layers, batch_local);
+  if (rc != PNCE_OK) return rc;
+  if (world < 1) return PNCE_ERR_ARG;
+  if ((long long)world * batch_local > 0x7fffffffLL || !head_mb_shapes_ok(layers, n_layers, world * batch_local, nc))
+    return PNCE_ERR_UNSUPPORTED;
+  pnce_layer_t vl[PNCE_MAX_LAYERS];
+  head_virtual_layers(layers, n_layers, nc, vl);
+  *slot_offset = carve_head(layers, n_layers, batch_local, nc, true, nullptr, nullptr) +
+                 carve_head_mb(layers, n_layers, batch_local, nullptr, nullptr);
+  *slot_bytes = carve_mb_slot(vl, n_layers, batch_local, true, nullptr, nullptr);
+  *bytes = *slot_offset + (size_t)world * *slot_bytes;
+  return PNCE_OK;
+}
+
+int pnce_head_mb_shard_keys(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch_local,
+                            int dtype, int layout, int nc, int world, int rank, int math_mode, void* ws,
+                            size_t ws_bytes, int* nonfinite, void* stream) {
+  static thread_local HeadPlan hp;
+  static thread_local Params kd;                               // slot `rank`: where the keys and the flags go
+  pnce_layer_t vl[PNCE_MAX_LAYERS];
+  size_t prefix = 0, slot_bytes = 0;
+  int rc = head_shard_plan(layers, heads, n_layers, batch_local, dtype, layout, nc, world, rank, math_mode, ws, ws_bytes,
+                           hp, vl, &prefix, &slot_bytes);
+  if (rc != PNCE_OK) return rc;
+  const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
+  memset(&kd, 0, sizeof(kd));
+  carve_mb_slot(vl, n_layers, batch_local, x3, static_cast<unsigned char*>(ws) + prefix + (size_t)rank * slot_bytes, &kd);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  head_fwd_setup(hp, batch_local, dtype, layout, math_mode, 1.0f, nullptr, nonfinite, true);
+  rc = head_fwd_keys(hp, layers, heads, n_layers, batch_local, nc, x3, true, nonfinite, kd, st);
+  if (rc != PNCE_OK) return rc;
+  // this rank's "a query row is non-finite" flags, next to its keys (see above for why k_mb_qbad is exact here)
+  const Params& pl = hp.pl;
+  int* flags = const_cast<int*>(kd.qbad);
+  PNCE_CUDA(cudaMemsetAsync(flags, 0, PNCE_MAX_LAYERS * sizeof(int), st));
+  long long most = 1;
+  for (int l = 0; l < n_layers; ++l) {
+    const long long n = (long long)batch_local * pl.L[l].nchunk * pl.L[l].Ppad;
+    if ((n + kMbQbadFloats - 1) / kMbQbadFloats > most) most = (n + kMbQbadFloats - 1) / kMbQbadFloats;
+  }
+  if (most > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
+  launch_k<2>(k_mb_qbad, dim3((unsigned)most, (unsigned)n_layers), kThreads, 0, st, pl, flags);
+  PNCE_CUDA(cudaGetLastError());
+  return PNCE_OK;
+}
+
+int pnce_head_mb_shard_loss(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch_local,
+                            int dtype, int layout, int nc, int world, int rank, float temperature, int math_mode,
+                            void* ws, size_t ws_bytes, float* loss_out, int* nonfinite, void* stream) {
+  static thread_local HeadPlan hp;
+  pnce_layer_t vl[PNCE_MAX_LAYERS];
+  size_t prefix = 0, slot_bytes = 0;
+  int rc = head_shard_plan(layers, heads, n_layers, batch_local, dtype, layout, nc, world, rank, math_mode, ws, ws_bytes,
+                           hp, vl, &prefix, &slot_bytes);
+  if (rc != PNCE_OK) return rc;
+  if (loss_out == nullptr || !(temperature > 0.f)) return PNCE_ERR_ARG;
+  head_fwd_setup(hp, batch_local, dtype, layout, math_mode, temperature, loss_out, nonfinite, true);
+  // the virtual layers' key blobs and qbad: slot 0 of `world` (k_loss_tc_mb_gn steps to slot w by w * kslot)
+  carve_mb_slot(vl, n_layers, batch_local, math_mode == PNCE_MATH_TC_BF16X3, static_cast<unsigned char*>(ws) + prefix,
+                &hp.pl);
+  hp.pl.kworld = world;
+  hp.pl.kimg0 = rank * batch_local;
+  hp.pl.kslot = slot_bytes;
+  return head_fwd_loss(hp.pl, batch_local, static_cast<cudaStream_t>(stream));
 }
 
 

@@ -1397,17 +1397,19 @@ class PatchSampleF(nn.Module):
 
 class _HeadCall:
     """What the two fused head calls need that is not a differentiable input."""
-    __slots__ = ("src_feats", "ids_list", "temperature", "math", "dp_group", "mb")
+    __slots__ = ("src_feats", "ids_list", "temperature", "math", "dp_group", "mb", "group", "world")
 
-    def __init__(self, src_feats, ids_list, temperature, math, dp_group=None, mb=False):
+    def __init__(self, src_feats, ids_list, temperature, math, dp_group=None, mb=False, group=None, world=1):
         self.src_feats, self.ids_list, self.temperature, self.math = src_feats, ids_list, float(temperature), math
         self.dp_group = dp_group      # process group whose ranks average the head gradients (None: single process)
         self.mb = mb                  # minibatch negatives (pnce_head_mb_fwd; the per-image call at B = 1)
+        self.group = group            # global negatives: the process group of `world` ranks the keys are gathered over
+        self.world = world            # > 1: pnce_head_mb_shard_*; 1: the rank's own batch
 
 
 def _head_fwd(plan, nc, tgt, params):
-    """pnce_head_fwd_ex (pnce_head_mb_fwd with minibatch negatives) on one set of maps and head parameters
-    -> (workspace, out, state for _head_bwd)."""
+    """pnce_head_fwd_ex (pnce_head_mb_fwd with minibatch negatives, pnce_head_mb_shard_* with global negatives) on one
+    set of maps and head parameters -> (workspace, out, state for _head_bwd)."""
     lib = _lib.load()
     n = len(tgt)
     src, ids = plan.src_feats, plan.ids_list
@@ -1421,25 +1423,56 @@ def _head_fwd(plan, nc, tgt, params):
         h.w1, h.b1, h.w2, h.b2 = (params[4 * l].data_ptr(), params[4 * l + 1].data_ptr(),
                                   params[4 * l + 2].data_ptr(), params[4 * l + 3].data_ptr())
     layout = _lib.LAYOUT_NHWC if _is_nhwc(tgt[0]) else _lib.LAYOUT_NCHW      # _prepare_maps made the layers uniform
-    mb = plan.mb and batch > 1        # B = 1: minibatch negatives ARE the per-image loss -- the per-image call, bit for bit
-    key = (dev.index, dtype, layout, nc, mb, tuple(t.shape for t in tgt), tuple(layers[l].P for l in range(n)))
+    world = plan.world
+    # B = 1 on one rank: minibatch negatives ARE the per-image loss -- the per-image call, bit for bit.  Under global
+    # negatives the test is on the GLOBAL batch: a shard of one image still has world - 1 images of negatives elsewhere.
+    mb = plan.mb and (batch > 1 or world > 1)
+    key = (dev.index, dtype, layout, nc, mb, tuple(t.shape for t in tgt), tuple(layers[l].P for l in range(n)), world)
     ws_bytes = _HEAD_WS_BYTES.get(key)
     if ws_bytes is None:
-        nbytes = ctypes.c_size_t(0)
-        query = lib.pnce_head_mb_workspace_bytes if mb else lib.pnce_head_workspace_bytes
-        _lib.check(query(layers, n, batch, nc, ctypes.byref(nbytes)), "pnce_head_workspace_bytes")
-        if len(_HEAD_WS_BYTES) > 256:
+        if len(_HEAD_WS_BYTES) > 256:       # a caller cycling through many shapes: do not grow without bound
             _HEAD_WS_BYTES.clear()
+            _HEAD_SLOTS.clear()
+        nbytes = ctypes.c_size_t(0)
+        if world > 1:
+            so, sb = ctypes.c_size_t(0), ctypes.c_size_t(0)
+            _lib.check(lib.pnce_head_mb_shard_workspace_bytes(layers, n, batch, world, nc, ctypes.byref(nbytes),
+                                                              ctypes.byref(so), ctypes.byref(sb)),
+                       "pnce_head_mb_shard_workspace_bytes")
+            _HEAD_SLOTS[key] = (so.value, sb.value)
+        else:
+            query = lib.pnce_head_mb_workspace_bytes if mb else lib.pnce_head_workspace_bytes
+            _lib.check(query(layers, n, batch, nc, ctypes.byref(nbytes)), "pnce_head_workspace_bytes")
         ws_bytes = _HEAD_WS_BYTES[key] = nbytes.value
     with _on_device(dev):
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         out = torch.empty(1 + n, dtype=torch.float32, device=dev)
         wq = _warn_queue(dev)
         slot, flag_ptr = wq.acquire(plan.mb)
-        fwd = lib.pnce_head_mb_fwd if mb else lib.pnce_head_fwd_ex
-        _lib.check(fwd(layers, heads, n, batch, dtype, layout, nc, plan.temperature, _MATH[plan.math],
-                       ws.data_ptr(), ws_bytes, out.data_ptr(), flag_ptr or None, _stream_ptr(dev)), "pnce_head_fwd")
+        if world > 1:
+            _head_fwd_global(lib, plan, nc, key, layers, heads, batch, dtype, layout, ws, ws_bytes, out, flag_ptr or None,
+                             _stream_ptr(dev))
+        else:
+            fwd = lib.pnce_head_mb_fwd if mb else lib.pnce_head_fwd_ex
+            _lib.check(fwd(layers, heads, n, batch, dtype, layout, nc, plan.temperature, _MATH[plan.math],
+                           ws.data_ptr(), ws_bytes, out.data_ptr(), flag_ptr or None, _stream_ptr(dev)), "pnce_head_fwd")
     return ws, out, (ws_bytes, layout, dev, batch, dtype, heads)
+
+
+def _head_fwd_global(lib, plan, nc, key, layers, heads, batch, dtype, layout, ws, ws_bytes, out, flag_ptr, st):
+    """Global negatives: this rank's head output up to its keys, which go into its slot of the workspace; the all-gather
+    of the slots (the one collective of the mode; keys carry no gradient, so the backward is local); then the loss over
+    every rank's keys."""
+    from . import dp
+    n, world, math = len(layers), plan.world, _MATH[plan.math]
+    rank = dist.get_rank(plan.group)
+    so, sb = _HEAD_SLOTS[key]
+    _lib.check(lib.pnce_head_mb_shard_keys(layers, heads, n, batch, dtype, layout, nc, world, rank, math, ws.data_ptr(),
+                                           ws_bytes, flag_ptr, st), "pnce_head_mb_shard_keys")
+    dp.allgather_slots_(ws[so:so + world * sb], rank, plan.group)
+    _lib.check(lib.pnce_head_mb_shard_loss(layers, heads, n, batch, dtype, layout, nc, world, rank, plan.temperature,
+                                           math, ws.data_ptr(), ws_bytes, out.data_ptr(), flag_ptr, st),
+               "pnce_head_mb_shard_loss")
 
 
 def _head_bwd(plan, nc, tgt, params, ws, state, g, flat=None):
@@ -1519,7 +1552,8 @@ class _FusedHeadPatchNCE(torch.autograd.Function):
         return (None, None, *grads, *pgrads)
 
 
-_HEAD_WS_BYTES = {}      # pnce_head_workspace_bytes per (device, dtype, layout, nc, map shapes, patch counts)
+_HEAD_WS_BYTES = {}      # pnce_head_workspace_bytes per (device, dtype, layout, nc, mb, map shapes, patch counts, world)
+_HEAD_SLOTS = {}         # global negatives: (slot offset, slot bytes) per key of _HEAD_WS_BYTES
 
 
 def _head_params(netF, n):
@@ -1579,15 +1613,19 @@ def patchnce_with_head(netF: "PatchSampleF", src_feats, tgt_feats, temperature=0
     return loss, ids
 
 
-def _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group, mb=False):
+def _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group, mb=False,
+                negatives_group=None):
     """Argument handling + id draw of one fused head call -> (plan, tgt maps, head parameters, ids).
-    ``mb``: minibatch negatives -- the envelope (mb_check) is checked before anything touches the device."""
+    ``mb``: minibatch negatives -- the envelope (mb_check) is checked before anything touches the device.
+    ``negatives_group`` (with ``mb``): global negatives -- the envelope applies to the global batch, and is checked
+    before any collective as well."""
     if not fused_head_supported(netF, tgt_feats, num_patches):
         raise RuntimeError("fused head: nc must be 128 or 256, num_patches <= 1024 and C <= 256")
+    group, world = _negatives_group(mb, negatives_group)
     if mb:
         p_list = ([int(i.numel()) for i in patch_ids] if patch_ids is not None else
                   [patch_count(num_patches, f.shape[2] * f.shape[3]) for f in tgt_feats])
-        mb_check(tgt_feats[0].shape[0], [f.shape[1] for f in tgt_feats], p_list, math or DEFAULT_MATH)
+        mb_check(tgt_feats[0].shape[0], [f.shape[1] for f in tgt_feats], p_list, math or DEFAULT_MATH, world=world)
     if not netF.mlp_init:
         netF.create_mlp(tgt_feats)
     src, tgt, _, uniform = _prepare_maps(src_feats, tgt_feats, math or DEFAULT_MATH, int(num_patches))
@@ -1601,7 +1639,7 @@ def _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids,
     if dp_group is not None:
         from . import dp
         dp_group = dp.resolve_group(dp_group)          # None when not initialised or world size 1
-    plan = _HeadCall(src, ids, temperature, math or DEFAULT_MATH, dp_group, mb)
+    plan = _HeadCall(src, ids, temperature, math or DEFAULT_MATH, dp_group, mb, group, world)
     _warn_queue(tgt[0].device).poll()
     return plan, tgt, params, ids
 
@@ -1621,13 +1659,43 @@ def patchnce_with_head_minibatch(netF: "PatchSampleF", src_feats, tgt_feats, tem
     ``patchnce_with_head``.
 
     ``dp_group``: as in ``patchnce_with_head`` -- the head gradients are averaged over the group, and the negatives are
-    the rank's own shard, as upstream CUT under DDP.
+    the rank's own shard, as upstream CUT under DDP.  ``patchnce_with_head_global_negatives`` takes the negatives from
+    every rank's shard instead.
 
     Envelope: nc = 128 or 256, tensor-core math (not simt_f32), C <= 256, P <= 1024 and B * round_up(P, 128) <= 65536
     per layer.  Outside it a RuntimeError is raised before any launch; there is no other implementation to fall back to.
     """
     plan, tgt, params, ids = _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group,
                                          mb=True)
+    loss = _FusedHeadPatchNCE.apply(plan, netF.nc, *tgt, *params)
+    return loss, ids
+
+
+def patchnce_with_head_global_negatives(netF: "PatchSampleF", src_feats, tgt_feats, temperature=0.07, num_patches=256,
+                                        patch_ids=None, math: Optional[str] = None, negatives_group=True, dp_group=None):
+    """``patchnce_with_head_minibatch`` with the negatives of the whole data-parallel batch (global negatives, the head's
+    counterpart of ``PatchNCELoss(negatives_group=...)``).  Returns ``(loss, ids)``.
+
+    ``negatives_group``: ``True`` (the default process group) or a ``ProcessGroup`` of W ranks.  Each rank holds an
+    equal shard of B_l images, in rank order (``dp.shard_batch``), and every rank passes the same ids (one seed, or
+    ``dp.broadcast_patch_ids``) and the same head parameters; neither is checked at run time.  Per layer, the rank's
+    B_l * P query rows ``normalize(netF(raw tgt patches))`` are contrasted with the keys
+    ``normalize(netF(raw src patches)).detach()`` of all W * B_l images, which are all-gathered without gradient in the
+    forward; row i's positive is the key of the same global (image, patch).  Each rank returns the mean CE over its own
+    rows, so the mean of the W losses is ``patchnce_with_head_minibatch`` on the global batch, and averaging the
+    gradients over the ranks reproduces one GPU.  The guard is global: a layer is guarded on every rank (loss 0, zero
+    gradients, one warning per forward) exactly when the one-GPU call on the global batch guards it.  ``None``, no
+    process group, or a group of one rank: ``patchnce_with_head_minibatch`` itself, bit for bit.
+
+    ``dp_group``: independent of ``negatives_group`` -- as in ``patchnce_with_head``, the head gradients are averaged
+    over it (hidden under the dense-gradient kernel).  With ``negatives_group`` alone the head gradients are the rank's
+    own: average netF's gradients yourself (``dp.GradReducer``, DDP).
+
+    Envelope: ``patchnce_with_head_minibatch``'s applied to the global batch -- nc = 128 or 256, tensor-core math, C <= 256,
+    P <= 1024 and W * B_l * round_up(P, 128) <= 65536 per layer.  Outside it a RuntimeError is raised before any launch
+    or collective."""
+    plan, tgt, params, ids = _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group,
+                                         mb=True, negatives_group=negatives_group)
     loss = _FusedHeadPatchNCE.apply(plan, netF.nc, *tgt, *params)
     return loss, ids
 
@@ -1659,6 +1727,19 @@ def head_minibatch_loss_and_grads(netF: "PatchSampleF", src_feats, tgt_feats, te
     ``patchnce_with_head_minibatch(...)`` followed by ``loss.backward(grad_output)``; same envelope and errors."""
     plan, tgt, params, ids = _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group,
                                          mb=True)
+    return _head_loss_and_grads(netF, plan, tgt, params, ids, grad_output)
+
+
+def head_global_negatives_loss_and_grads(netF: "PatchSampleF", src_feats, tgt_feats, temperature=0.07,
+                                         num_patches=256, patch_ids=None, math: Optional[str] = None,
+                                         grad_output: Optional[torch.Tensor] = None, negatives_group=True,
+                                         dp_group=None):
+    """``patchnce_with_head_global_negatives`` and its complete backward in ONE call, without autograd: returns
+    ``(loss, [d (grad_output * loss) / d tgt_feats[l]], ids)`` and ACCUMULATES the head gradients into ``p.grad`` of
+    netF's parameters exactly as ``head_minibatch_loss_and_grads`` does.  Same ids, kernels, collectives and values as
+    ``patchnce_with_head_global_negatives(...)`` followed by ``loss.backward(grad_output)``; same envelope and errors."""
+    plan, tgt, params, ids = _head_begin(netF, src_feats, tgt_feats, temperature, num_patches, patch_ids, math, dp_group,
+                                         mb=True, negatives_group=negatives_group)
     return _head_loss_and_grads(netF, plan, tgt, params, ids, grad_output)
 
 

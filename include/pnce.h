@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define PNCE_ABI_VERSION 8
+#define PNCE_ABI_VERSION 9
 #define PNCE_MAX_LAYERS 8      /* nce_layers per call (reference config uses 5 ids -> 4 maps)   */
 #define PNCE_MAX_PATCHES 4096  /* P = min(num_patches, H*W)  patchnce_cut.py:60; argument check only: the
                                 * kernels take P <= 1024 (tensor cores, C <= 256) or P <= 1280 (fp32 CUDA cores),
@@ -325,6 +325,39 @@ int pnce_head_mb_workspace_bytes(const pnce_layer_t* layers, int n_layers, int b
 int pnce_head_mb_fwd(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch, int dtype, int layout,
                      int nc, float temperature, int math_mode, void* dev_workspace, size_t workspace_bytes,
                      float* dev_loss_out, int* dev_nonfinite, void* stream);
+
+/* ---- netF head with global negatives: minibatch negatives across data-parallel ranks (ABI 9) ------------------------
+ * The law of pnce_mb_shard_* on the head's output.  `world` ranks each hold batch_local images, rank r global images
+ * r * batch_local ... r * batch_local + batch_local - 1, every rank with the same ids and head parameters.  Per layer,
+ * rank r's query rows q = normalize(netF(raw tgt patches)) are contrasted with the keys
+ * k = normalize(netF(raw src patches)) (no gradient) of ALL world * batch_local images; row i's positive is the key of
+ * the same global (image, patch).  Rank r's loss is the mean row CE over its own rows, so the mean of the ranks' losses
+ * is pnce_head_mb_fwd's loss on the global batch, d loss_r / d tgt_r divided by world is the one-GPU gradient of shard
+ * r, and the rank-mean of the head gradients is the one-GPU head gradient.  The guard is global: a layer is guarded on
+ * every rank exactly when pnce_head_mb_fwd on the global batch guards it (dev_nonfinite[0] counts guarded layers).  The
+ * envelope is pnce_head_mb_fwd's, applied to the global batch.  The caller exchanges the slots:
+ *   pnce_head_mb_shard_workspace_bytes : total bytes, where the `world` slots start (slot_offset, always
+ *                                        pnce_head_mb_workspace_bytes(batch_local)) and their stride (slot_bytes,
+ *                                        256-aligned; the slot format of pnce_mb_shard_workspace_bytes with C = nc)
+ *   pnce_head_mb_shard_keys            : prep, weight blobs, gather and both head GEMMs; the keys go straight into slot
+ *                                        `rank`, with this rank's "a query row is non-finite" flags
+ *   -- the caller all-gathers the slot region [slot_offset, slot_offset + world * slot_bytes) in place --
+ *   pnce_head_mb_shard_loss            : logits, CE and d loss / d (head output) over every slot's keys
+ *                                        (k_loss_tc_mb_gn); the backward is pnce_head_bwd_ex(batch_local, any phases) on
+ *                                        the same workspace, layout and math mode
+ * Keys carry no gradient, so the backward needs no exchange.  world < 1, rank outside [0, world), dtype, layout or math
+ * mode out of range, NULL heads or weights: PNCE_ERR_ARG; simt_f32, nc not 128 / 256 or a global batch outside the
+ * envelope: PNCE_ERR_UNSUPPORTED; NULL, misaligned or short workspace: PNCE_ERR_WORKSPACE -- all before any CUDA call.
+ * dev_nonfinite may be NULL; when given, [1] receives the tensor-core protocol-timeout flag as in pnce_head_fwd_ex.   */
+int pnce_head_mb_shard_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch_local, int world, int nc,
+                                       size_t* bytes, size_t* slot_offset, size_t* slot_bytes);
+int pnce_head_mb_shard_keys(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch_local,
+                            int dtype, int layout, int nc, int world, int rank, int math_mode, void* dev_workspace,
+                            size_t workspace_bytes, int* dev_nonfinite, void* stream);
+int pnce_head_mb_shard_loss(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch_local,
+                            int dtype, int layout, int nc, int world, int rank, float temperature, int math_mode,
+                            void* dev_workspace, size_t workspace_bytes, float* dev_loss_out, int* dev_nonfinite,
+                            void* stream);
 
 /* ---- PatchSampleF(use_mlp=True).forward(feats, num_patches, patch_ids) as a module of its own (north_star's netF
  * signature; absent from the reference, SURVEY.md section 8 row a13): for every map, raw gather -> Linear(C_l, nc) ->
