@@ -27,6 +27,7 @@ from .patchnce import (  # noqa: F401
     pinned_as_device,
     poll_nonfinite_warnings,
     rows_patchnce,
+    rows_patchnce_global_negatives,
     rows_patchnce_multi,
     set_gradient_compression,
 )
@@ -38,6 +39,7 @@ from .dp import GradReducer, allreduce_head_grads, broadcast_patch_ids, shard_ba
 
 __all__ = [
     "PatchNCELoss", "PatchSampleF", "compute_patchnce_loss", "fused_patchnce", "rows_patchnce", "rows_patchnce_multi",
+    "rows_patchnce_global_negatives",
     "draw_patch_ids", "draw_patch_ids_all", "draw_ids", "pinned_as_device", "patch_count", "install_reference_shim", "poll_nonfinite_warnings",
     "DEFAULT_MATH", "patchnce_with_head", "head_loss_and_grads", "patchnce_with_head_minibatch",
     "head_minibatch_loss_and_grads", "patchnce_with_head_global_negatives", "head_global_negatives_loss_and_grads",

@@ -11,7 +11,7 @@ MATH_SIMT_F32, MATH_TC_BF16X3, MATH_TC_BF16 = 0, 1, 2
 MAX_LAYERS = 8
 MAX_PATCHES = 4096
 MAX_CHANNELS = 1024
-ABI_VERSION = 9
+ABI_VERSION = 10
 LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
 
 EXPORTS = [
@@ -28,6 +28,7 @@ EXPORTS = [
     "pnce_mb_shard_workspace_bytes", "pnce_mb_shard_keys", "pnce_mb_shard_loss",
     "pnce_head_mb_workspace_bytes", "pnce_head_mb_fwd",
     "pnce_head_mb_shard_workspace_bytes", "pnce_head_mb_shard_keys", "pnce_head_mb_shard_loss",
+    "pnce_rows_mb_shard_workspace_bytes", "pnce_rows_mb_shard_keys", "pnce_rows_mb_shard_loss",
 ]
 
 
@@ -107,6 +108,10 @@ def load():
     lib.pnce_mb_fwd.argtypes = lib.pnce_fwd_ex.argtypes
     lib.pnce_rows_mb_workspace_bytes.argtypes = lib.pnce_rows_loss_multi_workspace_bytes.argtypes
     lib.pnce_rows_mb_fwd_bwd.argtypes = lib.pnce_rows_loss_multi_fwd_bwd.argtypes
+    lib.pnce_rows_mb_shard_workspace_bytes.argtypes = [ctypes.POINTER(PnceRows), i32, i32, i32, ctypes.POINTER(sz),
+                                                       ctypes.POINTER(sz), ctypes.POINTER(sz)]
+    lib.pnce_rows_mb_shard_keys.argtypes = [ctypes.POINTER(PnceRows), i32, i32, i32, i32, i32, vp, sz, vp]
+    lib.pnce_rows_mb_shard_loss.argtypes = [ctypes.POINTER(PnceRows), i32, i32, i32, i32, f32, i32, vp, sz, vp, vp, vp]
     lib.pnce_mb_shard_workspace_bytes.argtypes = [ctypes.POINTER(PnceLayer), i32, i32, i32, ctypes.POINTER(sz),
                                                   ctypes.POINTER(sz), ctypes.POINTER(sz)]
     lib.pnce_mb_shard_keys.argtypes = [ctypes.POINTER(PnceLayer), i32, i32, i32, i32, i32, i32, i32, vp, sz, vp, sz,

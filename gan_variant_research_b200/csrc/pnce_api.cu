@@ -1568,6 +1568,123 @@ int pnce_rows_mb_fwd_bwd(const pnce_rows_t* rows, int n_layers, int batch, float
   return launch_loss_tc(t, st);
 }
 
+// ---- row route with global negatives: minibatch negatives over the row shards of every rank ---------------------------
+// Workspace: the prefix pnce_rows_mb_workspace_bytes(batch_local) (carve_rows_multi_tc: counter, per-layer losses, the
+// query blobs and sums of squares, the row-loss partials), then `world` slots in the format of pnce_mb_shard_*
+// (carve_mb_slot with C = D).  k_rows_pack writes this rank's keys straight into its slot (its key blobs and kss are the
+// gather's, one key block per image); carve_rows_multi_tc's own key blobs stay unused in this mode.
+//
+// The query flags: k_mb_qbad on the prefix's qss.  k_rows_pack writes 1 (chunk 0) and 0 (the others) for a finite row,
+// NaN for every chunk of a row holding a NaN / Inf, 0 for padding, so a flag is raised exactly for a row holding a
+// non-finite element -- exactly the loss kernel's own row test (badq).  Rows are used as given (norm words 1), so a finite
+// row's loss is non-finite only when its exp2 row sum overflows or underflows in the single-pass branch (|q . k| / tau
+// beyond ~88 - ln N: rows far from unit norm, DESIGN.md 4.15): the one case where the owning rank guards alone.
+
+// The envelope of the GLOBAL batch (world * batch_local images) and the slot geometry (vl: the layers carve_mb_slot
+// reads, C = D); no CUDA call.
+static int rows_shard_geometry(const pnce_rows_t* rows, int n, int batch_local, int world, pnce_layer_t* vl,
+                               size_t* prefix, size_t* slot_bytes) {
+  if (world < 1 || batch_local < 1) return PNCE_ERR_ARG;
+  if ((long long)world * batch_local > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
+  const int rc = check_rows_mb(rows, n, world * batch_local);
+  if (rc != PNCE_OK) return rc;
+  for (int l = 0; l < n; ++l) {
+    memset(&vl[l], 0, sizeof(vl[l]));
+    vl[l].C = rows[l].D;
+    vl[l].P = rows[l].P;
+  }
+  *prefix = carve_rows_multi_tc(rows, n, batch_local, true, nullptr, nullptr);
+  *slot_bytes = carve_mb_slot(vl, n, batch_local, true, nullptr, nullptr);
+  return PNCE_OK;
+}
+
+// The checks of both shard calls, all before any CUDA call, then the carve: the prefix into t, and slot `slot`'s key
+// blobs and flags over t's.
+static int rows_shard_params(const pnce_rows_t* rows, int n, int batch_local, int world, int rank, int math_mode,
+                             void* ws, size_t ws_bytes, int slot, Params& t, size_t* slot_bytes) {
+  pnce_layer_t vl[PNCE_MAX_LAYERS];
+  size_t prefix = 0;
+  int rc = rows_shard_geometry(rows, n, batch_local, world, vl, &prefix, slot_bytes);
+  if (rc != PNCE_OK) return rc;
+  if (rank < 0 || rank >= world) return PNCE_ERR_ARG;
+  if (math_mode < PNCE_MATH_SIMT_F32 || math_mode > PNCE_MATH_TC_BF16) return PNCE_ERR_ARG;
+  if (math_mode == PNCE_MATH_SIMT_F32) return PNCE_ERR_UNSUPPORTED;
+  if (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 255u)) return PNCE_ERR_WORKSPACE;
+  if (prefix + (size_t)world * *slot_bytes > ws_bytes) return PNCE_ERR_WORKSPACE;
+  const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
+  carve_rows_multi_tc(rows, n, batch_local, x3, ws, &t);
+  carve_mb_slot(vl, n, batch_local, x3, static_cast<unsigned char*>(ws) + prefix + (size_t)slot * *slot_bytes, &t);
+  t.math = math_mode;
+  t.b0 = 0; t.bn = batch_local;
+  t.mb = 1;
+  return PNCE_OK;
+}
+
+int pnce_rows_mb_shard_workspace_bytes(const pnce_rows_t* rows, int n_layers, int batch_local, int world, size_t* bytes,
+                                       size_t* slot_offset, size_t* slot_bytes) {
+  if (bytes == nullptr || slot_offset == nullptr || slot_bytes == nullptr) return PNCE_ERR_ARG;
+  pnce_layer_t vl[PNCE_MAX_LAYERS];
+  const int rc = rows_shard_geometry(rows, n_layers, batch_local, world, vl, slot_offset, slot_bytes);
+  if (rc != PNCE_OK) return rc;
+  *bytes = *slot_offset + (size_t)world * *slot_bytes;
+  return PNCE_OK;
+}
+
+int pnce_rows_mb_shard_keys(const pnce_rows_t* rows, int n_layers, int batch_local, int world, int rank, int math_mode,
+                            void* ws, size_t ws_bytes, void* stream) {
+  static thread_local Params t;
+  size_t slot_bytes = 0;
+  int rc = rows_shard_params(rows, n_layers, batch_local, world, rank, math_mode, ws, ws_bytes, rank, t, &slot_bytes);
+  if (rc != PNCE_OK) return rc;
+  for (int l = 0; l < n_layers; ++l)
+    if (!rows[l].q || !rows[l].k) return PNCE_ERR_ARG;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  PNCE_CUDA(cudaMemsetAsync(t.counter, 0, 2 * sizeof(unsigned), st));
+  // the pack: queries into the prefix, keys straight into slot `rank`
+  long long most = 0;
+  for (int l = 0; l < n_layers; ++l) {
+    const long long threads = 2ll * batch_local * t.L[l].Ppad * (t.L[l].Cp >> 3);
+    if (threads > most) most = threads;
+  }
+  launch_k(k_rows_pack, dim3((unsigned)((most + kThreads - 1) / kThreads), (unsigned)n_layers), kThreads, 0, st, t);
+  PNCE_CUDA(cudaGetLastError());
+  // this rank's "a query row is non-finite" flags, next to its keys (see above for why k_mb_qbad is exact here)
+  int* flags = const_cast<int*>(t.qbad);
+  PNCE_CUDA(cudaMemsetAsync(flags, 0, PNCE_MAX_LAYERS * sizeof(int), st));
+  most = 1;
+  for (int l = 0; l < n_layers; ++l) {
+    const long long nq = (long long)batch_local * t.L[l].nchunk * t.L[l].Ppad;
+    if ((nq + kMbQbadFloats - 1) / kMbQbadFloats > most) most = (nq + kMbQbadFloats - 1) / kMbQbadFloats;
+  }
+  launch_k<2>(k_mb_qbad, dim3((unsigned)most, (unsigned)n_layers), kThreads, 0, st, t, flags);
+  PNCE_CUDA(cudaGetLastError());
+  return PNCE_OK;
+}
+
+int pnce_rows_mb_shard_loss(const pnce_rows_t* rows, int n_layers, int batch_local, int world, int rank,
+                            float temperature, int math_mode, void* ws, size_t ws_bytes, float* loss_out, int* nonfinite,
+                            void* stream) {
+  static thread_local Params t;
+  size_t slot_bytes = 0;
+  // the key blobs and qbad: slot 0 of `world` (k_loss_tc_mb_gn steps to slot w by w * kslot)
+  int rc = rows_shard_params(rows, n_layers, batch_local, world, rank, math_mode, ws, ws_bytes, 0, t, &slot_bytes);
+  if (rc != PNCE_OK) return rc;
+  if (loss_out == nullptr || !(temperature > 0.f)) return PNCE_ERR_ARG;
+  for (int l = 0; l < n_layers; ++l) {
+    if (!rows[l].dq) return PNCE_ERR_ARG;
+    if (reinterpret_cast<uintptr_t>(rows[l].dq) & 31u) return PNCE_ERR_ALIGN;   // 32-byte row stores (k_loss_tc_mb_gn)
+  }
+  t.tau = temperature;
+  t.loss_out = loss_out;
+  t.nonfinite = nonfinite;
+  t.kworld = world;
+  t.kimg0 = rank * batch_local;
+  t.kslot = slot_bytes;
+  t.total_ctas = 0;
+  for (int l = 0; l < n_layers; ++l) t.total_ctas += (unsigned)(batch_local * (t.L[l].Ppad / 128));
+  return launch_loss_tc(t, static_cast<cudaStream_t>(stream));
+}
+
 // ---- netF head (tcgen05) ---------------------------------------------------------------------
 
 namespace pnce {

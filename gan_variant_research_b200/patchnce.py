@@ -803,7 +803,7 @@ class PatchNCELoss(nn.Module):
     Each rank returns the mean over its own rows, so averaging gradients over the ranks (``dp.GradReducer``, DDP)
     reproduces one GPU on the global batch; a non-finite row or key anywhere zeroes the layer on every rank.  The
     envelope above applies to the global batch.  ``None`` (default), or a group of one rank: the rank's own batch.
-    Maps route only: the row route raises RuntimeError."""
+    Maps route only: the row route raises RuntimeError (its form is ``rows_patchnce_global_negatives``)."""
 
     def __init__(self, temperature: float = 0.07, num_patches: int = 256,
                  nce_layers: Sequence[int] = (0, 4, 8, 12, 16), math: Optional[str] = None,
@@ -832,8 +832,9 @@ class PatchNCELoss(nn.Module):
         rows = (isinstance(a, torch.Tensor) and a.dim() == 2) or (not isinstance(a, torch.Tensor) and len(a) > 0
                                                                    and a[0].dim() == 2)
         if rows and self.negatives_group is not None:
-            raise RuntimeError("negatives_group covers the maps route (PatchNCELoss(src_feats, tgt_feats)); global "
-                               "negatives on the row route (PatchNCELoss(feat_q, feat_k)) are out of scope")
+            raise RuntimeError("negatives_group covers the maps route (PatchNCELoss(src_feats, tgt_feats)); for global "
+                               "negatives on the row route (PatchNCELoss(feat_q, feat_k)) call "
+                               "rows_patchnce_global_negatives(feat_q, feat_k)")
         if isinstance(a, torch.Tensor) and a.dim() == 2:
             if mb:
                 return rows_patchnce_multi([a], [b], self.temperature, self.num_patches, batch_size, self.math, True)
@@ -1225,16 +1226,18 @@ class _RowsLossFn(torch.autograd.Function):
 class _RowsLossMultiFn(torch.autograd.Function):
     """``mean_l PatchNCELoss(feat_q[l], feat_k[l])`` for every layer of a ``PatchSampleF`` output in ONE call of the
     library (pnce_rows_loss_multi_fwd_bwd: one pack launch, one tcgen05 loss launch).  Inputs: batch, temperature, math,
-    n, mb (minibatch negatives: pnce_rows_mb_fwd_bwd), the n query row tensors, the n (detached) key row tensors."""
+    n, mb (minibatch negatives: pnce_rows_mb_fwd_bwd), group (with mb: global negatives over that process group of more
+    than one rank, pnce_rows_mb_shard_*; None otherwise), the n query row tensors, the n (detached) key row tensors."""
 
     @staticmethod
-    def forward(ctx, batch, temperature, math, n, mb, *args):
+    def forward(ctx, batch, temperature, math, n, mb, group, *args):
         lib = _lib.load()
         qs = [_f32c(a) for a in args[:n]]
         ks = [_f32c(a) for a in args[n:]]
         dev = qs[0].device
         rows = (_lib.PnceRows * n)()
-        key = ["mb" if mb else "multi", batch]
+        world = dist.get_world_size(group) if group is not None else 1
+        key = ["mb" if mb else "multi", batch, world]
         with _on_device(dev):
             dqs = [torch.empty_like(q) for q in qs]
             for l in range(n):
@@ -1246,15 +1249,27 @@ class _RowsLossMultiFn(torch.autograd.Function):
             ws_bytes = _ROWS_WS_BYTES.get(key)
             if ws_bytes is None:
                 nbytes = ctypes.c_size_t(0)
-                wsq = lib.pnce_rows_mb_workspace_bytes if mb else lib.pnce_rows_loss_multi_workspace_bytes
-                _lib.check(wsq(rows, n, batch, ctypes.byref(nbytes)), "rows workspace query")
+                if world > 1:
+                    so, sb = ctypes.c_size_t(0), ctypes.c_size_t(0)
+                    _lib.check(lib.pnce_rows_mb_shard_workspace_bytes(rows, n, batch, world, ctypes.byref(nbytes),
+                                                                      ctypes.byref(so), ctypes.byref(sb)),
+                               "pnce_rows_mb_shard_workspace_bytes")
+                    _ROWS_SLOTS[key] = (so.value, sb.value)
+                else:
+                    wsq = lib.pnce_rows_mb_workspace_bytes if mb else lib.pnce_rows_loss_multi_workspace_bytes
+                    _lib.check(wsq(rows, n, batch, ctypes.byref(nbytes)), "rows workspace query")
                 ws_bytes = _ROWS_WS_BYTES[key] = nbytes.value
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
             out = torch.empty(1 + n, dtype=torch.float32, device=dev)
             slot, flag_ptr = _warn_queue(dev).acquire(mb)
-            fn = lib.pnce_rows_mb_fwd_bwd if mb else lib.pnce_rows_loss_multi_fwd_bwd
-            _lib.check(fn(rows, n, batch, temperature, _MATH[math], ws.data_ptr(), ws_bytes, out.data_ptr(),
-                          flag_ptr or None, _stream_ptr(dev)), "pnce_rows_mb_fwd_bwd" if mb else "pnce_rows_loss_multi_fwd_bwd")
+            if world > 1:
+                _rows_fwd_global(lib, rows, n, batch, temperature, math, group, world, _ROWS_SLOTS[key], ws, ws_bytes,
+                                 out, flag_ptr or None, _stream_ptr(dev))
+            else:
+                fn = lib.pnce_rows_mb_fwd_bwd if mb else lib.pnce_rows_loss_multi_fwd_bwd
+                _lib.check(fn(rows, n, batch, temperature, _MATH[math], ws.data_ptr(), ws_bytes, out.data_ptr(),
+                              flag_ptr or None, _stream_ptr(dev)),
+                           "pnce_rows_mb_fwd_bwd" if mb else "pnce_rows_loss_multi_fwd_bwd")
         ctx.save_for_backward(*dqs)
         ctx.q_dtypes = [a.dtype for a in args[:n]]
         ctx.layer_losses = out[1:]
@@ -1264,20 +1279,32 @@ class _RowsLossMultiFn(torch.autograd.Function):
     def backward(ctx, grad_out):
         dqs = torch._foreach_mul(list(ctx.saved_tensors), grad_out)            # one launch for every layer
         dqs = [d if d.dtype is dt else d.to(dt) for d, dt in zip(dqs, ctx.q_dtypes)]
-        return (None, None, None, None, None, *dqs, *([None] * len(dqs)))
+        return (None, None, None, None, None, None, *dqs, *([None] * len(dqs)))
 
 
-def rows_patchnce_multi(feat_q, feat_k, temperature=0.07, num_patches=256, batch_size=None, math=None, mb=False):
-    """``mean_l PatchNCELoss(feat_q[l], feat_k[l])`` over two LISTS of row tensors (one (B*P_l, D_l) pair per layer, as
-    ``PatchSampleF`` returns them) -- upstream CUT's ``for f_q, f_k in zip(feat_q, feat_k): total += crit(f_q, f_k)``
-    followed by ``/ n_layers``, as one call of the library when every layer fits the tensor-core kernel (P, D <= 256);
-    other shapes take the per-layer calls.  ``mb``: minibatch negatives (``PatchNCELoss``), one library call
-    (pnce_rows_mb_fwd_bwd) for every layer."""
+_ROWS_SLOTS = {}         # global negatives: (slot offset, slot bytes) per key of _ROWS_WS_BYTES
+
+
+def _rows_fwd_global(lib, rows, n, batch, temperature, math, group, world, slots, ws, ws_bytes, out, flag_ptr, st):
+    """Global negatives on the row route: this rank's keys packed into its slot of the workspace, the all-gather of the
+    slots (the one collective of the mode; keys carry no gradient, so the backward is local), then the loss and d q over
+    every rank's keys."""
+    from . import dp
+    rank = dist.get_rank(group)
+    so, sb = slots
+    _lib.check(lib.pnce_rows_mb_shard_keys(rows, n, batch, world, rank, _MATH[math], ws.data_ptr(), ws_bytes, st),
+               "pnce_rows_mb_shard_keys")
+    dp.allgather_slots_(ws[so:so + world * sb], rank, group)
+    _lib.check(lib.pnce_rows_mb_shard_loss(rows, n, batch, world, rank, temperature, _MATH[math], ws.data_ptr(),
+                                           ws_bytes, out.data_ptr(), flag_ptr, st), "pnce_rows_mb_shard_loss")
+
+
+def _rows_batches(feat_q, feat_k, num_patches, batch_size):
+    """Argument checks of the multi-layer row calls -> (feat_q list, feat_k list, images per layer)."""
     feat_q, feat_k = list(feat_q), list(feat_k)
     n = len(feat_q)
     if n == 0 or n != len(feat_k):
         raise RuntimeError("feat_q and feat_k must be two lists of the same, non-zero length")
-    math = math or DEFAULT_MATH
     batches = []
     for q, k in zip(feat_q, feat_k):
         _require_cuda(q, "feat_q")
@@ -1294,14 +1321,33 @@ def rows_patchnce_multi(feat_q, feat_k, temperature=0.07, num_patches=256, batch
             if rows % batch_size:
                 raise RuntimeError(f"{rows} rows are not a multiple of batch_size={batch_size}")
             batches.append(int(batch_size))
+    return feat_q, feat_k, batches
+
+
+def _rows_mb_apply(feat_q, feat_k, batches, temperature, math, group=None, world=1):
+    """The minibatch row loss of every layer in one library call: envelope first (mb_check on the global batch of
+    ``world`` shards), then _RowsLossMultiFn."""
+    n, b0, dev = len(feat_q), batches[0], feat_q[0].device
+    if any(b != b0 for b in batches) or any(q.device != dev for q in feat_q) or n > _lib.MAX_LAYERS:
+        raise RuntimeError("nce_includes_all_negatives_from_minibatch on rows needs layers of one batch size and "
+                           f"device, at most {_lib.MAX_LAYERS} of them")
+    mb_check(b0, [q.shape[1] for q in feat_q], [q.shape[0] // b0 for q in feat_q], math, rows=True, world=world)
+    ks = [k.detach() if k.requires_grad else k for k in feat_k]          # upstream CUT and the reference (:142) detach k
+    return _RowsLossMultiFn.apply(b0, float(temperature), math, n, True, group, *feat_q, *ks)
+
+
+def rows_patchnce_multi(feat_q, feat_k, temperature=0.07, num_patches=256, batch_size=None, math=None, mb=False):
+    """``mean_l PatchNCELoss(feat_q[l], feat_k[l])`` over two LISTS of row tensors (one (B*P_l, D_l) pair per layer, as
+    ``PatchSampleF`` returns them) -- upstream CUT's ``for f_q, f_k in zip(feat_q, feat_k): total += crit(f_q, f_k)``
+    followed by ``/ n_layers``, as one call of the library when every layer fits the tensor-core kernel (P, D <= 256);
+    other shapes take the per-layer calls.  ``mb``: minibatch negatives (``PatchNCELoss``), one library call
+    (pnce_rows_mb_fwd_bwd) for every layer."""
+    feat_q, feat_k, batches = _rows_batches(feat_q, feat_k, num_patches, batch_size)
+    n = len(feat_q)
+    math = math or DEFAULT_MATH
     b0, dev = batches[0], feat_q[0].device
     if mb and b0 > 1:
-        if any(b != b0 for b in batches) or any(q.device != dev for q in feat_q) or n > _lib.MAX_LAYERS:
-            raise RuntimeError("nce_includes_all_negatives_from_minibatch on rows needs layers of one batch size and "
-                               f"device, at most {_lib.MAX_LAYERS} of them")
-        mb_check(b0, [q.shape[1] for q in feat_q], [q.shape[0] // b0 for q in feat_q], math, rows=True)
-        ks = [k.detach() if k.requires_grad else k for k in feat_k]      # upstream CUT and the reference (:142) detach k
-        return _RowsLossMultiFn.apply(b0, float(temperature), math, n, True, *feat_q, *ks)
+        return _rows_mb_apply(feat_q, feat_k, batches, temperature, math)
     fused = (math != "simt_f32" and n <= _lib.MAX_LAYERS and all(b == b0 for b in batches)
              and all(q.device == dev and q.shape[0] // b0 <= 256 and q.shape[1] <= 256 for q in feat_q))
     if not fused:
@@ -1311,7 +1357,40 @@ def rows_patchnce_multi(feat_q, feat_k, temperature=0.07, num_patches=256, batch
             total = l if total is None else total + l
         return total / n
     ks = [k.detach() if k.requires_grad else k for k in feat_k]          # upstream CUT and the reference (:142) detach k
-    return _RowsLossMultiFn.apply(b0, float(temperature), math, n, False, *feat_q, *ks)
+    return _RowsLossMultiFn.apply(b0, float(temperature), math, n, False, None, *feat_q, *ks)
+
+
+def rows_patchnce_global_negatives(feat_q, feat_k, temperature=0.07, num_patches=256, batch_size=None, math=None,
+                                   negatives_group=True):
+    """Minibatch negatives across data-parallel ranks on the row route (module split: ``PatchSampleF`` on both sides,
+    then this instead of ``PatchNCELoss(..., nce_includes_all_negatives_from_minibatch=True)(feat_q, feat_k)``).
+    ``feat_q`` / ``feat_k``: one (B_l * P, D) pair of row tensors, or two lists of them (one pair per layer, as
+    ``PatchSampleF`` returns them; every layer in one pack, one key exchange and one loss launch).  Rows are grouped per
+    image and already L2-normalised; the keys carry no gradient.  Returns the scalar loss, differentiable w.r.t.
+    ``feat_q``.  The number of images is inferred as in ``rows_patchnce_multi``.
+
+    ``negatives_group``: ``True`` (the default process group) or a ``ProcessGroup`` of W ranks, each holding an equal
+    shard of B_l images in rank order (``dp.shard_batch``) and using the same patch ids (neither is checked at run
+    time).  Per layer, the rank's B_l * P query rows are contrasted with the key rows of all W * B_l images, which are
+    all-gathered without gradient in the forward; row i's positive is the key of the same global row.  Each rank returns
+    the mean CE over its own rows, then the mean over layers, so the mean of the W losses is
+    ``PatchNCELoss(tau, P, nce_includes_all_negatives_from_minibatch=True)`` on the global rows and averaging the
+    gradients over the ranks (``dp.GradReducer``, DDP) reproduces one GPU.  The guard is global: a non-finite query row
+    on any rank, or a non-finite key, zeroes the layer on every rank (loss 0, zero gradient, one warning per guarded
+    layer through ``poll_nonfinite_warnings``).  ``None``, no process group, or a group of one rank:
+    ``rows_patchnce_multi(feat_q, feat_k, ..., mb=True)`` itself, bit for bit.
+
+    Envelope: tensor-core math, D <= 256, P <= 256 and W * B_l * round_up(P, 128) <= 65536 per layer, layers of one
+    batch size and device, at most ``MAX_LAYERS`` of them; outside it a RuntimeError is raised before any launch or
+    collective."""
+    if isinstance(feat_q, torch.Tensor):
+        feat_q, feat_k = [feat_q], [feat_k]
+    group, world = _negatives_group(True, negatives_group)
+    math = math or DEFAULT_MATH
+    if group is None:
+        return rows_patchnce_multi(feat_q, feat_k, temperature, num_patches, batch_size, math, True)
+    feat_q, feat_k, batches = _rows_batches(feat_q, feat_k, num_patches, batch_size)
+    return _rows_mb_apply(feat_q, feat_k, batches, temperature, math, group, world)
 
 
 def rows_patchnce(feat_q, feat_k, temperature=0.07, num_patches=256, batch_size=None, math=None):

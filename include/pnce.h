@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define PNCE_ABI_VERSION 9
+#define PNCE_ABI_VERSION 10
 #define PNCE_MAX_LAYERS 8      /* nce_layers per call (reference config uses 5 ids -> 4 maps)   */
 #define PNCE_MAX_PATCHES 4096  /* P = min(num_patches, H*W)  patchnce_cut.py:60; argument check only: the
                                 * kernels take P <= 1024 (tensor cores, C <= 256) or P <= 1280 (fp32 CUDA cores),
@@ -244,6 +244,35 @@ int pnce_rows_mb_workspace_bytes(const pnce_rows_t* rows, int n_layers, int batc
 int pnce_rows_mb_fwd_bwd(const pnce_rows_t* rows, int n_layers, int batch, float temperature, int math_mode,
                          void* dev_workspace, size_t workspace_bytes, float* dev_loss_out, int* dev_nonfinite,
                          void* stream);
+/* ---- row route with global negatives: minibatch negatives across data-parallel ranks (ABI 10) -----------------------
+ * The law of pnce_mb_shard_* on rows used as given.  `world` ranks each hold batch_local images, rank r global images
+ * r * batch_local ... r * batch_local + batch_local - 1, every rank with the same ids; rows[l].q / .k are the rank's
+ * (batch_local * P, D) rows of layer l, grouped per image and already L2-normalised (PatchSampleF's output).  Per layer,
+ * rank r's query rows are contrasted with the key rows of ALL world * batch_local images in global (image, patch) order;
+ * row i's positive is the key of the same global row; Z = clamp(q k^T / tau, -50, 50).  Rank r's loss is the mean row
+ * CE over its own rows, then the mean over layers, so the mean of the ranks' losses is pnce_rows_mb_fwd_bwd's loss on
+ * the global rows and rows[l].dq / world is that call's d loss / d q restricted to shard r.  The guard is global: a
+ * non-finite query row on any rank, or a non-finite key, zeroes the layer on every rank (its dq rows are 0, as one GPU
+ * writes them); dev_nonfinite[0] counts guarded layers.  The envelope is pnce_rows_mb_fwd_bwd's applied to the global
+ * batch: tensor-core math, P <= 256, D <= 256, world * batch_local * round_up(P, 128) <= 65536 per layer.
+ *   pnce_rows_mb_shard_workspace_bytes : total bytes, where the `world` slots start (slot_offset, always
+ *                                        pnce_rows_mb_workspace_bytes(batch_local)) and their stride (slot_bytes,
+ *                                        256-aligned; the slot format of pnce_mb_shard_workspace_bytes with C = D)
+ *   pnce_rows_mb_shard_keys            : the row pack (k_rows_pack): queries into the prefix, keys straight into slot
+ *                                        `rank`, with this rank's "a query row is non-finite" flags (reads q, k)
+ *   -- the caller all-gathers the slot region [slot_offset, slot_offset + world * slot_bytes) in place --
+ *   pnce_rows_mb_shard_loss            : logits, CE and d loss / d q over every slot's keys (k_loss_tc_mb_gn); writes
+ *                                        rows[l].dq row-major (32-byte aligned: PNCE_ERR_ALIGN otherwise)
+ * Keys carry no gradient, so nothing is exchanged for the backward.  world < 1, rank outside [0, world), math mode out of
+ * range, NULL rows / loss or a bad shape: PNCE_ERR_ARG; simt_f32 or a global batch outside the envelope:
+ * PNCE_ERR_UNSUPPORTED; NULL, misaligned or short workspace: PNCE_ERR_WORKSPACE -- all before any CUDA call.           */
+int pnce_rows_mb_shard_workspace_bytes(const pnce_rows_t* rows, int n_layers, int batch_local, int world, size_t* bytes,
+                                       size_t* slot_offset, size_t* slot_bytes);
+int pnce_rows_mb_shard_keys(const pnce_rows_t* rows, int n_layers, int batch_local, int world, int rank, int math_mode,
+                            void* dev_workspace, size_t workspace_bytes, void* stream);
+int pnce_rows_mb_shard_loss(const pnce_rows_t* rows, int n_layers, int batch_local, int world, int rank,
+                            float temperature, int math_mode, void* dev_workspace, size_t workspace_bytes,
+                            float* dev_loss_out, int* dev_nonfinite, void* stream);
 
 /* All maps of one PatchSampleF call in ONE launch each way (the per-map entry points above cost a launch per
  * layer and leave the GPU half empty on the small layers): forward reads feat / ids and writes rows (and inv,
