@@ -81,6 +81,14 @@ static bool mb_shapes_ok(const pnce_layer_t* layers, int n_layers, int B) {
   return true;
 }
 
+// global negatives: the envelope of the GLOBAL batch of world * batch_local images -- the product must fit an int, then
+// pass the route's shape test (a status: PNCE_OK, or the code to return)
+template <typename ShapeTest>
+static int global_batch_check(int world, int batch_local, ShapeTest shapes) {
+  if ((long long)world * batch_local > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
+  return shapes(world * batch_local);
+}
+
 // Fills Params (pointers into the workspace) for the fused path; returns bytes used.
 // tc = carve the tensor-core operand blobs instead of the fp32 normalised rows.
 // The id bookkeeping of every layer (k_prep's outputs): sid, perm, rank, cslot.  It lives at the head of the
@@ -1011,6 +1019,45 @@ static size_t carve_mb_slot(const pnce_layer_t* layers, int n_layers, int B, boo
   return align_up(cv.off, 256);
 }
 
+// Keys call, after this rank's query sums of squares exist: its "a query row is non-finite" flags (k_mb_qbad on p's qss,
+// every layer) into `flags`, which live in its slot next to its keys.
+static int launch_mb_qbad(const Params& p, int* flags, cudaStream_t st) {
+  PNCE_CUDA(cudaMemsetAsync(flags, 0, PNCE_MAX_LAYERS * sizeof(int), st));
+  long long most = 1;
+  for (int l = 0; l < p.n_layers; ++l) {
+    const long long n = (long long)p.B * p.L[l].nchunk * p.L[l].Ppad;
+    if ((n + kMbQbadFloats - 1) / kMbQbadFloats > most) most = (n + kMbQbadFloats - 1) / kMbQbadFloats;
+  }
+  if (most > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
+  launch_k<2>(k_mb_qbad, dim3((unsigned)most, (unsigned)p.n_layers), kThreads, 0, st, p, flags);
+  PNCE_CUDA(cudaGetLastError());
+  return PNCE_OK;
+}
+
+// Loss call, once p's key blobs and qbad point at slot 0: k_loss_tc_mb_gn steps to slot w by w * kslot, and this rank's
+// query images are global images rank * B on.
+static void point_at_slots(Params& p, int world, int rank, size_t slot_bytes) {
+  p.kworld = world;
+  p.kimg0 = rank * p.B;
+  p.kslot = slot_bytes;
+  int ctas_per_image = 0;
+  for (int l = 0; l < p.n_layers; ++l) ctas_per_image += p.L[l].Ppad / 128;
+  p.total_ctas = (unsigned)(p.B * ctas_per_image);
+}
+
+// The envelope of the global batch and the slot geometry: *prefix, the slots' offset; *slot_bytes, their stride.  No
+// CUDA call.
+static int mb_shard_geometry(const pnce_layer_t* layers, int n_layers, int batch_local, int world, size_t* prefix,
+                             size_t* slot_bytes) {
+  const int rc = global_batch_check(world, batch_local, [&](int B) {
+    return mb_shapes_ok(layers, n_layers, B) ? PNCE_OK : PNCE_ERR_UNSUPPORTED;
+  });
+  if (rc != PNCE_OK) return rc;
+  *prefix = carve_fused(layers, n_layers, batch_local, true, true, nullptr, nullptr);
+  *slot_bytes = carve_mb_slot(layers, n_layers, batch_local, true, nullptr, nullptr);
+  return PNCE_OK;
+}
+
 // The checks of both shard calls, all before any CUDA call; fills Params with the prefix carve and with slot `slot`'s
 // key blobs.  *slot_bytes: the slot stride.
 static int mb_shard_params(const pnce_layer_t* layers, int n_layers, int batch_local, int dtype, int layout, int world,
@@ -1023,18 +1070,17 @@ static int mb_shard_params(const pnce_layer_t* layers, int n_layers, int batch_l
   if (layout != PNCE_LAYOUT_NCHW && layout != PNCE_LAYOUT_NHWC) return PNCE_ERR_ARG;
   if (math_mode < PNCE_MATH_SIMT_F32 || math_mode > PNCE_MATH_TC_BF16) return PNCE_ERR_ARG;
   if (math_mode == PNCE_MATH_SIMT_F32) return PNCE_ERR_UNSUPPORTED;
-  if ((long long)world * batch_local > 0x7fffffffLL || !mb_shapes_ok(layers, n_layers, world * batch_local))
-    return PNCE_ERR_UNSUPPORTED;                               // the envelope of the GLOBAL batch
+  size_t prefix = 0;
+  rc = mb_shard_geometry(layers, n_layers, batch_local, world, &prefix, slot_bytes);
+  if (rc != PNCE_OK) return rc;
   rc = check_alignment(layers, n_layers, dtype, false);
   if (rc != PNCE_OK) return rc;
   if (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 255u)) return PNCE_ERR_WORKSPACE;
   if (plan != nullptr &&
       ((reinterpret_cast<uintptr_t>(plan) & 255u) || carve_plan(layers, n_layers, nullptr, nullptr) > plan_bytes))
     return PNCE_ERR_WORKSPACE;
-  const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
-  const size_t prefix = carve_fused(layers, n_layers, batch_local, true, true, nullptr, nullptr);
-  *slot_bytes = carve_mb_slot(layers, n_layers, batch_local, true, nullptr, nullptr);
   if (prefix + (size_t)world * *slot_bytes > ws_bytes) return PNCE_ERR_WORKSPACE;
+  const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
   carve_fused(layers, n_layers, batch_local, true, x3, ws, p, plan);
   carve_mb_slot(layers, n_layers, batch_local, x3, static_cast<unsigned char*>(ws) + prefix + (size_t)slot * *slot_bytes, p);
   p->dtype = dtype;
@@ -1048,13 +1094,11 @@ static int mb_shard_params(const pnce_layer_t* layers, int n_layers, int batch_l
 int pnce_mb_shard_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch_local, int world, size_t* bytes,
                                   size_t* slot_offset, size_t* slot_bytes) {
   if (bytes == nullptr || slot_offset == nullptr || slot_bytes == nullptr) return PNCE_ERR_ARG;
-  const int rc = check_layers(layers, n_layers, batch_local);
+  int rc = check_layers(layers, n_layers, batch_local);
   if (rc != PNCE_OK) return rc;
   if (world < 1) return PNCE_ERR_ARG;
-  if ((long long)world * batch_local > 0x7fffffffLL || !mb_shapes_ok(layers, n_layers, world * batch_local))
-    return PNCE_ERR_UNSUPPORTED;
-  *slot_offset = carve_fused(layers, n_layers, batch_local, true, true, nullptr, nullptr);
-  *slot_bytes = carve_mb_slot(layers, n_layers, batch_local, true, nullptr, nullptr);
+  rc = mb_shard_geometry(layers, n_layers, batch_local, world, slot_offset, slot_bytes);
+  if (rc != PNCE_OK) return rc;
   *bytes = *slot_offset + (size_t)world * *slot_bytes;
   return PNCE_OK;
 }
@@ -1078,17 +1122,7 @@ int pnce_mb_shard_keys(const pnce_layer_t* layers, int n_layers, int batch_local
   if (rc != PNCE_OK) return rc;
   rc = launch_gather_tc(p, st, fold);
   if (rc != PNCE_OK) return rc;
-  int* flags = const_cast<int*>(p.qbad);
-  PNCE_CUDA(cudaMemsetAsync(flags, 0, PNCE_MAX_LAYERS * sizeof(int), st));
-  long long most = 1;
-  for (int l = 0; l < n_layers; ++l) {
-    const long long n = (long long)batch_local * p.L[l].nchunk * p.L[l].Ppad;
-    if ((n + kMbQbadFloats - 1) / kMbQbadFloats > most) most = (n + kMbQbadFloats - 1) / kMbQbadFloats;
-  }
-  if (most > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
-  launch_k<2>(k_mb_qbad, dim3((unsigned)most, (unsigned)n_layers), kThreads, 0, st, p, flags);
-  PNCE_CUDA(cudaGetLastError());
-  return PNCE_OK;
+  return launch_mb_qbad(p, const_cast<int*>(p.qbad), st);
 }
 
 int pnce_mb_shard_loss(const pnce_layer_t* layers, int n_layers, int batch_local, int dtype, int layout, int world,
@@ -1104,12 +1138,7 @@ int pnce_mb_shard_loss(const pnce_layer_t* layers, int n_layers, int batch_local
   p.loss_out = loss_out;
   p.nonfinite = nonfinite;
   p.trace = g_dbg.trace;
-  p.kworld = world;
-  p.kimg0 = rank * batch_local;
-  p.kslot = slot_bytes;
-  int ctas_per_image = 0;
-  for (int l = 0; l < n_layers; ++l) ctas_per_image += p.L[l].Ppad / 128;
-  p.total_ctas = (unsigned)(batch_local * ctas_per_image);
+  point_at_slots(p, world, rank, slot_bytes);
   return launch_loss_tc(p, static_cast<cudaStream_t>(stream));
 }
 
@@ -1334,99 +1363,9 @@ static size_t carve_rows_loss(int B, int P, int D, void* ws, Params* out) {
   return align_up(cv.off, 256);
 }
 
-// the same problem on the tensor-core kernel (P, D <= 256): operand blobs + per-chunk norm words
+// the same problem on the tensor-core kernel (P, D <= 256): operand blobs + per-chunk norm words, for every layer of a
+// PatchSampleF output at once (one pack launch + one loss launch)
 static bool rows_tc_ok(int P, int D) { return P <= 256 && D <= 256; }
-static size_t carve_rows_loss_tc(int B, int P, int D, bool x3, void* ws, Params* out) {
-  Carver cv(ws);
-  Params p;
-  memset(&p, 0, sizeof(p));
-  p.n_layers = 1; p.B = B; p.rows_mode = 1;
-  p.counter = cv.take<unsigned>(64);
-  p.lossimg = cv.take<float>(B);
-  p.valid = cv.take<int>(B);
-  LayerDev& L = p.L[0];
-  L.C = D; L.P = P; L.HW = 1; L.nwords = 1;
-  L.ntiles = (P + kRowTile - 1) / kRowTile;
-  L.sorted = 1;
-  L.Cp = (D + 31) / 32 * 32;
-  L.Ppad = (P + 127) / 128 * 128;
-  L.nchunk = L.Cp / 32;
-  L.nparts = L.Ppad / 128;
-  L.dxpitch = L.Ppad;
-  const size_t blob = (size_t)B * L.Ppad * L.Cp;
-  L.qhi = cv.take<__nv_bfloat16>(blob);
-  L.khi = cv.take<__nv_bfloat16>(blob);
-  L.k2hi = cv.take<__nv_bfloat16>(blob);
-  if (x3) {
-    L.qlo = cv.take<__nv_bfloat16>(blob);
-    L.klo = cv.take<__nv_bfloat16>(blob);
-    L.k2lo = cv.take<__nv_bfloat16>(blob);
-  }
-  L.qss = cv.take<float>((size_t)B * L.nchunk * L.Ppad);
-  L.kss = cv.take<float>((size_t)B * L.nchunk * L.Ppad);
-  L.partial = cv.take<float>((size_t)B * 2);
-  if (out) *out = p;
-  return align_up(cv.off, 256);
-}
-
-int pnce_rows_loss_workspace_bytes(int batch, int P, int D, size_t* bytes) {
-  if (bytes == nullptr || batch < 1 || P < 1 || D < 1) return PNCE_ERR_ARG;
-  if (P > PNCE_MAX_PATCHES || D > PNCE_MAX_CHANNELS) return PNCE_ERR_UNSUPPORTED;
-  size_t need = carve_rows_loss(batch, P, D, nullptr, nullptr);
-  if (rows_tc_ok(P, D)) {
-    const size_t t = carve_rows_loss_tc(batch, P, D, true, nullptr, nullptr);
-    if (t > need) need = t;
-  }
-  *bytes = need;
-  return PNCE_OK;
-}
-
-int pnce_rows_loss_fwd_bwd(const float* q, const float* k, int batch, int P, int D, float temperature,
-                           int math_mode, void* ws, size_t ws_bytes, float* loss_out, int* nonfinite,
-                           float* dq_out, float* dk_out, void* stream) {
-  if (!q || !k || !loss_out || !dq_out || batch < 1 || P < 1 || D < 1 || !(temperature > 0.f)) return PNCE_ERR_ARG;
-  if (P > PNCE_MAX_PATCHES || D > PNCE_MAX_CHANNELS) return PNCE_ERR_UNSUPPORTED;
-  if (dk_out != nullptr) return PNCE_ERR_UNSUPPORTED;   // feat_k is detached in the reference (:142)
-  if (math_mode < PNCE_MATH_SIMT_F32 || math_mode > PNCE_MATH_TC_BF16) return PNCE_ERR_ARG;
-  if (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 255u)) return PNCE_ERR_WORKSPACE;
-  cudaStream_t st0 = static_cast<cudaStream_t>(stream);
-  if (math_mode != PNCE_MATH_SIMT_F32 && rows_tc_ok(P, D)) {
-    // tensor-core modes: re-tile the rows into operand blobs (k_rows_pack), then the tcgen05 loss kernel in
-    // rows mode (rows used as given, d loss / d q written row-major).  P or D > 256: CUDA-core kernel below.
-    const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
-    Params t;
-    if (carve_rows_loss_tc(batch, P, D, x3, ws, &t) > ws_bytes) return PNCE_ERR_WORKSPACE;
-    t.math = math_mode;
-    t.tau = temperature;
-    t.loss_out = loss_out;
-    t.nonfinite = nonfinite;
-    t.b0 = 0; t.bn = batch;
-    LayerDev& T = t.L[0];
-    T.qn = const_cast<float*>(q);
-    T.kn = const_cast<float*>(k);
-    T.dq_rows = dq_out;
-    PNCE_CUDA(cudaMemsetAsync(t.counter, 0, 2 * sizeof(unsigned), st0));
-    const long long threads = 2ll * batch * T.Ppad * (T.Cp >> 3);
-    launch_k(k_rows_pack, (unsigned)((threads + kThreads - 1) / kThreads), kThreads, 0, st0, t);
-    PNCE_CUDA(cudaGetLastError());
-    return launch_loss_tc(t, st0);
-  }
-  // fp32 CUDA-core kernel on the rows as they are
-  Params p;
-  if (carve_rows_loss(batch, P, D, ws, &p) > ws_bytes) return PNCE_ERR_WORKSPACE;
-  p.tau = temperature;
-  p.loss_out = loss_out;
-  p.nonfinite = nonfinite;
-  LayerDev& L = p.L[0];
-  L.qn = const_cast<float*>(q);
-  L.kn = const_cast<float*>(k);
-  L.dq_rows = dq_out;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  PNCE_CUDA(cudaMemsetAsync(p.counter, 0, 2 * sizeof(unsigned), st));
-  return launch_loss_simt(p, st);
-}
-
-// every layer of a PatchSampleF output in one pack launch + one loss launch (tensor-core modes)
 static size_t carve_rows_multi_tc(const pnce_rows_t* rows, int n, int B, bool x3, void* ws, pnce::Params* out) {
   using namespace pnce;
   Carver cv(ws);
@@ -1467,6 +1406,72 @@ static size_t carve_rows_multi_tc(const pnce_rows_t* rows, int n, int B, bool x3
   return align_up(cv.off, 256);
 }
 
+// Re-tiles the rows of every layer into operand blobs (k_rows_pack), after the counter reset the loss kernel relies on.
+static int launch_rows_pack(const Params& t, cudaStream_t st) {
+  PNCE_CUDA(cudaMemsetAsync(t.counter, 0, 2 * sizeof(unsigned), st));
+  long long most = 0;
+  for (int l = 0; l < t.n_layers; ++l) {
+    const long long threads = 2ll * t.B * t.L[l].Ppad * (t.L[l].Cp >> 3);
+    if (threads > most) most = threads;
+  }
+  launch_k(k_rows_pack, dim3((unsigned)((most + kThreads - 1) / kThreads), (unsigned)t.n_layers), kThreads, 0, st, t);
+  PNCE_CUDA(cudaGetLastError());
+  return PNCE_OK;
+}
+
+int pnce_rows_loss_workspace_bytes(int batch, int P, int D, size_t* bytes) {
+  if (bytes == nullptr || batch < 1 || P < 1 || D < 1) return PNCE_ERR_ARG;
+  if (P > PNCE_MAX_PATCHES || D > PNCE_MAX_CHANNELS) return PNCE_ERR_UNSUPPORTED;
+  size_t need = carve_rows_loss(batch, P, D, nullptr, nullptr);
+  if (rows_tc_ok(P, D)) {
+    const pnce_rows_t row = {nullptr, nullptr, nullptr, P, D};
+    const size_t t = carve_rows_multi_tc(&row, 1, batch, true, nullptr, nullptr);
+    if (t > need) need = t;
+  }
+  *bytes = need;
+  return PNCE_OK;
+}
+
+int pnce_rows_loss_fwd_bwd(const float* q, const float* k, int batch, int P, int D, float temperature,
+                           int math_mode, void* ws, size_t ws_bytes, float* loss_out, int* nonfinite,
+                           float* dq_out, float* dk_out, void* stream) {
+  if (!q || !k || !loss_out || !dq_out || batch < 1 || P < 1 || D < 1 || !(temperature > 0.f)) return PNCE_ERR_ARG;
+  if (P > PNCE_MAX_PATCHES || D > PNCE_MAX_CHANNELS) return PNCE_ERR_UNSUPPORTED;
+  if (dk_out != nullptr) return PNCE_ERR_UNSUPPORTED;   // feat_k is detached in the reference (:142)
+  if (math_mode < PNCE_MATH_SIMT_F32 || math_mode > PNCE_MATH_TC_BF16) return PNCE_ERR_ARG;
+  if (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 255u)) return PNCE_ERR_WORKSPACE;
+  cudaStream_t st0 = static_cast<cudaStream_t>(stream);
+  if (math_mode != PNCE_MATH_SIMT_F32 && rows_tc_ok(P, D)) {
+    // tensor-core modes: re-tile the rows into operand blobs (k_rows_pack), then the tcgen05 loss kernel in
+    // rows mode (rows used as given, d loss / d q written row-major).  P or D > 256: CUDA-core kernel below.
+    const pnce_rows_t row = {q, k, dq_out, P, D};
+    Params t;
+    if (carve_rows_multi_tc(&row, 1, batch, math_mode == PNCE_MATH_TC_BF16X3, ws, &t) > ws_bytes)
+      return PNCE_ERR_WORKSPACE;
+    t.math = math_mode;
+    t.tau = temperature;
+    t.loss_out = loss_out;
+    t.nonfinite = nonfinite;
+    t.b0 = 0; t.bn = batch;
+    const int rc = launch_rows_pack(t, st0);
+    if (rc != PNCE_OK) return rc;
+    return launch_loss_tc(t, st0);
+  }
+  // fp32 CUDA-core kernel on the rows as they are
+  Params p;
+  if (carve_rows_loss(batch, P, D, ws, &p) > ws_bytes) return PNCE_ERR_WORKSPACE;
+  p.tau = temperature;
+  p.loss_out = loss_out;
+  p.nonfinite = nonfinite;
+  LayerDev& L = p.L[0];
+  L.qn = const_cast<float*>(q);
+  L.kn = const_cast<float*>(k);
+  L.dq_rows = dq_out;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  PNCE_CUDA(cudaMemsetAsync(p.counter, 0, 2 * sizeof(unsigned), st));
+  return launch_loss_simt(p, st);
+}
+
 static int check_rows_multi(const pnce_rows_t* rows, int n, int batch) {
   if (rows == nullptr || n < 1 || n > PNCE_MAX_LAYERS || batch < 1) return PNCE_ERR_ARG;
   for (int l = 0; l < n; ++l) {
@@ -1503,15 +1508,8 @@ int pnce_rows_loss_multi_fwd_bwd(const pnce_rows_t* rows, int n_layers, int batc
   t.loss_out = loss_out;
   t.nonfinite = nonfinite;
   t.b0 = 0; t.bn = batch;
-  PNCE_CUDA(cudaMemsetAsync(t.counter, 0, 2 * sizeof(unsigned), st));
-  long long most = 0;
-  for (int l = 0; l < n_layers; ++l) {
-    const long long threads = 2ll * batch * t.L[l].Ppad * (t.L[l].Cp >> 3);
-    if (threads > most) most = threads;
-  }
-  const dim3 grid((unsigned)((most + kThreads - 1) / kThreads), (unsigned)n_layers);
-  launch_k(k_rows_pack, grid, kThreads, 0, st, t);
-  PNCE_CUDA(cudaGetLastError());
+  rc = launch_rows_pack(t, st);
+  if (rc != PNCE_OK) return rc;
   return launch_loss_tc(t, st);
 }
 
@@ -1556,15 +1554,8 @@ int pnce_rows_mb_fwd_bwd(const pnce_rows_t* rows, int n_layers, int batch, float
   t.mb = 1;
   t.total_ctas = 0;
   for (int l = 0; l < n_layers; ++l) t.total_ctas += (unsigned)(batch * (t.L[l].Ppad / 128));
-  PNCE_CUDA(cudaMemsetAsync(t.counter, 0, 2 * sizeof(unsigned), st));
-  long long most = 0;
-  for (int l = 0; l < n_layers; ++l) {
-    const long long threads = 2ll * batch * t.L[l].Ppad * (t.L[l].Cp >> 3);
-    if (threads > most) most = threads;
-  }
-  const dim3 grid((unsigned)((most + kThreads - 1) / kThreads), (unsigned)n_layers);
-  launch_k(k_rows_pack, grid, kThreads, 0, st, t);
-  PNCE_CUDA(cudaGetLastError());
+  rc = launch_rows_pack(t, st);
+  if (rc != PNCE_OK) return rc;
   return launch_loss_tc(t, st);
 }
 
@@ -1585,8 +1576,7 @@ int pnce_rows_mb_fwd_bwd(const pnce_rows_t* rows, int n_layers, int batch, float
 static int rows_shard_geometry(const pnce_rows_t* rows, int n, int batch_local, int world, pnce_layer_t* vl,
                                size_t* prefix, size_t* slot_bytes) {
   if (world < 1 || batch_local < 1) return PNCE_ERR_ARG;
-  if ((long long)world * batch_local > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
-  const int rc = check_rows_mb(rows, n, world * batch_local);
+  const int rc = global_batch_check(world, batch_local, [&](int B) { return check_rows_mb(rows, n, B); });
   if (rc != PNCE_OK) return rc;
   for (int l = 0; l < n; ++l) {
     memset(&vl[l], 0, sizeof(vl[l]));
@@ -1639,26 +1629,11 @@ int pnce_rows_mb_shard_keys(const pnce_rows_t* rows, int n_layers, int batch_loc
   for (int l = 0; l < n_layers; ++l)
     if (!rows[l].q || !rows[l].k) return PNCE_ERR_ARG;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  PNCE_CUDA(cudaMemsetAsync(t.counter, 0, 2 * sizeof(unsigned), st));
-  // the pack: queries into the prefix, keys straight into slot `rank`
-  long long most = 0;
-  for (int l = 0; l < n_layers; ++l) {
-    const long long threads = 2ll * batch_local * t.L[l].Ppad * (t.L[l].Cp >> 3);
-    if (threads > most) most = threads;
-  }
-  launch_k(k_rows_pack, dim3((unsigned)((most + kThreads - 1) / kThreads), (unsigned)n_layers), kThreads, 0, st, t);
-  PNCE_CUDA(cudaGetLastError());
-  // this rank's "a query row is non-finite" flags, next to its keys (see above for why k_mb_qbad is exact here)
-  int* flags = const_cast<int*>(t.qbad);
-  PNCE_CUDA(cudaMemsetAsync(flags, 0, PNCE_MAX_LAYERS * sizeof(int), st));
-  most = 1;
-  for (int l = 0; l < n_layers; ++l) {
-    const long long nq = (long long)batch_local * t.L[l].nchunk * t.L[l].Ppad;
-    if ((nq + kMbQbadFloats - 1) / kMbQbadFloats > most) most = (nq + kMbQbadFloats - 1) / kMbQbadFloats;
-  }
-  launch_k<2>(k_mb_qbad, dim3((unsigned)most, (unsigned)n_layers), kThreads, 0, st, t, flags);
-  PNCE_CUDA(cudaGetLastError());
-  return PNCE_OK;
+  // the pack: queries into the prefix, keys straight into slot `rank`; then this rank's query flags next to its keys
+  // (see above for why k_mb_qbad is exact here)
+  rc = launch_rows_pack(t, st);
+  if (rc != PNCE_OK) return rc;
+  return launch_mb_qbad(t, const_cast<int*>(t.qbad), st);
 }
 
 int pnce_rows_mb_shard_loss(const pnce_rows_t* rows, int n_layers, int batch_local, int world, int rank,
@@ -1666,7 +1641,7 @@ int pnce_rows_mb_shard_loss(const pnce_rows_t* rows, int n_layers, int batch_loc
                             void* stream) {
   static thread_local Params t;
   size_t slot_bytes = 0;
-  // the key blobs and qbad: slot 0 of `world` (k_loss_tc_mb_gn steps to slot w by w * kslot)
+  // the key blobs and qbad: slot 0 of `world` (point_at_slots)
   int rc = rows_shard_params(rows, n_layers, batch_local, world, rank, math_mode, ws, ws_bytes, 0, t, &slot_bytes);
   if (rc != PNCE_OK) return rc;
   if (loss_out == nullptr || !(temperature > 0.f)) return PNCE_ERR_ARG;
@@ -1677,11 +1652,7 @@ int pnce_rows_mb_shard_loss(const pnce_rows_t* rows, int n_layers, int batch_loc
   t.tau = temperature;
   t.loss_out = loss_out;
   t.nonfinite = nonfinite;
-  t.kworld = world;
-  t.kimg0 = rank * batch_local;
-  t.kslot = slot_bytes;
-  t.total_ctas = 0;
-  for (int l = 0; l < n_layers; ++l) t.total_ctas += (unsigned)(batch_local * (t.L[l].Ppad / 128));
+  point_at_slots(t, world, rank, slot_bytes);
   return launch_loss_tc(t, static_cast<cudaStream_t>(stream));
 }
 
@@ -2181,15 +2152,27 @@ int pnce_head_mb_fwd(const pnce_layer_t* layers, const pnce_head_t* heads, int n
 // only through the experiment build's knob 6, stores +Inf for an overflowing chunk: not covered.)  An unflagged row and
 // key then have norms below 5.2e19, and their logit is non-finite only when q . k overflows fp32, i.e. both norms above
 // 6.5e18: the one window where the owning rank guards alone (DESIGN.md 4.14).
-static void head_virtual_layers(const pnce_layer_t* layers, int n_layers, int nc, pnce_layer_t* out) {
+
+// The envelope of the GLOBAL batch and the slot geometry: *prefix, the slots' offset; *slot_bytes, their stride; vl, the
+// virtual layers (C = nc) the slots are carved on.  No CUDA call.
+static int head_shard_geometry(const pnce_layer_t* layers, int n_layers, int batch_local, int world, int nc,
+                               pnce_layer_t* vl, size_t* prefix, size_t* slot_bytes) {
+  const int rc = global_batch_check(world, batch_local, [&](int B) {
+    return head_mb_shapes_ok(layers, n_layers, B, nc) ? PNCE_OK : PNCE_ERR_UNSUPPORTED;
+  });
+  if (rc != PNCE_OK) return rc;
   for (int l = 0; l < n_layers; ++l) {
-    out[l] = layers[l];
-    out[l].C = nc;
+    vl[l] = layers[l];
+    vl[l].C = nc;
   }
+  *prefix = carve_head(layers, n_layers, batch_local, nc, true, nullptr, nullptr) +
+            carve_head_mb(layers, n_layers, batch_local, nullptr, nullptr);
+  *slot_bytes = carve_mb_slot(vl, n_layers, batch_local, true, nullptr, nullptr);
+  return PNCE_OK;
 }
 
-// The checks of the two shard calls, all before any CUDA call, then the carve of the prefix into hp.  *prefix: the
-// slots' offset; *slot_bytes: their stride; vl: the virtual layers (C = nc) the slots are carved on.
+// The checks of the two shard calls, all before any CUDA call, then the carve of the prefix into hp.  *prefix,
+// *slot_bytes, vl: head_shard_geometry's.
 static int head_shard_plan(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch_local,
                            int dtype, int layout, int nc, int world, int rank, int math_mode, void* ws, size_t ws_bytes,
                            HeadPlan& hp, pnce_layer_t* vl, size_t* prefix, size_t* slot_bytes) {
@@ -2203,15 +2186,11 @@ static int head_shard_plan(const pnce_layer_t* layers, const pnce_head_t* heads,
   for (int l = 0; l < n_layers; ++l)
     if (!heads[l].w1 || !heads[l].b1 || !heads[l].w2 || !heads[l].b2) return PNCE_ERR_ARG;
   if (math_mode == PNCE_MATH_SIMT_F32) return PNCE_ERR_UNSUPPORTED;
-  if ((long long)world * batch_local > 0x7fffffffLL || !head_mb_shapes_ok(layers, n_layers, world * batch_local, nc))
-    return PNCE_ERR_UNSUPPORTED;                               // the envelope of the GLOBAL batch
+  rc = head_shard_geometry(layers, n_layers, batch_local, world, nc, vl, prefix, slot_bytes);
+  if (rc != PNCE_OK) return rc;
   rc = check_alignment(layers, n_layers, dtype, false);
   if (rc != PNCE_OK) return rc;
   if (ws == nullptr || (reinterpret_cast<uintptr_t>(ws) & 255u)) return PNCE_ERR_WORKSPACE;
-  head_virtual_layers(layers, n_layers, nc, vl);
-  *prefix = carve_head(layers, n_layers, batch_local, nc, true, nullptr, nullptr) +
-            carve_head_mb(layers, n_layers, batch_local, nullptr, nullptr);
-  *slot_bytes = carve_mb_slot(vl, n_layers, batch_local, true, nullptr, nullptr);
   if (*prefix + (size_t)world * *slot_bytes > ws_bytes) return PNCE_ERR_WORKSPACE;
   const bool x3 = math_mode == PNCE_MATH_TC_BF16X3;
   const size_t used = carve_head(layers, n_layers, batch_local, nc, x3, ws, &hp);
@@ -2222,16 +2201,12 @@ static int head_shard_plan(const pnce_layer_t* layers, const pnce_head_t* heads,
 int pnce_head_mb_shard_workspace_bytes(const pnce_layer_t* layers, int n_layers, int batch_local, int world, int nc,
                                        size_t* bytes, size_t* slot_offset, size_t* slot_bytes) {
   if (bytes == nullptr || slot_offset == nullptr || slot_bytes == nullptr) return PNCE_ERR_ARG;
-  const int rc = check_layers(layers, n_layers, batch_local);
+  int rc = check_layers(layers, n_layers, batch_local);
   if (rc != PNCE_OK) return rc;
   if (world < 1) return PNCE_ERR_ARG;
-  if ((long long)world * batch_local > 0x7fffffffLL || !head_mb_shapes_ok(layers, n_layers, world * batch_local, nc))
-    return PNCE_ERR_UNSUPPORTED;
   pnce_layer_t vl[PNCE_MAX_LAYERS];
-  head_virtual_layers(layers, n_layers, nc, vl);
-  *slot_offset = carve_head(layers, n_layers, batch_local, nc, true, nullptr, nullptr) +
-                 carve_head_mb(layers, n_layers, batch_local, nullptr, nullptr);
-  *slot_bytes = carve_mb_slot(vl, n_layers, batch_local, true, nullptr, nullptr);
+  rc = head_shard_geometry(layers, n_layers, batch_local, world, nc, vl, slot_offset, slot_bytes);
+  if (rc != PNCE_OK) return rc;
   *bytes = *slot_offset + (size_t)world * *slot_bytes;
   return PNCE_OK;
 }
@@ -2254,18 +2229,7 @@ int pnce_head_mb_shard_keys(const pnce_layer_t* layers, const pnce_head_t* heads
   rc = head_fwd_keys(hp, layers, heads, n_layers, batch_local, nc, x3, true, nonfinite, kd, st);
   if (rc != PNCE_OK) return rc;
   // this rank's "a query row is non-finite" flags, next to its keys (see above for why k_mb_qbad is exact here)
-  const Params& pl = hp.pl;
-  int* flags = const_cast<int*>(kd.qbad);
-  PNCE_CUDA(cudaMemsetAsync(flags, 0, PNCE_MAX_LAYERS * sizeof(int), st));
-  long long most = 1;
-  for (int l = 0; l < n_layers; ++l) {
-    const long long n = (long long)batch_local * pl.L[l].nchunk * pl.L[l].Ppad;
-    if ((n + kMbQbadFloats - 1) / kMbQbadFloats > most) most = (n + kMbQbadFloats - 1) / kMbQbadFloats;
-  }
-  if (most > 0x7fffffffLL) return PNCE_ERR_UNSUPPORTED;
-  launch_k<2>(k_mb_qbad, dim3((unsigned)most, (unsigned)n_layers), kThreads, 0, st, pl, flags);
-  PNCE_CUDA(cudaGetLastError());
-  return PNCE_OK;
+  return launch_mb_qbad(hp.pl, const_cast<int*>(kd.qbad), st);
 }
 
 int pnce_head_mb_shard_loss(const pnce_layer_t* layers, const pnce_head_t* heads, int n_layers, int batch_local,
@@ -2279,12 +2243,10 @@ int pnce_head_mb_shard_loss(const pnce_layer_t* layers, const pnce_head_t* heads
   if (rc != PNCE_OK) return rc;
   if (loss_out == nullptr || !(temperature > 0.f)) return PNCE_ERR_ARG;
   head_fwd_setup(hp, batch_local, dtype, layout, math_mode, temperature, loss_out, nonfinite, true);
-  // the virtual layers' key blobs and qbad: slot 0 of `world` (k_loss_tc_mb_gn steps to slot w by w * kslot)
+  // the virtual layers' key blobs and qbad: slot 0 of `world` (point_at_slots)
   carve_mb_slot(vl, n_layers, batch_local, math_mode == PNCE_MATH_TC_BF16X3, static_cast<unsigned char*>(ws) + prefix,
                 &hp.pl);
-  hp.pl.kworld = world;
-  hp.pl.kimg0 = rank * batch_local;
-  hp.pl.kslot = slot_bytes;
+  point_at_slots(hp.pl, world, rank, slot_bytes);
   return head_fwd_loss(hp.pl, batch_local, static_cast<cudaStream_t>(stream));
 }
 

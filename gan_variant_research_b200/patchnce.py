@@ -499,7 +499,19 @@ def _run_fwd(call: _Call, tgt_feats):
                 a = layers[l]
                 a.src, a.tgt, a.ids = src[l].data_ptr(), tgt_feats[l].data_ptr(), ids[l].data_ptr()
             if sp.world > 1:
-                rc = _run_fwd_global(lib, call, layers, ws, out, flag_ptr, st)
+                rank = dist.get_rank(call.group)
+                layout = _lib.LAYOUT_NHWC if sp.nhwc else _lib.LAYOUT_NCHW
+                philox = (ctypes.c_ulonglong * 2)(call.rng[0], call.rng[1]) if call.rng is not None else None
+                pl = call.idplan
+                plp, pln = (pl.data_ptr(), pl.numel()) if pl is not None else (None, 0)
+                shard = (layers, n, sp.batch, sp.dtype_code, layout, sp.world, rank)
+                _exchange_keys(lib.pnce_mb_shard_keys,
+                               (*shard, sp.math_code, ws.data_ptr(), sp.ws_bytes, plp, pln, philox, st),
+                               lib.pnce_mb_shard_loss,
+                               (*shard, call.temperature, sp.math_code, ws.data_ptr(), sp.ws_bytes, plp, pln,
+                                out.data_ptr(), flag_ptr or None, st),
+                               ws, sp.slot_offset, sp.slot_bytes, sp.world, rank, call.group)
+                rc = 0
             elif sp.mb:
                 philox = (ctypes.c_ulonglong * 2)(call.rng[0], call.rng[1]) if call.rng is not None else None
                 pl = call.idplan
@@ -529,23 +541,25 @@ def _run_fwd(call: _Call, tgt_feats):
     return ws, out
 
 
-def _run_fwd_global(lib, call: _Call, layers, ws, out, flag_ptr, st) -> int:
-    """Global negatives: this rank's keys into its slot of the workspace, the all-gather of the slots (the one
-    collective of the mode; keys carry no gradient, so the backward is local), then the loss over every rank's keys."""
+class _WsBytes(int):
+    """A workspace size in bytes, cached per shape, that also records where the slots of global negatives lie in that
+    workspace: ``slot_offset`` and ``slot_bytes`` (both 0 on one rank)."""
+
+    def __new__(cls, nbytes, slot_offset=0, slot_bytes=0):
+        self = super().__new__(cls, nbytes)
+        self.slot_offset, self.slot_bytes = slot_offset, slot_bytes
+        return self
+
+
+def _exchange_keys(keys, keys_args, loss, loss_args, ws, slot_offset, slot_bytes, world, rank, group):
+    """Global negatives on any route (maps, netF head, rows): ``keys`` (the route's pnce_*_mb_shard_keys) puts this
+    rank's keys into its slot of the workspace, the slots ``ws[slot_offset : slot_offset + world * slot_bytes]`` are
+    all-gathered (the one collective of the mode; keys carry no gradient, so the backward is local), then ``loss``
+    (pnce_*_mb_shard_loss) contrasts every rank's keys.  Raises on a failed status, under the entry point's name."""
     from . import dp
-    sp = call.sp
-    rank = dist.get_rank(call.group)
-    layout = _lib.LAYOUT_NHWC if sp.nhwc else _lib.LAYOUT_NCHW
-    philox = (ctypes.c_ulonglong * 2)(call.rng[0], call.rng[1]) if call.rng is not None else None
-    pl = call.idplan
-    plp, pln = (pl.data_ptr(), pl.numel()) if pl is not None else (None, 0)
-    rc = lib.pnce_mb_shard_keys(layers, sp.n, sp.batch, sp.dtype_code, layout, sp.world, rank, sp.math_code,
-                                ws.data_ptr(), sp.ws_bytes, plp, pln, philox, st)
-    if rc != 0:
-        return rc
-    dp.allgather_slots_(ws[sp.slot_offset:sp.slot_offset + sp.world * sp.slot_bytes], rank, call.group)
-    return lib.pnce_mb_shard_loss(layers, sp.n, sp.batch, sp.dtype_code, layout, sp.world, rank, call.temperature,
-                                  sp.math_code, ws.data_ptr(), sp.ws_bytes, plp, pln, out.data_ptr(), flag_ptr or None, st)
+    _lib.check(keys(*keys_args), keys.__name__)
+    dp.allgather_slots_(ws[slot_offset:slot_offset + world * slot_bytes], rank, group)
+    _lib.check(loss(*loss_args), loss.__name__)
 
 
 # ---- compressible memory for the dense gradients (csrc/comp_alloc.cuh) ---------------------------------------------
@@ -1248,23 +1262,25 @@ class _RowsLossMultiFn(torch.autograd.Function):
             key = tuple(key)
             ws_bytes = _ROWS_WS_BYTES.get(key)
             if ws_bytes is None:
-                nbytes = ctypes.c_size_t(0)
+                nbytes, so, sb = ctypes.c_size_t(0), ctypes.c_size_t(0), ctypes.c_size_t(0)
                 if world > 1:
-                    so, sb = ctypes.c_size_t(0), ctypes.c_size_t(0)
                     _lib.check(lib.pnce_rows_mb_shard_workspace_bytes(rows, n, batch, world, ctypes.byref(nbytes),
                                                                       ctypes.byref(so), ctypes.byref(sb)),
                                "pnce_rows_mb_shard_workspace_bytes")
-                    _ROWS_SLOTS[key] = (so.value, sb.value)
                 else:
                     wsq = lib.pnce_rows_mb_workspace_bytes if mb else lib.pnce_rows_loss_multi_workspace_bytes
                     _lib.check(wsq(rows, n, batch, ctypes.byref(nbytes)), "rows workspace query")
-                ws_bytes = _ROWS_WS_BYTES[key] = nbytes.value
+                ws_bytes = _ROWS_WS_BYTES[key] = _WsBytes(nbytes.value, so.value, sb.value)
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
             out = torch.empty(1 + n, dtype=torch.float32, device=dev)
             slot, flag_ptr = _warn_queue(dev).acquire(mb)
             if world > 1:
-                _rows_fwd_global(lib, rows, n, batch, temperature, math, group, world, _ROWS_SLOTS[key], ws, ws_bytes,
-                                 out, flag_ptr or None, _stream_ptr(dev))
+                rank, m, st = dist.get_rank(group), _MATH[math], _stream_ptr(dev)
+                shard = (rows, n, batch, world, rank)
+                _exchange_keys(lib.pnce_rows_mb_shard_keys, (*shard, m, ws.data_ptr(), ws_bytes, st),
+                               lib.pnce_rows_mb_shard_loss, (*shard, temperature, m, ws.data_ptr(), ws_bytes,
+                                                             out.data_ptr(), flag_ptr or None, st),
+                               ws, ws_bytes.slot_offset, ws_bytes.slot_bytes, world, rank, group)
             else:
                 fn = lib.pnce_rows_mb_fwd_bwd if mb else lib.pnce_rows_loss_multi_fwd_bwd
                 _lib.check(fn(rows, n, batch, temperature, _MATH[math], ws.data_ptr(), ws_bytes, out.data_ptr(),
@@ -1280,23 +1296,6 @@ class _RowsLossMultiFn(torch.autograd.Function):
         dqs = torch._foreach_mul(list(ctx.saved_tensors), grad_out)            # one launch for every layer
         dqs = [d if d.dtype is dt else d.to(dt) for d, dt in zip(dqs, ctx.q_dtypes)]
         return (None, None, None, None, None, None, *dqs, *([None] * len(dqs)))
-
-
-_ROWS_SLOTS = {}         # global negatives: (slot offset, slot bytes) per key of _ROWS_WS_BYTES
-
-
-def _rows_fwd_global(lib, rows, n, batch, temperature, math, group, world, slots, ws, ws_bytes, out, flag_ptr, st):
-    """Global negatives on the row route: this rank's keys packed into its slot of the workspace, the all-gather of the
-    slots (the one collective of the mode; keys carry no gradient, so the backward is local), then the loss and d q over
-    every rank's keys."""
-    from . import dp
-    rank = dist.get_rank(group)
-    so, sb = slots
-    _lib.check(lib.pnce_rows_mb_shard_keys(rows, n, batch, world, rank, _MATH[math], ws.data_ptr(), ws_bytes, st),
-               "pnce_rows_mb_shard_keys")
-    dp.allgather_slots_(ws[so:so + world * sb], rank, group)
-    _lib.check(lib.pnce_rows_mb_shard_loss(rows, n, batch, world, rank, temperature, _MATH[math], ws.data_ptr(),
-                                           ws_bytes, out.data_ptr(), flag_ptr, st), "pnce_rows_mb_shard_loss")
 
 
 def _rows_batches(feat_q, feat_k, num_patches, batch_size):
@@ -1511,47 +1510,32 @@ def _head_fwd(plan, nc, tgt, params):
     if ws_bytes is None:
         if len(_HEAD_WS_BYTES) > 256:       # a caller cycling through many shapes: do not grow without bound
             _HEAD_WS_BYTES.clear()
-            _HEAD_SLOTS.clear()
-        nbytes = ctypes.c_size_t(0)
+        nbytes, so, sb = ctypes.c_size_t(0), ctypes.c_size_t(0), ctypes.c_size_t(0)
         if world > 1:
-            so, sb = ctypes.c_size_t(0), ctypes.c_size_t(0)
             _lib.check(lib.pnce_head_mb_shard_workspace_bytes(layers, n, batch, world, nc, ctypes.byref(nbytes),
                                                               ctypes.byref(so), ctypes.byref(sb)),
                        "pnce_head_mb_shard_workspace_bytes")
-            _HEAD_SLOTS[key] = (so.value, sb.value)
         else:
             query = lib.pnce_head_mb_workspace_bytes if mb else lib.pnce_head_workspace_bytes
             _lib.check(query(layers, n, batch, nc, ctypes.byref(nbytes)), "pnce_head_workspace_bytes")
-        ws_bytes = _HEAD_WS_BYTES[key] = nbytes.value
+        ws_bytes = _HEAD_WS_BYTES[key] = _WsBytes(nbytes.value, so.value, sb.value)
     with _on_device(dev):
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         out = torch.empty(1 + n, dtype=torch.float32, device=dev)
         wq = _warn_queue(dev)
         slot, flag_ptr = wq.acquire(plan.mb)
         if world > 1:
-            _head_fwd_global(lib, plan, nc, key, layers, heads, batch, dtype, layout, ws, ws_bytes, out, flag_ptr or None,
-                             _stream_ptr(dev))
+            rank, math, st = dist.get_rank(plan.group), _MATH[plan.math], _stream_ptr(dev)
+            shard = (layers, heads, n, batch, dtype, layout, nc, world, rank)
+            _exchange_keys(lib.pnce_head_mb_shard_keys, (*shard, math, ws.data_ptr(), ws_bytes, flag_ptr or None, st),
+                           lib.pnce_head_mb_shard_loss, (*shard, plan.temperature, math, ws.data_ptr(), ws_bytes,
+                                                         out.data_ptr(), flag_ptr or None, st),
+                           ws, ws_bytes.slot_offset, ws_bytes.slot_bytes, world, rank, plan.group)
         else:
             fwd = lib.pnce_head_mb_fwd if mb else lib.pnce_head_fwd_ex
             _lib.check(fwd(layers, heads, n, batch, dtype, layout, nc, plan.temperature, _MATH[plan.math],
                            ws.data_ptr(), ws_bytes, out.data_ptr(), flag_ptr or None, _stream_ptr(dev)), "pnce_head_fwd")
     return ws, out, (ws_bytes, layout, dev, batch, dtype, heads)
-
-
-def _head_fwd_global(lib, plan, nc, key, layers, heads, batch, dtype, layout, ws, ws_bytes, out, flag_ptr, st):
-    """Global negatives: this rank's head output up to its keys, which go into its slot of the workspace; the all-gather
-    of the slots (the one collective of the mode; keys carry no gradient, so the backward is local); then the loss over
-    every rank's keys."""
-    from . import dp
-    n, world, math = len(layers), plan.world, _MATH[plan.math]
-    rank = dist.get_rank(plan.group)
-    so, sb = _HEAD_SLOTS[key]
-    _lib.check(lib.pnce_head_mb_shard_keys(layers, heads, n, batch, dtype, layout, nc, world, rank, math, ws.data_ptr(),
-                                           ws_bytes, flag_ptr, st), "pnce_head_mb_shard_keys")
-    dp.allgather_slots_(ws[so:so + world * sb], rank, plan.group)
-    _lib.check(lib.pnce_head_mb_shard_loss(layers, heads, n, batch, dtype, layout, nc, world, rank, plan.temperature,
-                                           math, ws.data_ptr(), ws_bytes, out.data_ptr(), flag_ptr, st),
-               "pnce_head_mb_shard_loss")
 
 
 def _head_bwd(plan, nc, tgt, params, ws, state, g, flat=None):
@@ -1632,7 +1616,6 @@ class _FusedHeadPatchNCE(torch.autograd.Function):
 
 
 _HEAD_WS_BYTES = {}      # pnce_head_workspace_bytes per (device, dtype, layout, nc, mb, map shapes, patch counts, world)
-_HEAD_SLOTS = {}         # global negatives: (slot offset, slot bytes) per key of _HEAD_WS_BYTES
 
 
 def _head_params(netF, n):
