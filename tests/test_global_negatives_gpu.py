@@ -74,6 +74,7 @@ def _virtual_shards(src, tgt, ids, tau, math, world):
         _lib.check(lib.pnce_bwd_ex(arrs[r], n, bl, dcode, _lib.LAYOUT_NCHW, mcode, ws[r].data_ptr(), nb.value, None, 0,
                                    None, st), "pnce_bwd_ex")
     torch.cuda.synchronize()
+    assert all(int(f[1].item()) == 0 for f in flags)             # no tensor-core protocol timeout
     return [o[0].item() for o in outs], grads, [int(f[0].item()) for f in flags]
 
 
